@@ -2,7 +2,7 @@
 """Benchmark of the batched phase-vocoder hot path (BASELINE.json metric: audio-seconds per wall-second,
 2048-point pitch shift, batched streams).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--streams S] [--secs T]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--streams S] [--secs T] [--dump-outputs DIR]
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
   python bench.py --impl reference      # the reference's own CPU path on the host cores
 
@@ -77,7 +77,11 @@ def parse():
     ap.add_argument("--parity-rows", type=int, default=4)
     ap.add_argument("--host-alloc", default="numa", choices=["numa", "numa-huge", "torch"],
                     help="pinned host buffers of the e2e legs: pvgpu_host_alloc on the GPU's NUMA node (default), the same on explicit 2 MB pages, or torch pin_memory")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed to DIR/<name>.npy (rank 0; a fixed sample of rows, see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
     global SR, CHANNELS, TIMERATIO, SEMITONES, MODE, COREMODE, FFT
     SR, CHANNELS, TIMERATIO, SEMITONES, MODE, COREMODE, FFT, default_streams = WORKLOADS[args.workload]
     if args.streams <= 0:
@@ -482,6 +486,8 @@ def main():
     value = audio_sec_per_step / (ms_step / 1e3)
     n_out_min = int(n_out.min())
     checksum = float(d_out[:, :n_out_min].double().abs().mean().item())
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, torch, d_out, n_out, n_streams)
 
     # rows of THIS batch checked against the reference after the timed regions (first / last / spread in between)
     pr = sorted(set(int(round(i * (n_streams - 1) / max(args.parity_rows - 1, 1))) for i in range(min(args.parity_rows, n_streams))))
@@ -604,6 +610,41 @@ def main():
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()
+
+
+DUMP_ROWS, DUMP_BYTES = 16, 48 << 20
+
+
+def dump_outputs(out_dir, torch, d_out, n_out, n_streams):
+    """Write what the last timed step left in d_out, so that two builds can be compared output for output (the inputs are
+    seeded: the same arguments give the same inputs).  Every stream's output length and, per channel, the float64 sum and sum
+    of squares over all its samples; and the samples themselves of a fixed, seeded choice of streams -- at most DUMP_ROWS, as
+    many as fit in DUMP_BYTES, cut to that size if one stream alone is larger.  Samples past a stream's length are zero."""
+    os.makedirs(out_dir, exist_ok=True)
+    n_out = np.asarray(n_out, dtype=np.int64)
+    width = int(n_out.max())
+    lengths = torch.as_tensor(np.repeat(n_out, CHANNELS), device=d_out.device)
+    col = torch.arange(width, device=d_out.device)
+    sums, sumsq = [], []
+    for r0 in range(0, d_out.shape[0], 64):
+        blk = d_out[r0:r0 + 64, :width].double()
+        blk *= col[None, :] < lengths[r0:r0 + 64, None]
+        sums.append(blk.sum(1))
+        sumsq.append((blk * blk).sum(1))
+        del blk
+    k = max(1, min(DUMP_ROWS, n_streams, DUMP_BYTES // (4 * CHANNELS * width)))
+    cols = min(width, DUMP_BYTES // (4 * CHANNELS * k))
+    pick = np.sort(np.random.default_rng(0).choice(n_streams, k, replace=False))
+    rows = torch.as_tensor((pick[:, None] * CHANNELS + np.arange(CHANNELS)[None, :]).reshape(-1), device=d_out.device)
+    sample = d_out[:, :cols].index_select(0, rows).cpu().numpy().reshape(k, CHANNELS, cols)
+    for i, s in enumerate(pick):
+        sample[i, :, n_out[s]:] = 0.0
+    out = {"output_rows": sample, "output_row_streams": pick.astype(np.float64),
+           "output_lengths": n_out.astype(np.float64),
+           "output_row_sums": torch.cat(sums).cpu().numpy().reshape(n_streams, CHANNELS),
+           "output_row_sumsq": torch.cat(sumsq).cpu().numpy().reshape(n_streams, CHANNELS)}
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def _block(n, world, rank):

@@ -40,6 +40,20 @@ def make_input(name, sr, ch, secs, seed):
     return x
 
 
+GOLDEN_EDGE, GOLDEN_INNER = 128, 512
+
+
+def golden_cols(n):
+    """The fixed sample positions (of an output n samples long) at which tests/golden/make_gpu_golden.py stores outputs: the
+    first and last GOLDEN_EDGE samples (start-up and flush) and GOLDEN_INNER seeded positions in between.  Whole outputs
+    would make the stored vectors too large to keep in the repository."""
+    import numpy as np
+    edge = min(GOLDEN_EDGE, n)
+    inner = np.arange(edge, max(edge, n - edge))
+    pick = np.random.default_rng(n).choice(inner, min(inner.size, GOLDEN_INNER), replace=False)
+    return np.unique(np.concatenate([np.arange(edge), np.arange(max(0, n - edge), n), pick]))
+
+
 def ctor_args(kw):
     """(timeratio, semitones, mode, coremode, fftsize) in the reference constructor's order."""
     return (kw.get("timeratio", 1.0), kw.get("semitones", 0.0), kw.get("mode", 0), kw.get("coremode", 1), kw.get("fftsize", 2048))

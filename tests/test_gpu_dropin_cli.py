@@ -31,7 +31,7 @@ def _read_wav(path):
                                      (["formant_pitchshift", "4", "1", "2048"], 1), (["robotic"], 2)])
 def test_reference_cli_on_gpu_library(tmp_path, args, ch):
     if not (os.path.exists(REF) and os.path.exists(GPU)):
-        pytest.skip("oracle/_ref CLI binaries were not built (need /root/reference at build time)")
+        pytest.skip("oracle/_ref/audiomod-exe or audiomod-exe-gpu is absent: make -C oracle ref REF=<reference sources> builds them")
     from audiomod_b200.synth import synth_int16
     sr = 48000 if args[0] == "time_stretch" else 44100
     pcm = synth_int16(1001, sr, 1.5, ch)

@@ -11,7 +11,7 @@ import os
 import numpy as np
 import pytest
 
-from cases import CASES, ctor_args, make_input
+from cases import CASES, ctor_args, golden_cols, make_input
 
 pytestmark = pytest.mark.gpu
 
@@ -35,6 +35,13 @@ def assert_parity(y, ref, what=""):
         snr = 10 * np.log10(pw / e) if e > 0 and pw > 0 else float("inf")
         assert mx <= MAX_ABS, f"{what} ch{c}: max-abs {mx:.3e}"
         assert snr >= MIN_SNR_DB, f"{what} ch{c}: SNR {snr:.1f} dB"
+
+
+def assert_parity_golden(y, gold, key, what=""):
+    """assert_parity against an output stored as its length (key__n) and its samples at cases.golden_cols (key)."""
+    n = int(gold[key + "__n"])
+    assert y.shape[1] == n, f"{what}: sample count {y.shape[1]} != stored {n}"
+    assert_parity(y[:, golden_cols(n)], gold[key], what)
 
 
 @pytest.fixture(scope="module")
