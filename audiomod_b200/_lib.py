@@ -44,6 +44,8 @@ class WavJob(C.Structure):
 
 _fp = C.POINTER(C.c_float)
 _fpp = C.POINTER(_fp)
+_sp = C.POINTER(C.c_int16)
+_spp = C.POINTER(_sp)
 _vpp = C.POINTER(C.c_void_p)
 _i64p = C.POINTER(C.c_int64)
 
@@ -60,6 +62,12 @@ SYMBOLS = {
     "pvgpu_process_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int, C.c_void_p]),
     "pvgpu_retrieve_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int, C.c_void_p]),
     "pvgpu_process_block_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int, C.c_void_p, C.POINTER(C.c_int)]),
+    "pvgpu_process_s16": (C.c_int, [C.c_void_p, _spp, C.c_int]),
+    "pvgpu_retrieve_s16": (C.c_int, [C.c_void_p, _spp, C.c_int]),
+    "pvgpu_process_block_s16": (C.c_int, [C.c_void_p, _spp, C.c_int, C.POINTER(C.c_int)]),
+    "pvgpu_process_device_s16": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int, C.c_void_p]),
+    "pvgpu_retrieve_device_s16": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int, C.c_void_p]),
+    "pvgpu_process_block_device_s16": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int, C.c_void_p, C.POINTER(C.c_int)]),
     "pvgpu_destroy": (None, [C.c_void_p]),
     "pvgpu_process": (C.c_int, [C.c_void_p, _fpp, C.c_int]),
     "pvgpu_available": (C.c_int, [C.c_void_p]),

@@ -22,6 +22,7 @@
 #include <new>
 #include <string>
 #include <thread>
+#include <type_traits>
 #include <vector>
 
 #include "../../include/pvgpu.h"
@@ -1496,7 +1497,10 @@ int pvgpu_test_princarg(int device, int64_t n, const double *a, double *out) {
 // those frames on the device and moves the produced samples into a host FIFO.
 // ------------------------------------------------------------------------------------------------
 // Small persistent pool for the per-row host copies of a live batch (thousands of rows per call: a single thread moves them at
-// ~6 GB/s, which is what bounds the call).  run(n, f) calls f(i) for i in [0, n) on the workers and the caller.
+// ~6 GB/s, which is what bounds the call).  run(n, samples_per_item, f) calls f(i) for i in [0, n) on the workers and the caller
+// when the call moves at least 256 K samples (1 MB of float32), else on the caller alone.  The threshold counts samples, not
+// bytes: 1024 rows of 480 int16 samples (983 KB) packed on one thread took 181 us per call against 64 us for the same rows of
+// float32 on the pool (B200 at 1000 W, profiles/r03_live_s16_latency_byte_threshold.jsonl).
 struct RowPool {
     std::vector<std::thread> workers;
     std::mutex m;
@@ -1533,8 +1537,8 @@ struct RowPool {
             l.lock();
         }
     }
-    template <typename F> void run(size_t count, size_t bytes_per_item, F &&f) {
-        if (workers.empty() || count * bytes_per_item < ((size_t)1 << 20)) { for (size_t i = 0; i < count; ++i) f(i); return; }
+    template <typename F> void run(size_t count, size_t samples_per_item, F &&f) {
+        if (workers.empty() || count * samples_per_item < ((size_t)1 << 18)) { for (size_t i = 0; i < count; ++i) f(i); return; }
         std::unique_lock<std::mutex> l(m);
         fn = std::forward<F>(f);
         n = count; next = 0; chunk = std::max<size_t>(1, count / (4 * (workers.size() + 1)));
@@ -1548,20 +1552,22 @@ struct RowPool {
 
 // Output FIFO of a streaming instance: every row holds the same number of samples (the rows advance in lock-step), so it is
 // one [rows][cap] block with a common read position -- a ring (cap a power of two), no per-row containers, no compaction.
-// The block is page-locked when it can be: the device-to-host copy of a call's output lands in the ring directly.
+// The block is page-locked when it can be: the device-to-host copy of a call's output lands in the ring directly.  T is the
+// instance's sample type (float, or int16_t for int16 rows).
+template <typename T>
 struct RowFifo {
-    float *buf = nullptr;
+    T *buf = nullptr;
     bool pinned = false;
     size_t rows = 0, cap = 0, rd = 0, count = 0;
     ~RowFifo() { release(); }
     void release() { if (buf) { if (pinned) cudaFreeHost(buf); else std::free(buf); } buf = nullptr; cap = 0; }
     void init(size_t rows_) { release(); rows = rows_; rd = count = 0; }
-    static float *alloc(size_t bytes, bool *pinned) {
+    static T *alloc(size_t bytes, bool *pinned) {
         void *p = nullptr;
-        if (cudaHostAlloc(&p, bytes, cudaHostAllocDefault) == cudaSuccess) { *pinned = true; return (float *)p; }
+        if (cudaHostAlloc(&p, bytes, cudaHostAllocDefault) == cudaSuccess) { *pinned = true; return (T *)p; }
         cudaGetLastError();
         *pinned = false;
-        return (float *)std::malloc(bytes);
+        return (T *)std::malloc(bytes);
     }
     // only between calls (no copy in flight)
     bool reserve(size_t need) {
@@ -1569,7 +1575,7 @@ struct RowFifo {
         size_t ncap = cap ? cap : 4096;
         while (ncap < need) ncap *= 2;
         bool np = false;
-        float *nb = alloc(sizeof(float) * rows * ncap, &np);
+        T *nb = alloc(sizeof(T) * rows * ncap, &np);
         if (!nb) return false;
         for (size_t r = 0; r < rows; ++r)
             for (size_t i = 0; i < count; ++i) nb[r * ncap + i] = buf[r * cap + ((rd + i) & (cap - 1))];
@@ -1581,12 +1587,12 @@ struct RowFifo {
     void write_span(size_t n, size_t *w, size_t *first) const { *w = (rd + count) & (cap - 1); *first = std::min(n, cap - *w); }
     void commit(size_t n) { count += n; }
     // remove the oldest k samples of every row into out[r]
-    void pop(float *const *out, size_t k, RowPool &pool) {
+    void pop(T *const *out, size_t k, RowPool &pool) {
         if (k == 0) return;
         const size_t first = std::min(k, cap - rd);
-        pool.run(rows, sizeof(float) * k, [&, first, k](size_t r) {
-            std::memcpy(out[r], &buf[r * cap + rd], sizeof(float) * first);
-            if (first < k) std::memcpy(out[r] + first, &buf[r * cap], sizeof(float) * (k - first));
+        pool.run(rows, k, [&, first, k](size_t r) {
+            std::memcpy(out[r], &buf[r * cap + rd], sizeof(T) * first);
+            if (first < k) std::memcpy(out[r] + first, &buf[r * cap], sizeof(T) * (k - first));
         });
         rd = (rd + k) & (cap - 1);
         count -= k;
@@ -1604,34 +1610,42 @@ struct pvgpu_stream {
     std::unique_ptr<Carrier> carrier;
     GlibcRand rng;
     Workspace ws;
-    // input fed by calls that completed no slice (not yet on the device): [rows][pend_cap], pend_len valid per row
-    std::vector<float> pend;
+    // Kind of rows the instance is fed, fixed by its first data call: 0 not used yet, 1 host rows, 2 device rows (float32),
+    // 3 host rows, 4 device rows (int16).  An int16 instance keeps int16 end to end: pending input, packed upload, device window,
+    // output rings; the kernels convert as they load and quantise as they store (g.fmt = PVGPU_S16).
+    int io_mode = 0;
+    bool dev_rows() const { return io_mode == 2 || io_mode == 4; }
+    size_t esz() const { return io_mode >= 3 ? sizeof(int16_t) : sizeof(float); }   // bytes per sample of the instance's rows
+    // input fed by calls that completed no slice (not yet on the device): [rows][pend_cap] samples of the instance's type,
+    // pend_len valid per row
+    std::vector<unsigned char> pend;
     size_t pend_cap = 0, pend_len = 0;
-    void pend_append(const float *const *in, size_t n) {
+    template <typename T> T *pend_row(size_t r) { return reinterpret_cast<T *>(pend.data()) + r * pend_cap; }
+    template <typename T> void pend_append(const T *const *in, size_t n) {
         const size_t R_ = (size_t)R();
         if (pend_len + n > pend_cap) {
             size_t ncap = pend_cap ? pend_cap : 1024;
             while (ncap < pend_len + n) ncap *= 2;
-            std::vector<float> nb(R_ * ncap);
-            for (size_t r = 0; r < R_; ++r) std::memcpy(&nb[r * ncap], pend.data() + r * pend_cap, sizeof(float) * pend_len);
+            std::vector<unsigned char> nb(sizeof(T) * R_ * ncap);
+            for (size_t r = 0; r < R_; ++r) std::memcpy(nb.data() + sizeof(T) * r * ncap, pend_row<T>(r), sizeof(T) * pend_len);
             pend.swap(nb);
             pend_cap = ncap;
         }
-        for (size_t r = 0; r < R_; ++r) std::memcpy(&pend[r * pend_cap + pend_len], in[r], sizeof(float) * n);
+        for (size_t r = 0; r < R_; ++r) std::memcpy(pend_row<T>(r) + pend_len, in[r], sizeof(T) * n);
         pend_len += n;
     }
-    // The input window [in_base, in_base + dev_len) lives on the device, in one of two buffers of in_cap floats per row: a call
+    // The input window [in_base, in_base + dev_len) lives on the device, in one of two buffers of in_cap samples per row: a call
     // uploads only the samples it was fed and compacts the still-needed part into the other buffer on the device.
     DevBuf d_inbuf[2];
     int cur_in = 0;
     int64_t in_cap = 0, dev_len = 0;
     std::vector<float> car_tail;
     int64_t in_base = 0;
-    RowFifo fifo;                          // output FIFO of all rows (the reference's outbuf ring)
+    RowFifo<float> fifo;                   // output FIFO of all rows (the reference's outbuf ring)
+    RowFifo<int16_t> fifo16;               // the same for int16 rows
     // Device-resident I/O (pvgpu_process_device / _retrieve_device): rows come from and go to device memory, everything is
     // enqueued on the caller's stream and no call waits for the device.  The output FIFO is a ring [rows][dfifo_cap] on the
     // device; what a call uploads is staged in one of four page-locked arenas, each guarded by an event.
-    int io_mode = 0;                       // 0 not used yet, 1 host rows, 2 device rows
     DevBuf d_fifo;
     size_t dfifo_cap = 0, dfifo_rd = 0, dfifo_count = 0;
     static constexpr int kDevArenas = 4;
@@ -1646,7 +1660,8 @@ struct pvgpu_stream {
     long tr_calls = 0;
     int num_res = 0;
     DevBuf d_out, d_car, d_len, d_stage;
-    std::vector<float> h_stage, h_pack, scratch;
+    std::vector<float> h_stage, scratch;
+    std::vector<unsigned char> h_pack;
     PinnedArena arena;
     cudaStream_t st = nullptr;
     static constexpr int kF = 64;
@@ -1662,24 +1677,32 @@ struct pvgpu_stream {
 static int stream_ensure_window(pvgpu_stream *s, int64_t len, cudaStream_t st) {
     if (len <= s->in_cap) return PVGPU_OK;
     const int R = s->R();
+    const size_t es = s->esz();
     const int64_t cap = (std::max<int64_t>(2 * s->in_cap, len + 4096) + 3) & ~(int64_t)3;
     DevBuf grown;
-    CU(grown.ensure(sizeof(float) * (size_t)R * cap));
+    CU(grown.ensure(es * (size_t)R * cap));
     if (s->dev_len > 0)
-        CU(cudaMemcpy2DAsync(grown.p, sizeof(float) * cap, s->d_inbuf[s->cur_in].p, sizeof(float) * s->in_cap, sizeof(float) * s->dev_len, R, cudaMemcpyDeviceToDevice, st));
+        CU(cudaMemcpy2DAsync(grown.p, es * cap, s->d_inbuf[s->cur_in].p, es * s->in_cap, es * s->dev_len, R, cudaMemcpyDeviceToDevice, st));
     CU(cudaStreamSynchronize(st));
     std::swap(s->d_inbuf[s->cur_in].p, grown.p);
     std::swap(s->d_inbuf[s->cur_in].bytes, grown.bytes);
     s->d_inbuf[s->cur_in ^ 1].release();
-    CU(s->d_inbuf[s->cur_in ^ 1].ensure(sizeof(float) * (size_t)R * cap));
+    CU(s->d_inbuf[s->cur_in ^ 1].ensure(es * (size_t)R * cap));
     s->in_cap = cap;
     return PVGPU_OK;
 }
 
+template <typename T> static RowFifo<T> &host_fifo(pvgpu_stream *s) {
+    if constexpr (std::is_same<T, float>::value) return s->fifo; else return s->fifo16;
+}
+
 // One pvgpu_process call that completed `added` new slices starting at slice k0.  Steady state: no heap allocation (the
 // vectors keep their capacity), every upload goes through the page-locked arena, one stream synchronisation at the end.
-static int stream_run_new(pvgpu_stream *s, long k0, int added, const float *const *in, int n_new, cudaStream_t user_st = nullptr) {
-    const bool dev = s->io_mode == 2;      // device rows: the input is already in the window, everything goes on the caller's stream
+// T is the sample type of the instance's rows (float or int16_t).
+template <typename T>
+static int stream_run_new(pvgpu_stream *s, long k0, int added, const T *const *in, int n_new, cudaStream_t user_st = nullptr) {
+    static_assert(std::is_same<T, float>::value || std::is_same<T, int16_t>::value, "float32 or int16 rows");
+    const bool dev = s->dev_rows();        // device rows: the input is already in the window, everything goes on the caller's stream
     cudaStream_t const st = dev ? user_st : s->st;
     Pipeline &pl = s->pl;
     Scheduler &sc = *s->sched;
@@ -1719,24 +1742,25 @@ static int stream_run_new(pvgpu_stream *s, long k0, int added, const float *cons
     int rc;
     if ((rc = stream_ensure_window(s, len, st))) return rc;
     const int64_t in_stride = s->in_cap;
-    float *d_in = s->d_inbuf[s->cur_in].as<float>();
+    T *d_in = s->d_inbuf[s->cur_in].as<T>();
     if (pend > 0) {
         // all rows' new samples straight from the caller's rows into one page-locked block, one copy (a live batch of thousands
         // of rows must not issue a copy per row); without page-locked memory the same block is pageable and the copy synchronous
-        const int64_t pp = (pend + 15) & ~(int64_t)15;   // packed row pitch: rows start on 64-byte lines
-        float *pin = (float *)s->arena.take(sizeof(float) * (size_t)R * pp);
+        constexpr int64_t line = 64 / sizeof(T);
+        const int64_t pp = (pend + line - 1) & ~(line - 1);   // packed row pitch: rows start on 64-byte lines
+        T *pin = (T *)s->arena.take(sizeof(T) * (size_t)R * pp);
         const bool locked = pin != nullptr;
-        if (!pin) { s->h_pack.resize((size_t)R * pp); pin = s->h_pack.data(); }
+        if (!pin) { s->h_pack.resize(sizeof(T) * (size_t)R * pp); pin = (T *)s->h_pack.data(); }
         const size_t pl_ = s->pend_len;
         // non-temporal stores: the copy engine reads this block next, and lines left dirty in several cores' caches slow it 4-7x
-        s->pool.run((size_t)R, sizeof(float) * (size_t)pend, [&, pl_, pin, pp, locked](size_t r) {
+        s->pool.run((size_t)R, (size_t)pend, [&, pl_, pin, pp, locked](size_t r) {
             if (locked) {
-                if (pl_) copy_nt(pin + r * pp, s->pend.data() + r * s->pend_cap, pl_);
+                if (pl_) copy_nt(pin + r * pp, s->pend_row<T>(r), pl_);
                 if (n_new) copy_nt(pin + r * pp + pl_, in[r], (size_t)n_new);
                 copy_nt_fence();
             } else {
-                if (pl_) std::memcpy(pin + r * pp, s->pend.data() + r * s->pend_cap, sizeof(float) * pl_);
-                if (n_new) std::memcpy(pin + r * pp + pl_, in[r], sizeof(float) * (size_t)n_new);
+                if (pl_) std::memcpy(pin + r * pp, s->pend_row<T>(r), sizeof(T) * pl_);
+                if (n_new) std::memcpy(pin + r * pp + pl_, in[r], sizeof(T) * (size_t)n_new);
             }
         });
         mark(0);   // pack
@@ -1744,11 +1768,11 @@ static int stream_run_new(pvgpu_stream *s, long k0, int added, const float *cons
         if (R >= 64) {
             // many short rows: one contiguous copy over PCIe, then the pitched placement on the device (a host-to-device 2-D copy
             // of 4096 rows of 1.9 KB to 4-byte-aligned destinations ran at 7 GB/s, and so did the device-to-device one)
-            CU(s->d_stage.ensure(sizeof(float) * (size_t)R * pp));
-            CU(cudaMemcpyAsync(s->d_stage.p, pin, sizeof(float) * (size_t)R * pp, cudaMemcpyHostToDevice, st));
-            launch_place_rows(d_in + s->dev_len, in_stride, s->d_stage.as<float>(), pp, (int)pend, R, st);
+            CU(s->d_stage.ensure(sizeof(T) * (size_t)R * pp));
+            CU(cudaMemcpyAsync(s->d_stage.p, pin, sizeof(T) * (size_t)R * pp, cudaMemcpyHostToDevice, st));
+            launch_place_rows(d_in + s->dev_len, in_stride, s->d_stage.as<T>(), pp, (int)pend, R, st);
         } else {
-            CU(cudaMemcpy2DAsync(d_in + s->dev_len, sizeof(float) * in_stride, pin, sizeof(float) * pp, sizeof(float) * pend, R, cudaMemcpyHostToDevice, st));
+            CU(cudaMemcpy2DAsync(d_in + s->dev_len, sizeof(T) * in_stride, pin, sizeof(T) * pp, sizeof(T) * pend, R, cudaMemcpyHostToDevice, st));
         }
         if (trace) cudaEventRecord(s->tr_ev[6], st);   // input placed
     }
@@ -1760,13 +1784,14 @@ static int stream_run_new(pvgpu_stream *s, long k0, int added, const float *cons
     if ((rc = pl.h2d(s->d_len.p, s->lim.data(), sizeof(int64_t) * (2 * (size_t)R + 1), st))) return rc;
     if ((rc = pl.upload_schedule(sc, st))) return rc;
     if ((rc = pl.build_resample_runs(k0, k0 + added, pl.fused ? pl.fa.run : ola_run_limit(p, 8, pl.max_consumed, pl.max_out), st))) return rc;
-    CU(s->d_out.ensure(sizeof(float) * (size_t)R * out_stride));
+    CU(s->d_out.ensure(sizeof(T) * (size_t)R * out_stride));
     if (!pl.fused && halo_of(sc.recs(), sc.recs_base(), p.rs_active ? (int)p.rs_filt_len : 1) > s->ws.Fr - s->ws.F) return fail(PVGPU_ESTATE, "too many overlapping (dropped) slices; retrieve output more often");
     DevRows g{};
     g.rows = R; g.channels = C;
     g.in = d_in; g.in_stride = in_stride; g.in_base = s->in_base;
+    g.fmt = std::is_same<T, int16_t>::value ? PVGPU_S16 : PVGPU_F32;   // int16: the kernels convert on load and quantise on store
     g.n_in = s->d_len.as<int64_t>(); g.n_out = s->d_len.as<int64_t>() + R;
-    g.out = s->d_out.as<float>(); g.out_stride = out_stride; g.out_base = out_base;
+    g.out = s->d_out.as<T>(); g.out_stride = out_stride; g.out_base = out_base;
     s->ws.bind(pl, g);
     g.aux_base = k0;
     if (pl.d.whisper) {   // whisperSlice draws rand() channel-major per slice (:814-822): the next added * C * H values of this instance's generator
@@ -1800,23 +1825,24 @@ static int stream_run_new(pvgpu_stream *s, long k0, int added, const float *cons
             size_t ncap = s->dfifo_cap ? s->dfifo_cap : 4096;
             while (ncap < s->dfifo_count + (size_t)new_out) ncap *= 2;
             DevBuf grown;
-            CU(grown.ensure(sizeof(float) * (size_t)R * ncap));
-            if (s->dfifo_count) launch_ring_rows(grown.as<float>(), (int64_t)ncap, 0, -1, s->d_fifo.as<float>(), (int64_t)s->dfifo_cap, (int64_t)s->dfifo_rd, (int64_t)s->dfifo_cap - 1, (int)s->dfifo_count, R, st);
+            CU(grown.ensure(sizeof(T) * (size_t)R * ncap));
+            if (s->dfifo_count) launch_ring_rows(grown.as<T>(), (int64_t)ncap, 0, -1, s->d_fifo.as<T>(), (int64_t)s->dfifo_cap, (int64_t)s->dfifo_rd, (int64_t)s->dfifo_cap - 1, (int)s->dfifo_count, R, st);
             CU(cudaStreamSynchronize(st));
             std::swap(s->d_fifo.p, grown.p);
             std::swap(s->d_fifo.bytes, grown.bytes);
             s->dfifo_cap = ncap; s->dfifo_rd = 0;
         }
-        launch_ring_rows(s->d_fifo.as<float>(), (int64_t)s->dfifo_cap, (int64_t)((s->dfifo_rd + s->dfifo_count) & (s->dfifo_cap - 1)), (int64_t)s->dfifo_cap - 1, s->d_out.as<float>(), out_stride, 0, -1,
+        launch_ring_rows(s->d_fifo.as<T>(), (int64_t)s->dfifo_cap, (int64_t)((s->dfifo_rd + s->dfifo_count) & (s->dfifo_cap - 1)), (int64_t)s->dfifo_cap - 1, s->d_out.as<T>(), out_stride, 0, -1,
                          (int)new_out, R, st);
         s->dfifo_count += (size_t)new_out;
     } else if (new_out > 0) {   // the output goes straight into the (page-locked) FIFO ring
-        if (!s->fifo.reserve(s->fifo.count + (size_t)new_out)) return fail(PVGPU_ENOMEM, "out of host memory");
+        RowFifo<T> &fifo = host_fifo<T>(s);
+        if (!fifo.reserve(fifo.count + (size_t)new_out)) return fail(PVGPU_ENOMEM, "out of host memory");
         size_t w, first;
-        s->fifo.write_span((size_t)new_out, &w, &first);
-        CU(cudaMemcpy2DAsync(s->fifo.buf + w, sizeof(float) * s->fifo.cap, s->d_out.p, sizeof(float) * out_stride, sizeof(float) * first, R, cudaMemcpyDeviceToHost, st));
+        fifo.write_span((size_t)new_out, &w, &first);
+        CU(cudaMemcpy2DAsync(fifo.buf + w, sizeof(T) * fifo.cap, s->d_out.p, sizeof(T) * out_stride, sizeof(T) * first, R, cudaMemcpyDeviceToHost, st));
         if (first < (size_t)new_out)
-            CU(cudaMemcpy2DAsync(s->fifo.buf, sizeof(float) * s->fifo.cap, s->d_out.as<float>() + first, sizeof(float) * out_stride, sizeof(float) * ((size_t)new_out - first), R,
+            CU(cudaMemcpy2DAsync(fifo.buf, sizeof(T) * fifo.cap, s->d_out.as<T>() + first, sizeof(T) * out_stride, sizeof(T) * ((size_t)new_out - first), R,
                                  cudaMemcpyDeviceToHost, st));
     }
     if (trace) cudaEventRecord(s->tr_ev[3], st);   // output copy done
@@ -1827,7 +1853,7 @@ static int stream_run_new(pvgpu_stream *s, long k0, int added, const float *cons
     const int64_t keep = len - dropn;
     if (dropn > 0) {
         if (keep > 0)
-            CU(cudaMemcpy2DAsync(s->d_inbuf[s->cur_in ^ 1].p, sizeof(float) * in_stride, d_in + dropn, sizeof(float) * in_stride, sizeof(float) * keep, R, cudaMemcpyDeviceToDevice, st));
+            CU(cudaMemcpy2DAsync(s->d_inbuf[s->cur_in ^ 1].p, sizeof(T) * in_stride, d_in + dropn, sizeof(T) * in_stride, sizeof(T) * keep, R, cudaMemcpyDeviceToDevice, st));
         s->cur_in ^= 1;
     }
     if (trace) cudaEventRecord(s->tr_ev[4], st);   // window compaction done
@@ -1843,7 +1869,7 @@ static int stream_run_new(pvgpu_stream *s, long k0, int added, const float *cons
     if (trace) for (int i = 0; i < 4; ++i) { float ms = 0; cudaEventElapsedTime(&ms, s->tr_ev[i], s->tr_ev[i + 1]); s->tr_dev[i] += 1e3 * ms; }
     if (trace && pend > 0) { float ms = 0; cudaEventElapsedTime(&ms, s->tr_ev[0], s->tr_ev[5]); s->tr_dev2[0] += 1e3 * ms; cudaEventElapsedTime(&ms, s->tr_ev[5], s->tr_ev[6]); s->tr_dev2[1] += 1e3 * ms; }
     pl.staged_all = true;
-    if (new_out > 0 && !dev) s->fifo.commit((size_t)new_out);
+    if (new_out > 0 && !dev) host_fifo<T>(s).commit((size_t)new_out);
     s->pend_len = 0;
     s->dev_len = keep;
     if (pl.d.vocoder) s->car_tail.erase(s->car_tail.begin(), s->car_tail.begin() + std::min<int64_t>(dropn, (int64_t)s->car_tail.size()));
@@ -1873,46 +1899,54 @@ static int stream_run_new(pvgpu_stream *s, long k0, int added, const float *cons
     return PVGPU_OK;
 }
 
-// Host-only self-test of the live batch's containers (no device work): the ring FIFO across wrap-arounds and growth, the
-// row-copy pool against a serial copy, non-temporal copies at every alignment.  Returns 0 or the number of the failed check.
-static int host_structs_selftest() {
-    {   // RowFifo
-        const size_t R = 7;
-        RowFifo f;
-        f.init(R);
-        RowPool none;
-        std::vector<std::vector<float>> model(R);
-        std::vector<float> block;
-        std::vector<float *> out(R);
-        std::vector<std::vector<float>> got(R);
-        unsigned seed = 12345;
-        float next = 0.f;
-        for (int it = 0; it < 400; ++it) {
-            seed = seed * 1664525u + 1013904223u;
-            const size_t n = (seed >> 16) % (it % 50 == 49 ? 9000 : 700);
-            if (!f.reserve(f.count + n)) return 1;
-            size_t w, first;
-            f.write_span(n, &w, &first);
-            for (size_t r = 0; r < R; ++r)
-                for (size_t i = 0; i < n; ++i) {
-                    const float v = next + (float)r * 0.25f + (float)i;
-                    model[r].push_back(v);
-                    if (i < first) f.buf[r * f.cap + w + i] = v; else f.buf[r * f.cap + (i - first)] = v;
-                }
-            next += 1000.f;
-            f.commit(n);
-            seed = seed * 1664525u + 1013904223u;
-            const size_t k = std::min<size_t>(f.count, (seed >> 16) % 900);
-            for (size_t r = 0; r < R; ++r) { got[r].assign(k + 1, -1.f); out[r] = got[r].data(); }
-            f.pop(out.data(), k, none);
-            for (size_t r = 0; r < R; ++r) {
-                for (size_t i = 0; i < k; ++i) if (got[r][i] != model[r][i]) return 2;
-                if (got[r][k] != -1.f) return 3;
-                model[r].erase(model[r].begin(), model[r].begin() + (long)k);
+// Ring FIFO of one sample type across wrap-arounds, growth and partial pops against a plain model.  Returns 0 or base + the
+// number of the failed check (1 reserve, 2 popped samples, 3 a sample past the popped ones written, 4 count).
+template <typename T> static int fifo_selftest(int base) {
+    const size_t R = 7;
+    RowFifo<T> f;
+    f.init(R);
+    RowPool none;
+    std::vector<std::vector<T>> model(R);
+    std::vector<T *> out(R);
+    std::vector<std::vector<T>> got(R);
+    unsigned seed = 12345;
+    float next = 0.f;
+    for (int it = 0; it < 400; ++it) {
+        seed = seed * 1664525u + 1013904223u;
+        const size_t n = (seed >> 16) % (it % 50 == 49 ? 9000 : 700);
+        if (!f.reserve(f.count + n)) return base + 1;
+        size_t w, first;
+        f.write_span(n, &w, &first);
+        for (size_t r = 0; r < R; ++r)
+            for (size_t i = 0; i < n; ++i) {
+                T v;
+                if constexpr (std::is_same<T, float>::value) v = next + (float)r * 0.25f + (float)i;
+                else v = (T)(uint16_t)((unsigned)it * 977u + (unsigned)r * 131u + (unsigned)i);   // every bit pattern, -1 included
+                model[r].push_back(v);
+                if (i < first) f.buf[r * f.cap + w + i] = v; else f.buf[r * f.cap + (i - first)] = v;
             }
-            if (f.count != model[0].size()) return 4;
+        next += 1000.f;
+        f.commit(n);
+        seed = seed * 1664525u + 1013904223u;
+        const size_t k = std::min<size_t>(f.count, (seed >> 16) % 900);
+        for (size_t r = 0; r < R; ++r) { got[r].assign(k + 1, (T)-1); out[r] = got[r].data(); }
+        f.pop(out.data(), k, none);
+        for (size_t r = 0; r < R; ++r) {
+            for (size_t i = 0; i < k; ++i) if (got[r][i] != model[r][i]) return base + 2;
+            if (got[r][k] != (T)-1) return base + 3;
+            model[r].erase(model[r].begin(), model[r].begin() + (long)k);
         }
+        if (f.count != model[0].size()) return base + 4;
     }
+    return 0;
+}
+
+// Host-only self-test of the live batch's containers (no device work): the ring FIFO across wrap-arounds and growth, the
+// row-copy pool against a serial copy, non-temporal copies at every alignment; float32 rows (checks 1-6), int16 rows (7-11).
+// Returns 0 or the number of the failed check.
+static int host_structs_selftest() {
+    int rc;
+    if ((rc = fifo_selftest<float>(0))) return rc;
     {   // RowPool + copy_nt
         RowPool pool;
         pool.start(3);
@@ -1921,15 +1955,30 @@ static int host_structs_selftest() {
         for (size_t i = 0; i < src.size(); ++i) src[i] = (float)(i % 9973) * 0.5f;
         for (int rep = 0; rep < 20; ++rep) {
             const size_t shift = (size_t)rep % 8;   // every destination alignment
-            pool.run(R, sizeof(float) * n, [&](size_t r) { copy_nt(&a[r * (n + 24) + shift], &src[r * n], n); copy_nt_fence(); });
+            pool.run(R, n, [&](size_t r) { copy_nt(&a[r * (n + 24) + shift], &src[r * n], n); copy_nt_fence(); });
             for (size_t r = 0; r < R; ++r) std::memcpy(&b[r * (n + 24) + shift], &src[r * n], sizeof(float) * n);
             if (std::memcmp(a.data(), b.data(), sizeof(float) * a.size()) != 0) return 5;
         }
         size_t hits = 0;
         std::vector<unsigned char> seen(R, 0);
-        pool.run(R, (size_t)1 << 20, [&](size_t r) { seen[r]++; });
+        pool.run(R, (size_t)1 << 18, [&](size_t r) { seen[r]++; });
         for (unsigned char c : seen) hits += c;
         if (hits != R) return 6;
+    }
+    if ((rc = fifo_selftest<int16_t>(6))) return rc;
+    {   // 16-bit copy_nt at every 2-byte destination alignment of a 16-byte line, odd and even lengths, through the pool
+        RowPool pool;
+        pool.start(3);
+        const size_t R = 600;
+        for (size_t n : {(size_t)0, (size_t)1, (size_t)2, (size_t)3, (size_t)8, (size_t)9, (size_t)17, (size_t)1031}) {
+            std::vector<int16_t> src(R * n), a(R * (n + 24), -2), b(R * (n + 24), -2);
+            for (size_t i = 0; i < src.size(); ++i) src[i] = (int16_t)(uint16_t)(i * 40503u);
+            for (size_t shift = 0; shift < 8; ++shift) {
+                pool.run(R, n, [&](size_t r) { copy_nt(&a[r * (n + 24) + shift], &src[r * n], n); copy_nt_fence(); });
+                for (size_t r = 0; r < R; ++r) std::memcpy(&b[r * (n + 24) + shift], &src[r * n], sizeof(int16_t) * n);
+                if (std::memcmp(a.data(), b.data(), sizeof(int16_t) * a.size()) != 0) return 11;
+            }
+        }
     }
     return 0;
 }
@@ -1963,6 +2012,7 @@ static int pvgpu_create_body(const pvgpu_config *cfg, int n_streams, pvgpu_strea
     s->sched.reset(new Scheduler(s->pl.d, true));
     if (s->pl.d.vocoder) s->carrier.reset(new Carrier(cfg->sample_rate, cfg->mode == PVGPU_VOCODER_CHORD));
     s->fifo.init((size_t)s->R());
+    s->fifo16.init((size_t)s->R());
     if (s->R() >= 256) s->pool.start((int)std::min(7u, std::max(1u, std::thread::hardware_concurrency() / 2)));   // live batch: parallel row copies
     CU(cudaStreamCreateWithFlags(&s->st, cudaStreamNonBlocking));
     const int halo = 80;
@@ -1999,15 +2049,33 @@ int pvgpu_stream_info(const pvgpu_stream *s, pvgpu_info *info) {
     return PVGPU_OK;
 }
 
-static int pvgpu_process_body(pvgpu_stream *s, const float *const *in, int n);
-int pvgpu_process(pvgpu_stream *s, const float *const *in, int n) {
-    return guarded([&]() -> int { return pvgpu_process_body(s, in, n); });
+}  // extern "C"
+
+// The kind of rows an instance takes is fixed by its first data call (pvgpu_stream::io_mode); a call of another kind is refused
+// with the name of the call to use.
+static const char *const kRowKind[5] = {"", "host", "device", "host int16", "device int16"};
+static const char *const kProcessCall[5] = {"", "pvgpu_process", "pvgpu_process_device", "pvgpu_process_s16", "pvgpu_process_device_s16"};
+static const char *const kRetrieveCall[5] = {"", "pvgpu_retrieve", "pvgpu_retrieve_device", "pvgpu_retrieve_s16", "pvgpu_retrieve_device_s16"};
+static int lock_rows(pvgpu_stream *s, int mode) {
+    const int have = s->io_mode;
+    if (have && have != mode)
+        return fail(PVGPU_ESTATE, "this instance is fed %s rows (%s); %s rows cannot be mixed", kRowKind[have], kProcessCall[have],
+                    (have >= 3) != (mode >= 3) ? "float32 and int16" : "host and device");
+    s->io_mode = mode;
+    return PVGPU_OK;
 }
-static int pvgpu_process_body(pvgpu_stream *s, const float *const *in, int n) {
+static int check_retrieve_rows(const pvgpu_stream *s, int mode) {
+    const int have = s->io_mode;
+    if (have && have != mode) return fail(PVGPU_ESTATE, "this instance is fed %s rows; use %s", kRowKind[have], kRetrieveCall[have]);
+    return PVGPU_OK;
+}
+
+template <typename T>
+static int process_host(pvgpu_stream *s, const T *const *in, int n) {
     if (!s || n < 0 || (n > 0 && !in)) return fail(PVGPU_EINVAL, "bad argument");
     if (!s->pl.d.valid_mode) { s->num_res = 0; return PVGPU_OK; }  // phasevocoder.cc:104-106: unknown mode does nothing
-    if (s->io_mode == 2) return fail(PVGPU_ESTATE, "this instance is fed device rows (pvgpu_process_device); host and device rows cannot be mixed");
-    s->io_mode = 1;
+    int rc;
+    if ((rc = lock_rows(s, std::is_same<T, float>::value ? 1 : 3))) return rc;
     if (s->carrier) {
         const size_t at = s->car_tail.size();
         s->car_tail.resize(at + n);
@@ -2016,37 +2084,37 @@ static int pvgpu_process_body(pvgpu_stream *s, const float *const *in, int n) {
     const long k0 = s->sched->recs_base() + s->sched->slices();
     const int added = s->sched->feed(n);   // the schedule does not depend on the data
     if (added > 0) {
-        int rc = stream_run_new(s, k0, added, in, n);
-        if (rc) return rc;
+        if ((rc = stream_run_new<T>(s, k0, added, in, n))) return rc;
     } else if (n > 0) {
-        s->pend_append(in, (size_t)n);
+        s->pend_append<T>(in, (size_t)n);
     }
     s->num_res = (int)s->sched->available();
     return PVGPU_OK;
 }
 
-int pvgpu_available(const pvgpu_stream *s) { return s ? s->num_res : 0; }
-
-int pvgpu_retrieve(pvgpu_stream *s, float *const *out, int n) {
+template <typename T>
+static int retrieve_host(pvgpu_stream *s, T *const *out, int n) {
     if (!s || n < 0 || (n > 0 && !out)) return -fail(PVGPU_EINVAL, "bad argument");
-    if (s->io_mode == 2) return -fail(PVGPU_ESTATE, "this instance is fed device rows; use pvgpu_retrieve_device");
+    if (check_retrieve_rows(s, std::is_same<T, float>::value ? 1 : 3)) return -PVGPU_ESTATE;
+    RowFifo<T> &fifo = host_fifo<T>(s);
     long k = std::min<long>(n, s->num_res);  // phasevocoder.cc:111-113
     k = std::min<long>(k, s->sched->available());
-    k = std::min<long>(k, (long)s->fifo.count);
-    s->fifo.pop(out, (size_t)k, s->pool);
+    k = std::min<long>(k, (long)fifo.count);
+    fifo.pop(out, (size_t)k, s->pool);
     s->sched->drain(k);
     return (int)k;
 }
 
-int pvgpu_process_block(pvgpu_stream *s, float *const *buf, int n, int *ready) {
+template <typename T>
+static int process_block_host(pvgpu_stream *s, T *const *buf, int n, int *ready) {
     if (!s || !ready) return fail(PVGPU_EINVAL, "bad argument");
     const int m = s->cfg.mode;
     if (m == PVGPU_NORMAL_STRETCH || m < -1 || m > PVGPU_FORMANT_CEPSTRAL) { *ready = 1; return PVGPU_OK; }  // processBlock routes neither (phasevocoder.cc:133-146)
-    int rc = pvgpu_process(s, buf, n);
+    int rc = guarded([&]() -> int { return process_host<T>(s, buf, n); });
     if (rc) return rc;
     if (s->num_res >= n) {  // processBlockNormal, phasevocoder.cc:156-183
         const int saved = s->num_res;
-        pvgpu_retrieve(s, buf, n);
+        retrieve_host<T>(s, buf, n);
         s->num_res = saved;
         *ready = 1;
     } else {
@@ -2055,11 +2123,12 @@ int pvgpu_process_block(pvgpu_stream *s, float *const *buf, int n, int *ready) {
     return PVGPU_OK;
 }
 
-static int pvgpu_process_device_body(pvgpu_stream *s, const float *d_in, int64_t in_pitch, int n, cudaStream_t st) {
+template <typename T>
+static int process_device(pvgpu_stream *s, const T *d_in, int64_t in_pitch, int n, cudaStream_t st) {
     if (!s || n < 0 || (n > 0 && !d_in) || in_pitch < n) return fail(PVGPU_EINVAL, "bad argument");
     if (!s->pl.d.valid_mode) { s->num_res = 0; return PVGPU_OK; }
-    if (s->io_mode == 1) return fail(PVGPU_ESTATE, "this instance is fed host rows (pvgpu_process); host and device rows cannot be mixed");
-    s->io_mode = 2;
+    int rc;
+    if ((rc = lock_rows(s, std::is_same<T, float>::value ? 2 : 4))) return rc;
     CU(cudaSetDevice(s->pl.device));
     if (s->carrier) {
         const size_t at = s->car_tail.size();
@@ -2068,29 +2137,26 @@ static int pvgpu_process_device_body(pvgpu_stream *s, const float *d_in, int64_t
     }
     const long k0 = s->sched->recs_base() + s->sched->slices();
     const int added = s->sched->feed(n);   // the schedule does not depend on the data: no call has to wait for the device
-    int rc;
     if (n > 0) {   // the new samples join the device-resident window right away
         if ((rc = stream_ensure_window(s, s->dev_len + n, st))) return rc;
-        launch_place_rows(s->d_inbuf[s->cur_in].as<float>() + s->dev_len, s->in_cap, d_in, in_pitch, n, s->R(), st);
+        launch_place_rows(s->d_inbuf[s->cur_in].as<T>() + s->dev_len, s->in_cap, d_in, in_pitch, n, s->R(), st);
         s->dev_len += n;
     }
-    if (added > 0 && (rc = stream_run_new(s, k0, added, nullptr, 0, st))) return rc;
+    if (added > 0 && (rc = stream_run_new<T>(s, k0, added, nullptr, 0, st))) return rc;
     s->num_res = (int)s->sched->available();
     return PVGPU_OK;
 }
-int pvgpu_process_device(pvgpu_stream *s, const float *d_in, int64_t in_pitch, int n, void *cuda_stream) {
-    return guarded([&]() -> int { return pvgpu_process_device_body(s, d_in, in_pitch, n, cuda_stream ? (cudaStream_t)cuda_stream : cudaStreamLegacy); });
-}
 
-int pvgpu_retrieve_device(pvgpu_stream *s, float *d_out, int64_t out_pitch, int n, void *cuda_stream) {
+template <typename T>
+static int retrieve_device(pvgpu_stream *s, T *d_out, int64_t out_pitch, int n, void *cuda_stream) {
     if (!s || n < 0 || (n > 0 && !d_out) || out_pitch < n) return -fail(PVGPU_EINVAL, "bad argument");
-    if (s->io_mode == 1) return -fail(PVGPU_ESTATE, "this instance is fed host rows; use pvgpu_retrieve");
+    if (check_retrieve_rows(s, std::is_same<T, float>::value ? 2 : 4)) return -PVGPU_ESTATE;
     long k = std::min<long>(n, s->num_res);
     k = std::min<long>(k, s->sched->available());
     k = std::min<long>(k, (long)s->dfifo_count);
     if (k > 0) {
         if (cudaSetDevice(s->pl.device) != cudaSuccess) return -fail(PVGPU_ECUDA, "cudaSetDevice failed");
-        launch_ring_rows(d_out, out_pitch, 0, -1, s->d_fifo.as<float>(), (int64_t)s->dfifo_cap, (int64_t)s->dfifo_rd, (int64_t)s->dfifo_cap - 1, (int)k, s->R(),
+        launch_ring_rows(d_out, out_pitch, 0, -1, s->d_fifo.as<T>(), (int64_t)s->dfifo_cap, (int64_t)s->dfifo_rd, (int64_t)s->dfifo_cap - 1, (int)k, s->R(),
                          cuda_stream ? (cudaStream_t)cuda_stream : cudaStreamLegacy);
         s->dfifo_rd = (s->dfifo_rd + (size_t)k) & (s->dfifo_cap - 1);
         s->dfifo_count -= (size_t)k;
@@ -2100,15 +2166,16 @@ int pvgpu_retrieve_device(pvgpu_stream *s, float *d_out, int64_t out_pitch, int 
     return (int)k;
 }
 
-int pvgpu_process_block_device(pvgpu_stream *s, float *d_buf, int64_t pitch, int n, void *cuda_stream, int *ready) {
+template <typename T>
+static int process_block_device(pvgpu_stream *s, T *d_buf, int64_t pitch, int n, void *cuda_stream, int *ready) {
     if (!s || !ready) return fail(PVGPU_EINVAL, "bad argument");
     const int m = s->cfg.mode;
     if (m == PVGPU_NORMAL_STRETCH || m < -1 || m > PVGPU_FORMANT_CEPSTRAL) { *ready = 1; return PVGPU_OK; }
-    int rc = pvgpu_process_device(s, d_buf, pitch, n, cuda_stream);
+    int rc = guarded([&]() -> int { return process_device<T>(s, d_buf, pitch, n, cuda_stream ? (cudaStream_t)cuda_stream : cudaStreamLegacy); });
     if (rc) return rc;
     if (s->num_res >= n) {
         const int saved = s->num_res;
-        const int k = pvgpu_retrieve_device(s, d_buf, pitch, n, cuda_stream);
+        const int k = retrieve_device<T>(s, d_buf, pitch, n, cuda_stream);
         if (k < 0) return -k;
         s->num_res = saved;
         *ready = 1;
@@ -2116,6 +2183,44 @@ int pvgpu_process_block_device(pvgpu_stream *s, float *d_buf, int64_t pitch, int
         *ready = 0;
     }
     return PVGPU_OK;
+}
+
+extern "C" {
+
+int pvgpu_process(pvgpu_stream *s, const float *const *in, int n) {
+    return guarded([&]() -> int { return process_host<float>(s, in, n); });
+}
+int pvgpu_process_s16(pvgpu_stream *s, const int16_t *const *in, int n) {
+    return guarded([&]() -> int { return process_host<int16_t>(s, in, n); });
+}
+
+int pvgpu_available(const pvgpu_stream *s) { return s ? s->num_res : 0; }
+
+int pvgpu_retrieve(pvgpu_stream *s, float *const *out, int n) { return retrieve_host<float>(s, out, n); }
+int pvgpu_retrieve_s16(pvgpu_stream *s, int16_t *const *out, int n) { return retrieve_host<int16_t>(s, out, n); }
+
+int pvgpu_process_block(pvgpu_stream *s, float *const *buf, int n, int *ready) { return process_block_host<float>(s, buf, n, ready); }
+int pvgpu_process_block_s16(pvgpu_stream *s, int16_t *const *buf, int n, int *ready) { return process_block_host<int16_t>(s, buf, n, ready); }
+
+int pvgpu_process_device(pvgpu_stream *s, const float *d_in, int64_t in_pitch, int n, void *cuda_stream) {
+    return guarded([&]() -> int { return process_device<float>(s, d_in, in_pitch, n, cuda_stream ? (cudaStream_t)cuda_stream : cudaStreamLegacy); });
+}
+int pvgpu_process_device_s16(pvgpu_stream *s, const int16_t *d_in, int64_t in_pitch, int n, void *cuda_stream) {
+    return guarded([&]() -> int { return process_device<int16_t>(s, d_in, in_pitch, n, cuda_stream ? (cudaStream_t)cuda_stream : cudaStreamLegacy); });
+}
+
+int pvgpu_retrieve_device(pvgpu_stream *s, float *d_out, int64_t out_pitch, int n, void *cuda_stream) {
+    return retrieve_device<float>(s, d_out, out_pitch, n, cuda_stream);
+}
+int pvgpu_retrieve_device_s16(pvgpu_stream *s, int16_t *d_out, int64_t out_pitch, int n, void *cuda_stream) {
+    return retrieve_device<int16_t>(s, d_out, out_pitch, n, cuda_stream);
+}
+
+int pvgpu_process_block_device(pvgpu_stream *s, float *d_buf, int64_t pitch, int n, void *cuda_stream, int *ready) {
+    return process_block_device<float>(s, d_buf, pitch, n, cuda_stream, ready);
+}
+int pvgpu_process_block_device_s16(pvgpu_stream *s, int16_t *d_buf, int64_t pitch, int n, void *cuda_stream, int *ready) {
+    return process_block_device<int16_t>(s, d_buf, pitch, n, cuda_stream, ready);
 }
 
 }  // extern "C"

@@ -1143,25 +1143,32 @@ void launch_synthesise(const DevPlan &p, const DevRows &g, const float *car_mag,
 }
 
 // dst[r * dst_pitch + ((dst_off + i) & dst_mask)] = src[r * src_pitch + ((src_off + i) & src_mask)], i < width: row-wise copy
-// with independent pitches and any 4-byte alignment; a mask of cap - 1 makes that side a ring of cap floats per row (the
+// with independent pitches and any element alignment; a mask of cap - 1 makes that side a ring of cap elements per row (the
 // device-resident output FIFO of a streaming instance), -1 a plain row.  Places the packed new input of a live batch behind the
-// rows' device-resident windows (a 2-D cudaMemcpy of 4096 such rows ran at 7 GB/s).
-__global__ void k_place_rows(float *__restrict__ dst, int64_t dst_pitch, int64_t dst_off, int64_t dst_mask, const float *__restrict__ src, int64_t src_pitch,
+// rows' device-resident windows (a 2-D cudaMemcpy of 4096 such rows ran at 7 GB/s).  T = float or short (int16 instances).
+template <typename T>
+__global__ void k_place_rows(T *__restrict__ dst, int64_t dst_pitch, int64_t dst_off, int64_t dst_mask, const T *__restrict__ src, int64_t src_pitch,
                              int64_t src_off, int64_t src_mask, int width) {
     const int r = blockIdx.y;
-    const float *__restrict__ s = src + (int64_t)r * src_pitch;
-    float *__restrict__ d = dst + (int64_t)r * dst_pitch;
+    const T *__restrict__ s = src + (int64_t)r * src_pitch;
+    T *__restrict__ d = dst + (int64_t)r * dst_pitch;
     for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < width; i += gridDim.x * blockDim.x) d[(dst_off + i) & dst_mask] = s[(src_off + i) & src_mask];
 }
-void launch_place_rows(float *dst, int64_t dst_pitch, const float *src, int64_t src_pitch, int width, int rows, cudaStream_t st) {
+template <typename T>
+void launch_place_rows(T *dst, int64_t dst_pitch, const T *src, int64_t src_pitch, int width, int rows, cudaStream_t st) {
     launch_ring_rows(dst, dst_pitch, 0, -1, src, src_pitch, 0, -1, width, rows, st);
 }
-void launch_ring_rows(float *dst, int64_t dst_pitch, int64_t dst_off, int64_t dst_mask, const float *src, int64_t src_pitch, int64_t src_off, int64_t src_mask,
+template <typename T>
+void launch_ring_rows(T *dst, int64_t dst_pitch, int64_t dst_off, int64_t dst_mask, const T *src, int64_t src_pitch, int64_t src_off, int64_t src_mask,
                       int width, int rows, cudaStream_t st) {
     if (width <= 0 || rows <= 0) return;
     dim3 grid((unsigned)std::min(8, (width + 255) / 256), (unsigned)rows);
-    k_place_rows<<<grid, 256, 0, st>>>(dst, dst_pitch, dst_off, dst_mask, src, src_pitch, src_off, src_mask, width);
+    k_place_rows<T><<<grid, 256, 0, st>>>(dst, dst_pitch, dst_off, dst_mask, src, src_pitch, src_off, src_mask, width);
 }
+template void launch_place_rows<float>(float *, int64_t, const float *, int64_t, int, int, cudaStream_t);
+template void launch_place_rows<short>(short *, int64_t, const short *, int64_t, int, int, cudaStream_t);
+template void launch_ring_rows<float>(float *, int64_t, int64_t, int64_t, const float *, int64_t, int64_t, int64_t, int, int, cudaStream_t);
+template void launch_ring_rows<short>(short *, int64_t, int64_t, int64_t, const short *, int64_t, int64_t, int64_t, int, int, cudaStream_t);
 
 int ola_max_table_slices() { return kOlaMaxSlices; }
 int ola_max_table_frames() { return kOlaMaxFrames; }

@@ -158,10 +158,12 @@ int postchain_state_stride(const PostChain &pc);
 void launch_postchain_reset(const PostChain &pc, float *state, int rows, cudaStream_t st);
 void launch_postchain(const DevRows &g, const PostChain &pc, float *state, int64_t col0, int64_t col1, cudaStream_t st);
 
-// row-wise copy with independent pitches and any 4-byte alignment (live batch input placement)
-void launch_place_rows(float *dst, int64_t dst_pitch, const float *src, int64_t src_pitch, int width, int rows, cudaStream_t st);
-// the same with either side a ring of (mask + 1) floats per row starting at element `off` (mask = -1: a plain row)
-void launch_ring_rows(float *dst, int64_t dst_pitch, int64_t dst_off, int64_t dst_mask, const float *src, int64_t src_pitch, int64_t src_off, int64_t src_mask,
+// row-wise copy with independent pitches (in elements) and any element alignment (live batch input placement); T = float or short
+template <typename T>
+void launch_place_rows(T *dst, int64_t dst_pitch, const T *src, int64_t src_pitch, int width, int rows, cudaStream_t st);
+// the same with either side a ring of (mask + 1) elements per row starting at element `off` (mask = -1: a plain row)
+template <typename T>
+void launch_ring_rows(T *dst, int64_t dst_pitch, int64_t dst_off, int64_t dst_mask, const T *src, int64_t src_pitch, int64_t src_off, int64_t src_mask,
                       int width, int rows, cudaStream_t st);
 
 void launch_test_atan2f(int64_t n, const float *y, const float *x, float *out, cudaStream_t st);

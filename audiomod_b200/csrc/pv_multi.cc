@@ -338,6 +338,19 @@ void copy_nt(float *dst, const float *src, size_t n) {
     std::memcpy(dst, src, sizeof(float) * n);
 #endif
 }
+void copy_nt(int16_t *dst, const int16_t *src, size_t n) {
+#if defined(__x86_64__)
+    auto pair = [&](size_t i) { int v; std::memcpy(&v, src + i, sizeof v); _mm_stream_si32(reinterpret_cast<int *>(dst + i), v); };
+    size_t i = 0;
+    if (n && ((uintptr_t)dst & 2)) { dst[0] = src[0]; i = 1; }   // _mm_stream_si32 needs 4-byte alignment: one plain store first
+    for (; i + 2 <= n && ((uintptr_t)(dst + i) & 15); i += 2) pair(i);
+    for (; i + 8 <= n; i += 8) _mm_stream_si128(reinterpret_cast<__m128i *>(dst + i), _mm_loadu_si128(reinterpret_cast<const __m128i *>(src + i)));
+    for (; i + 2 <= n; i += 2) pair(i);
+    if (i < n) dst[i] = src[i];   // an odd last sample
+#else
+    std::memcpy(dst, src, sizeof(int16_t) * n);
+#endif
+}
 void copy_nt_fence() {
 #if defined(__x86_64__)
     _mm_sfence();

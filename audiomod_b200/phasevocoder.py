@@ -23,6 +23,7 @@ GENDER_CEPSTRAL, FORMANT_CEPSTRAL = 8, 9
 NORMAL_PV, PHASE_LOCKED, INT_RATIO = 0, 1, 2
 
 _fp = C.POINTER(C.c_float)
+_sp = C.POINTER(C.c_int16)
 
 
 def _cfg(sampleRate, numChannels, timeratio, pitchshift, mode, coremode, fftsize, hopsize, device) -> Config:
@@ -52,10 +53,10 @@ def plan_counts(n_in, sampleRate, numChannels, timeratio, pitchshift, mode=NORMA
     return dict(n_out=v[0].value, n_slices=v[1].value, n_dropped=v[2].value)
 
 
-def _chan_ptrs(a: np.ndarray):
-    """float** for the rows of a 2-D float32 array (vectorised: a live batch has thousands of rows per call)."""
+def _chan_ptrs(a: np.ndarray, elem=_fp):
+    """float** (int16_t** with elem=_sp) for the rows of a 2-D array (vectorised: a live batch has thousands of rows per call)."""
     ptrs = (np.uintp(a.ctypes.data) + np.arange(a.shape[0], dtype=np.uintp) * np.uintp(a.strides[0])).astype(np.uintp)
-    return ptrs.ctypes.data_as(C.POINTER(_fp))   # keeps a reference to `ptrs`
+    return ptrs.ctypes.data_as(C.POINTER(elem))   # keeps a reference to `ptrs`
 
 
 class phasevocoder:
@@ -63,11 +64,27 @@ class phasevocoder:
 
     streams > 1 makes it a live batch (pvgpu_create_multi): `streams` objects of one configuration advancing in lock-step,
     buffers [streams * numChannels, n] with row = stream * numChannels + channel; every call serves all of them with one set
-    of kernel launches, and every stream gets the samples its own object would."""
+    of kernel launches, and every stream gets the samples its own object would.
+
+    fmt=S16 makes every buffer int16 PCM (the pvgpu_*_s16 calls): processInData / processBlock take int16 arrays (other dtypes
+    are rejected, not cast), getOutData returns int16, and the *Device methods take int16 device rows with pointer offsets and
+    pitches in int16 elements.  The samples are those of a float32 object fed s / 32768 whose output is quantised the way the
+    reference's WAV writer does."""
 
     def __init__(self, sampleRate, numChannels, timeratio, pitchshift, mode=NORMAL_SHIFT, coremode=PHASE_LOCKED,
-                 fftsize=2048, hopsize=0, device=0, streams=1):
+                 fftsize=2048, hopsize=0, device=0, streams=1, fmt=_lib.F32):
         self._h = C.c_void_p()
+        if fmt not in (_lib.F32, _lib.S16):
+            raise ValueError(f"fmt must be F32 or S16, not {fmt!r}")
+        self.fmt = fmt
+        s16 = fmt == _lib.S16
+        L = _lib.lib()
+        self._dtype, self._elem = (np.int16, _sp) if s16 else (np.float32, _fp)
+        self._process, self._retrieve, self._block = ((L.pvgpu_process_s16, L.pvgpu_retrieve_s16, L.pvgpu_process_block_s16) if s16
+                                                      else (L.pvgpu_process, L.pvgpu_retrieve, L.pvgpu_process_block))
+        self._process_dev, self._retrieve_dev, self._block_dev = (
+            (L.pvgpu_process_device_s16, L.pvgpu_retrieve_device_s16, L.pvgpu_process_block_device_s16) if s16
+            else (L.pvgpu_process_device, L.pvgpu_retrieve_device, L.pvgpu_process_block_device))
         self.streams_ = int(streams)
         self.num_channels_ = int(numChannels) * self.streams_    # rows of every buffer
         self._ready = False
@@ -90,43 +107,50 @@ class phasevocoder:
     def getParams(self, params):
         pass
 
+    def _check_dtype(self, a) -> None:
+        if self.fmt == _lib.S16 and np.asarray(a).dtype != np.int16:
+            raise TypeError(f"this instance takes int16 rows, not {np.asarray(a).dtype}")
+
     def processInData(self, inData: np.ndarray, num_in_samples: int | None = None) -> None:
-        x = np.ascontiguousarray(inData, dtype=np.float32)
+        self._check_dtype(inData)
+        x = np.ascontiguousarray(inData, dtype=self._dtype)
         n = x.shape[1] if num_in_samples is None else int(num_in_samples)
-        check(_lib.lib().pvgpu_process(self._h, _chan_ptrs(x), n))
+        check(self._process(self._h, _chan_ptrs(x, self._elem), n))
 
     def getOutSamples(self) -> int:
         return _lib.lib().pvgpu_available(self._h)
 
     def getOutData(self, num_out_samples: int) -> np.ndarray:
-        out = np.zeros((self.num_channels_, max(int(num_out_samples), 1)), dtype=np.float32)
-        k = _lib.lib().pvgpu_retrieve(self._h, _chan_ptrs(out), int(num_out_samples))
+        out = np.zeros((self.num_channels_, max(int(num_out_samples), 1)), dtype=self._dtype)
+        k = self._retrieve(self._h, _chan_ptrs(out, self._elem), int(num_out_samples))
         if k < 0:
             check(-k)
         self._ready = True
         return out[:, :k]
 
     def processBlock(self, bufferData: np.ndarray, num_samples: int | None = None) -> None:
-        """In place on a C-contiguous float32 [numChannels, n] array."""
-        assert bufferData.dtype == np.float32 and bufferData.flags.c_contiguous
+        """In place on a C-contiguous float32 (fmt=S16: int16) [numChannels, n] array."""
+        self._check_dtype(bufferData)
+        assert bufferData.dtype == self._dtype and bufferData.flags.c_contiguous
         n = bufferData.shape[1] if num_samples is None else int(num_samples)
         ready = C.c_int(0)
-        check(_lib.lib().pvgpu_process_block(self._h, _chan_ptrs(bufferData), n, C.byref(ready)))
+        check(self._block(self._h, _chan_ptrs(bufferData, self._elem), n, C.byref(ready)))
         self._ready = bool(ready.value)
 
-    # ---- device rows: float32 device memory, row r at ptr + r * pitch floats; enqueued on cuda_stream, no call waits ----
+    # ---- device rows: float32 (fmt=S16: int16) device memory, row r at ptr + r * pitch elements; enqueued on cuda_stream, no
+    # call waits ----
     def processInDataDevice(self, d_ptr: int, pitch: int, n: int, cuda_stream: int = 0) -> None:
-        check(_lib.lib().pvgpu_process_device(self._h, C.c_void_p(d_ptr), int(pitch), int(n), C.c_void_p(cuda_stream)))
+        check(self._process_dev(self._h, C.c_void_p(d_ptr), int(pitch), int(n), C.c_void_p(cuda_stream)))
 
     def getOutDataDevice(self, d_ptr: int, pitch: int, n: int, cuda_stream: int = 0) -> int:
-        k = _lib.lib().pvgpu_retrieve_device(self._h, C.c_void_p(d_ptr), int(pitch), int(n), C.c_void_p(cuda_stream))
+        k = self._retrieve_dev(self._h, C.c_void_p(d_ptr), int(pitch), int(n), C.c_void_p(cuda_stream))
         if k < 0:
             check(-k)
         return k
 
     def processBlockDevice(self, d_ptr: int, pitch: int, n: int, cuda_stream: int = 0) -> None:
         ready = C.c_int(0)
-        check(_lib.lib().pvgpu_process_block_device(self._h, C.c_void_p(d_ptr), int(pitch), int(n), C.c_void_p(cuda_stream), C.byref(ready)))
+        check(self._block_dev(self._h, C.c_void_p(d_ptr), int(pitch), int(n), C.c_void_p(cuda_stream), C.byref(ready)))
         self._ready = bool(ready.value)
 
     def outputReady(self) -> bool:

@@ -97,6 +97,20 @@ int pvgpu_stream_count(const pvgpu_stream *s);
 int pvgpu_process_device(pvgpu_stream *s, const float *d_in, int64_t in_pitch, int n, void *cuda_stream);
 int pvgpu_retrieve_device(pvgpu_stream *s, float *d_out, int64_t out_pitch, int n, void *cuda_stream);   /* returns the count, < 0: -error */
 int pvgpu_process_block_device(pvgpu_stream *s, float *d_buf, int64_t pitch, int n, void *cuda_stream, int *ready);
+/* int16 twins of the streaming calls, for hosts that hold audio as 16-bit PCM: the same semantics, counts, *ready rule and
+ * stream ordering as the float32 call of the same name without _s16.  Every stream of an instance fed int16 rows produces
+ * exactly what a float32 instance produces with the same calls when its input is fed as (float)(s * (1.0/32768)) and every
+ * output sample is quantised as (short)(int)clamp(x * 32768.f, -32768, 32767), truncating toward zero -- the batch's PVGPU_S16
+ * rules (main/wavfile.cc:733-752, 1294-1306).  The samples stay int16 from the caller's rows to the device and back (half the
+ * bytes of float32 to pack and copy); the kernels convert as they load and quantise as they store.  Device pitches are in int16
+ * elements; device rows may start at any 2-byte boundary.  The first data call fixes an instance's rows: host or device,
+ * float32 or int16 -- a call of another kind returns PVGPU_ESTATE and its message names the call to use. */
+int pvgpu_process_s16(pvgpu_stream *s, const int16_t *const *in, int n);
+int pvgpu_retrieve_s16(pvgpu_stream *s, int16_t *const *out, int n);                 /* returns the count, < 0: -error */
+int pvgpu_process_block_s16(pvgpu_stream *s, int16_t *const *buf, int n, int *ready);
+int pvgpu_process_device_s16(pvgpu_stream *s, const int16_t *d_in, int64_t in_pitch, int n, void *cuda_stream);
+int pvgpu_retrieve_device_s16(pvgpu_stream *s, int16_t *d_out, int64_t out_pitch, int n, void *cuda_stream);   /* returns the count, < 0: -error */
+int pvgpu_process_block_device_s16(pvgpu_stream *s, int16_t *d_buf, int64_t pitch, int n, void *cuda_stream, int *ready);
 /* phasevocoder::~phasevocoder (phasevocoder.cc:62-67) */
 void pvgpu_destroy(pvgpu_stream *s);
 /* modbase_offline::processInData (modbase.h:89, phasevocoder.cc:87-108): consume n samples per channel */
@@ -236,8 +250,8 @@ int pvgpu_test_inverse_polar(int device, int fftsize, int n_frames, const float 
 int pvgpu_test_atan2f(int device, int64_t n, const float *y, const float *x, float *out);
 /* princarg (src/common/system/sys.h:84-91) */
 int pvgpu_test_princarg(int device, int64_t n, const double *a, double *out);
-/* host-only self-test of the live batch's containers (ring FIFO, row-copy pool, non-temporal copies): 0 = ok, else the number of
- * the failed check (negative: an error code).  Needs no device. */
+/* host-only self-test of the live batch's containers (ring FIFO, row-copy pool, non-temporal copies; float32 and int16 samples):
+ * 0 = ok, else the number of the failed check (negative: an error code).  Needs no device. */
 int pvgpu_test_host_structs(void);
 
 #ifdef __cplusplus
