@@ -1041,10 +1041,13 @@ int pvgpu_equalizer_chain(const float *paramlist, pvgpu_fx *chain, int *n_fx) {
     return PVGPU_OK;
 }
 
-int pvgpu_batch_set_postchain(pvgpu_batch *b, const pvgpu_fx *chain, int n_fx) {
-    if (!b || n_fx < 0 || n_fx > kMaxPostFx || (n_fx > 0 && !chain)) return fail(PVGPU_EINVAL, "bad post-chain (at most %d effects)", kMaxPostFx);
+}  // extern "C"
+
+// pvgpu_fx entries -> the coefficients the kernels run with, as the reference's constructors compute them at sample rate sr; the
+// conversion and the argument checks of pvgpu_batch_set_postchain and pvgpu_set_postchain.  *out is only written on success.
+static int make_postchain(int sr, const pvgpu_fx *chain, int n_fx, PostChain *out) {
+    if (n_fx < 0 || n_fx > kMaxPostFx || (n_fx > 0 && !chain)) return fail(PVGPU_EINVAL, "bad post-chain (at most %d effects)", kMaxPostFx);
     PostChain pc{};
-    const int sr = b->cfg.sample_rate;
     for (int i = 0; i < n_fx; ++i) {
         const pvgpu_fx &f = chain[i];
         PostFx &o = pc.fx[i];
@@ -1073,8 +1076,15 @@ int pvgpu_batch_set_postchain(pvgpu_batch *b, const pvgpu_fx *chain, int n_fx) {
         }
     }
     pc.n = n_fx;
-    b->pl.post = pc;
+    *out = pc;
     return PVGPU_OK;
+}
+
+extern "C" {
+
+int pvgpu_batch_set_postchain(pvgpu_batch *b, const pvgpu_fx *chain, int n_fx) {
+    if (!b) return fail(PVGPU_EINVAL, "bad post-chain (at most %d effects)", kMaxPostFx);
+    return make_postchain(b->cfg.sample_rate, chain, n_fx, &b->pl.post);
 }
 
 int pvgpu_batch_set_fused(pvgpu_batch *b, int enable) {
@@ -1489,6 +1499,31 @@ int pvgpu_test_princarg(int device, int64_t n, const double *a, double *out) {
     return PVGPU_OK;
 }
 
+int pvgpu_test_postchain(int device, int sample_rate, const pvgpu_fx *chain, int n_fx, int rows, int64_t n, float *samples) {
+    if (rows < 1 || n < 0 || (n > 0 && !samples) || sample_rate < 1) return fail(PVGPU_EINVAL, "bad argument");
+    PostChain pc{};
+    int rc = make_postchain(sample_rate, chain, n_fx, &pc);
+    if (rc) return rc;
+    if (n == 0) return PVGPU_OK;
+    int ndev = 0;
+    if (cudaGetDeviceCount(&ndev) != cudaSuccess || device < 0 || device >= ndev) return fail(PVGPU_ECUDA, "no CUDA device");
+    CU(cudaSetDevice(device));
+    const size_t bytes = sizeof(float) * (size_t)rows * n;
+    DevBuf d_x, d_n, d_state;
+    if ((rc = Pipeline::upload(d_x, samples, bytes))) return rc;
+    const std::vector<int64_t> lim((size_t)rows, n);
+    if ((rc = Pipeline::upload(d_n, lim.data(), sizeof(int64_t) * lim.size()))) return rc;
+    CU(d_state.ensure(sizeof(float) * (size_t)rows * postchain_state_stride(pc)));
+    DevRows g{};
+    g.rows = rows; g.channels = 1;
+    g.out = d_x.p; g.out_stride = n; g.out_base = 0; g.n_out = d_n.as<int64_t>();
+    launch_postchain_reset(pc, d_state.as<float>(), rows, nullptr);
+    launch_postchain(g, pc, d_state.as<float>(), 0, n, nullptr);   // the batch's launch, from fresh state
+    CU(cudaGetLastError());
+    CU(cudaMemcpy(samples, d_x.p, bytes, cudaMemcpyDeviceToHost));
+    return PVGPU_OK;
+}
+
 }  // extern "C"
 
 // ------------------------------------------------------------------------------------------------
@@ -1660,6 +1695,11 @@ struct pvgpu_stream {
     long tr_calls = 0;
     int num_res = 0;
     DevBuf d_out, d_car, d_len, d_stage;
+    // Post-chain (pvgpu_set_postchain): the effects are pl.post, their per-row state is ws.post_state ([R][postchain_state_stride]
+    // floats), reset on the stream of the first call that runs the chain after a set (post_fresh).  int16 rows with a chain: the
+    // resynthesis stores float32 into post_in ([R][out_stride]) and the chain quantises into d_out.
+    DevBuf post_in;
+    bool post_fresh = false;
     std::vector<float> h_stage, scratch;
     std::vector<unsigned char> h_pack;
     PinnedArena arena;
@@ -1785,13 +1825,17 @@ static int stream_run_new(pvgpu_stream *s, long k0, int added, const T *const *i
     if ((rc = pl.upload_schedule(sc, st))) return rc;
     if ((rc = pl.build_resample_runs(k0, k0 + added, pl.fused ? pl.fa.run : ola_run_limit(p, 8, pl.max_consumed, pl.max_out), st))) return rc;
     CU(s->d_out.ensure(sizeof(T) * (size_t)R * out_stride));
+    const bool chain = pl.post.n > 0;
+    const bool chain_s16 = chain && std::is_same<T, int16_t>::value;   // float32 staging between the resynthesis and the chain
+    if (chain_s16) CU(s->post_in.ensure(sizeof(float) * (size_t)R * out_stride));
     if (!pl.fused && halo_of(sc.recs(), sc.recs_base(), p.rs_active ? (int)p.rs_filt_len : 1) > s->ws.Fr - s->ws.F) return fail(PVGPU_ESTATE, "too many overlapping (dropped) slices; retrieve output more often");
     DevRows g{};
     g.rows = R; g.channels = C;
     g.in = d_in; g.in_stride = in_stride; g.in_base = s->in_base;
     g.fmt = std::is_same<T, int16_t>::value ? PVGPU_S16 : PVGPU_F32;   // int16: the kernels convert on load and quantise on store
     g.n_in = s->d_len.as<int64_t>(); g.n_out = s->d_len.as<int64_t>() + R;
-    g.out = s->d_out.as<T>(); g.out_stride = out_stride; g.out_base = out_base;
+    g.out = chain_s16 ? s->post_in.p : s->d_out.p; g.out_stride = out_stride; g.out_base = out_base;
+    g.out_f32 = chain_s16 ? 1 : 0;
     s->ws.bind(pl, g);
     g.aux_base = k0;
     if (pl.d.whisper) {   // whisperSlice draws rand() channel-major per slice (:814-822): the next added * C * H values of this instance's generator
@@ -1818,6 +1862,11 @@ static int stream_run_new(pvgpu_stream *s, long k0, int added, const T *const *i
     if (trace) cudaEventRecord(s->tr_ev[1], st);   // uploads done
     for (long k = k0; k < k0 + added; k += s->ws.F)
         if ((rc = pl.run_frames(g, k, (int)std::min<long>(s->ws.F, k0 + added - k), st))) return rc;
+    if (chain && new_out > 0) {   // every sample the call produced, once and in order, before it enters an output ring
+        if (s->post_fresh) { launch_postchain_reset(pl.post, s->ws.post_state.as<float>(), R, st); s->post_fresh = false; }
+        launch_postchain_stream(g, pl.post, s->ws.post_state.as<float>(), out_base, out_base + new_out, s->d_out.p, g.fmt, st);
+        ++pl.launches;
+    }
     CU(cudaGetLastError());
     if (trace) cudaEventRecord(s->tr_ev[2], st);   // kernels done
     if (new_out > 0 && dev) {   // device rows: append to the device-resident ring
@@ -2047,6 +2096,27 @@ int pvgpu_stream_info(const pvgpu_stream *s, pvgpu_info *info) {
     if (!s || !info) return fail(PVGPU_EINVAL, "null argument");
     fill_info(s->pl.d, info);
     return PVGPU_OK;
+}
+
+static int pvgpu_set_postchain_body(pvgpu_stream *s, const pvgpu_fx *chain, int n_fx) {
+    if (!s) return fail(PVGPU_EINVAL, "bad post-chain (at most %d effects)", kMaxPostFx);
+    PostChain pc{};
+    int rc = make_postchain(s->cfg.sample_rate, chain, n_fx, &pc);
+    if (rc) return rc;
+    if (!s->pl.d.valid_mode) return PVGPU_OK;   // an instance of an unknown mode produces nothing (phasevocoder.cc:104-106)
+    CU(cudaSetDevice(s->pl.device));
+    // Earlier calls' kernels may still use the effect state (device-row calls do not wait): host-row calls ran on s->st, every
+    // device-row call recorded the event of its staging arena after its kernels.
+    CU(cudaStreamSynchronize(s->st));
+    for (int i = 0; i < pvgpu_stream::kDevArenas; ++i)
+        if (s->dev_arena_used[i]) CU(cudaEventSynchronize(s->dev_arena_ev[i]));
+    if (pc.n > 0) CU(s->ws.post_state.ensure(sizeof(float) * (size_t)s->R() * postchain_state_stride(pc)));
+    s->pl.post = pc;
+    s->post_fresh = pc.n > 0;   // fresh effect state, reset on the stream of the next call that runs the chain
+    return PVGPU_OK;
+}
+int pvgpu_set_postchain(pvgpu_stream *s, const pvgpu_fx *chain, int n_fx) {
+    return guarded([&]() -> int { return pvgpu_set_postchain_body(s, chain, n_fx); });
 }
 
 }  // extern "C"

@@ -121,7 +121,7 @@ __global__ void __launch_bounds__(FusedShape<N>::kThreads, N <= 2048 ? 3 : 2) k_
                 if (e < rc.consumed) {
                     const float v = s / nrm[e];
                     if (rs) s_in[rel + e] = v;
-                    else if (e < n_store) pcm_store(g.out, g.fmt, row_out + rc.out_off + e, v);
+                    else if (e < n_store) pcm_store(g.out, out_fmt(g), row_out + rc.out_off + e, v);
                 }
             }
         }

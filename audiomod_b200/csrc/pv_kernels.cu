@@ -951,7 +951,7 @@ __global__ void __launch_bounds__(256, 4) k_ola_resample(const DevPlan p, const 
                     s_in[e] = v;
                 } else if (sl >= first_run_slice && e - r0 < T.n_store[sl]) {
                     // no resampling: the normalised sample is the output sample (n_write / n_out clip)
-                    pcm_store(g.out, g.fmt, row_out + out_first + T.out_rel[sl] + (e - r0), v);
+                    pcm_store(g.out, out_fmt(g), row_out + out_first + T.out_rel[sl] + (e - r0), v);
                 }
             }
         }

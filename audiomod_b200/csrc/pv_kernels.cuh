@@ -39,7 +39,9 @@ struct DevRows {
     int rows;                 // channel rows in this group (streams * channels)
     int channels;
     const void *in;           // [rows][in_stride] float32 or int16 PCM (fmt), element 0 is input sample in_base
-    int fmt;                  // 0: float32 rows, 1: int16 rows (input and output)
+    int fmt;                  // 0: float32 rows, 1: int16 rows (input, and output unless out_f32)
+    int out_f32;              // 1: the resynthesis stores float32 rows whatever fmt is (an int16 streaming instance whose post-chain
+                              //    quantises); 0: it stores fmt.  Read through out_fmt() (pv_synth.cuh)
     int64_t in_stride, in_base;
     const int64_t *n_in;      // per row: valid input samples (zeros beyond), global coordinates
     float *mag, *phase;       // [rows][F][Hp] spectra of the current frame chunk
@@ -157,6 +159,9 @@ struct PostChain { int n; PostFx fx[kMaxPostFx]; };
 int postchain_state_stride(const PostChain &pc);
 void launch_postchain_reset(const PostChain &pc, float *state, int rows, cudaStream_t st);
 void launch_postchain(const DevRows &g, const PostChain &pc, float *state, int64_t col0, int64_t col1, cudaStream_t st);
+// the streaming instances' launch: g.out holds float32 rows, the chained samples go to dst (indexed like g.out) as dst_fmt
+// (PVGPU_F32: dst == g.out, in place; PVGPU_S16: quantised like pcm_store)
+void launch_postchain_stream(const DevRows &g, const PostChain &pc, float *state, int64_t col0, int64_t col1, void *dst, int dst_fmt, cudaStream_t st);
 
 // row-wise copy with independent pitches (in elements) and any element alignment (live batch input placement); T = float or short
 template <typename T>

@@ -8,7 +8,11 @@
 // sample tiles through shared memory so that every global access is a coalesced 128-byte row segment.
 // Arithmetic follows the reference's types expression by expression (float members, the double literals where it has them,
 // no FMA contraction); log10f / pow are CUDA's, within an ulp or two of glibc's (tolerance path, like the resampler).
+#include <cstdlib>
+
+#include "../../include/pvgpu.h"
 #include "pv_kernels.cuh"
+#include "pv_synth.cuh"
 
 namespace pvgpu {
 
@@ -57,18 +61,23 @@ __device__ __forceinline__ float fx_limiter(float x, const PostFx &f, FxRegs &s,
     return y;
 }
 
-constexpr int kPostWarps = 4;
+constexpr int kPostWarps = 4;   // the batch's shape: 4 warps of 32 rows per CTA
 
-// Columns [col0, col1) of every row's output (float32 rows); state: [rows][state_stride] floats (4 x 4 scalars, then the delay lines).
-__global__ void __launch_bounds__(32 * kPostWarps) k_postchain(const DevRows g, const PostChain pc, float *__restrict__ state, int state_stride,
-                                                               int64_t col0, int64_t col1) {
-    __shared__ float tile[kPostWarps][32][33];
+// Columns [col0, col1) of every row's float32 output in g.out; state: [rows][state_stride] floats (4 x 4 scalars, then the delay
+// lines).  The chained samples go to dst, indexed like g.out ([rows][out_stride], element 0 is output position out_base): float32
+// (DST_S16 false; dst == g.out, in place) or int16 quantised by pcm_store's rule (DST_S16 true: a streaming instance of int16 rows,
+// whose resynthesis stored float32 into g.out).  WARPS warps of 32 rows each per CTA.  The one-warp shape may take all 255
+// registers (without the bound ptxas stopped at 128 and spilled); the batch's shape keeps the plain bound (168 registers).
+template <int WARPS, bool DST_S16>
+__global__ void __launch_bounds__(32 * WARPS, WARPS == 1 ? 8 : 0) k_postchain(const DevRows g, const PostChain pc, float *__restrict__ state, int state_stride,
+                                                          int64_t col0, int64_t col1, void *dst) {
+    __shared__ float tile[WARPS][32][33];
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int row_base = (blockIdx.x * kPostWarps + warp) * 32;
+    const int row_base = (blockIdx.x * WARPS + warp) * 32;
     if (row_base >= g.rows) return;
     const int row = row_base + lane;
     const bool have_row = row < g.rows;
-    float *out = (float *)g.out;
+    const float *out = (const float *)g.out;
     float *st = state + (int64_t)(have_row ? row : row_base) * state_stride;
     FxRegs regs[kMaxPostFx];
     float *rings[kMaxPostFx];
@@ -118,7 +127,11 @@ __global__ void __launch_bounds__(32 * kPostWarps) k_postchain(const DevRows g, 
         for (int r = 0; r < 32; ++r) {
             const int rr = row_base + r;
             const int64_t idx = c + lane;
-            if (rr < g.rows && idx < col1 && idx < g.n_out[rr]) out[(int64_t)rr * g.out_stride - g.out_base + idx] = tile[warp][r][lane];
+            if (rr < g.rows && idx < col1 && idx < g.n_out[rr]) {
+                const int64_t o = (int64_t)rr * g.out_stride - g.out_base + idx;
+                if (DST_S16) pcm_store(dst, PVGPU_S16, o, tile[warp][r][lane]);
+                else ((float *)dst)[o] = tile[warp][r][lane];
+            }
         }
         __syncwarp();
     }
@@ -154,7 +167,26 @@ void launch_postchain_reset(const PostChain &pc, float *state, int rows, cudaStr
 void launch_postchain(const DevRows &g, const PostChain &pc, float *state, int64_t col0, int64_t col1, cudaStream_t st) {
     if (pc.n == 0 || col1 <= col0) return;
     const int rows_per_cta = 32 * kPostWarps;
-    k_postchain<<<(g.rows + rows_per_cta - 1) / rows_per_cta, 32 * kPostWarps, 0, st>>>(g, pc, state, postchain_state_stride(pc), col0, col1);
+    k_postchain<kPostWarps, false><<<(g.rows + rows_per_cta - 1) / rows_per_cta, 32 * kPostWarps, 0, st>>>(g, pc, state, postchain_state_stride(pc), col0, col1, g.out);
+}
+
+// Streaming instances: a call's few hundred columns per row are walked serially by one thread per row, so the rows are spread
+// over as many SMs as possible -- one warp (32 rows) per CTA, 128 CTAs for 4096 rows instead of the batch's 32.  Measured faster
+// at both sizes (compressor + limiter: 0.91 against 1.08 ms per call at 1024 rows, 1.68 against 2.08 ms at 4096; B200,
+// profiles/r04_live_postchain_latency.jsonl), so there is one shape.  PVGPU_POST_WARPS=4 selects the batch's shape (read at every
+// launch, for that comparison).
+void launch_postchain_stream(const DevRows &g, const PostChain &pc, float *state, int64_t col0, int64_t col1, void *dst, int dst_fmt, cudaStream_t st) {
+    if (pc.n == 0 || col1 <= col0) return;
+    const char *v = std::getenv("PVGPU_POST_WARPS");
+    const int warps = v && v[0] == '4' ? 4 : 1;
+    const int stride = postchain_state_stride(pc), ctas = (g.rows + 32 * warps - 1) / (32 * warps);
+    if (warps == 4) {
+        if (dst_fmt == PVGPU_S16) k_postchain<4, true><<<ctas, 128, 0, st>>>(g, pc, state, stride, col0, col1, dst);
+        else k_postchain<4, false><<<ctas, 128, 0, st>>>(g, pc, state, stride, col0, col1, dst);
+    } else {
+        if (dst_fmt == PVGPU_S16) k_postchain<1, true><<<ctas, 32, 0, st>>>(g, pc, state, stride, col0, col1, dst);
+        else k_postchain<1, false><<<ctas, 32, 0, st>>>(g, pc, state, stride, col0, col1, dst);
+    }
 }
 
 }  // namespace pvgpu

@@ -49,7 +49,7 @@ __device__ __forceinline__ void resample_step(const DevPlan &p, const DevRows &g
             float sum = 0.f;
             const float *__restrict__ tt = p.rs_table + (size_t)__float_as_uint(__ldg(&frac_tab[first + lane + 32 * u])) * L;
             for (int j = 0; j < L; ++j) sum += xs[u][j] * __ldg(&tt[j]);
-            pcm_store(g.out, g.fmt, orow + (ent[u] & 0xffffu), sum);
+            pcm_store(g.out, out_fmt(g), orow + (ent[u] & 0xffffu), sum);
         }
         return;
     }
@@ -97,7 +97,7 @@ __device__ __forceinline__ void resample_step(const DevPlan &p, const DevRows &g
 #pragma unroll
     for (int u = 0; u < ROWS; ++u) {
         if (!live[u]) continue;
-        pcm_store(g.out, g.fmt, orow + (ent[u] & 0xffffu), (ic[u].x * acc[u][0].x) + (ic[u].y * acc[u][0].y) + (ic[u].z * acc[u][1].x) + (ic[u].w * acc[u][1].y));
+        pcm_store(g.out, out_fmt(g), orow + (ent[u] & 0xffffu), (ic[u].x * acc[u][0].x) + (ic[u].y * acc[u][0].y) + (ic[u].z * acc[u][1].x) + (ic[u].w * acc[u][1].y));
     }
 }
 

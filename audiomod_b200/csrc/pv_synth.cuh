@@ -23,6 +23,9 @@ __device__ __forceinline__ void pcm_store(void *base, int fmt, int64_t idx, floa
     }
 }
 
+// format of the samples the resynthesis stores into g.out
+__device__ __forceinline__ int out_fmt(const DevRows &g) { return g.out_f32 ? 0 : g.fmt; }
+
 // (magnitude, phase) -> packed bin of the polar pipelines and of the phase-free modes on Cartesian spectra
 struct SynthBinLoader {
     const DevPlan &p;

@@ -59,6 +59,17 @@ def _chan_ptrs(a: np.ndarray, elem=_fp):
     return ptrs.ctypes.data_as(C.POINTER(elem))   # keeps a reference to `ptrs`
 
 
+def _fx_array(chain):
+    """(pvgpu_fx array, count) of a chain spelled as (kind name, constructor arguments...) tuples."""
+    kinds = {"gain": _lib.FX_GAIN, "compressor": _lib.FX_COMPRESSOR, "limiter": _lib.FX_LIMITER, "biquad": _lib.FX_BIQUAD}
+    arr = (_lib.Fx * max(len(chain), 1))()
+    for i, fx in enumerate(chain):
+        arr[i].kind = kinds[fx[0]]
+        for j, v in enumerate(fx[1:]):
+            arr[i].p[j] = float(v)
+    return arr, len(chain)
+
+
 class phasevocoder:
     """One stream.  Buffers are planar float32 arrays of shape [numChannels, n].
 
@@ -161,6 +172,16 @@ class phasevocoder:
         check(_lib.lib().pvgpu_stream_info(self._h, C.byref(info)))
         return _info_dict(info)
 
+    def set_postchain(self, chain):
+        """FFT-free effects on everything this instance outputs, in order (pvgpu_set_postchain): the chains of
+        PhaseVocoderBatch.set_postchain, spelled the same way.  Every output sample goes through the chain once before it
+        enters the output ring, with each effect's state carried per row from call to call -- what the reference's effect objects
+        compute when fed everything getOutData returns.  A live batch applies the chain to every stream; fmt=S16 instances
+        quantise the chained float samples.  A new chain starts from fresh effect state at the next call; samples already
+        waiting in the ring keep their values.  An empty list clears the chain."""
+        arr, n = _fx_array(chain)
+        check(_lib.lib().pvgpu_set_postchain(self._h, arr, n))
+
 
 class PhaseVocoderBatch:
     """n_streams independent streams with one configuration (rows are channel-planar)."""
@@ -229,17 +250,13 @@ class PhaseVocoderBatch:
         return outs
 
     def set_postchain(self, chain):
-        """FFT-free effects applied to the float32 output rows, in order (pvgpu_batch_set_postchain): a list of
+        """FFT-free effects applied to the float32 output rows, in order (pvgpu_batch_set_postchain; phasevocoder.set_postchain
+        takes the same chains for streaming instances): a list of
         ("gain", g), ("compressor", dBThreshold, ratio, dBMakeUpGain, attackMs, releaseMs), ("limiter", dBThreshold, dBMakeUpGain,
         attackMs, releaseMs), ("biquad", type, cutoffFreq, q, dBGain) -- the reference objects' constructor arguments;
         equalizer_chain() expands the equalizer object into biquad entries.  An empty list clears the chain."""
-        kinds = {"gain": _lib.FX_GAIN, "compressor": _lib.FX_COMPRESSOR, "limiter": _lib.FX_LIMITER, "biquad": _lib.FX_BIQUAD}
-        arr = (_lib.Fx * max(len(chain), 1))()
-        for i, fx in enumerate(chain):
-            arr[i].kind = kinds[fx[0]]
-            for j, v in enumerate(fx[1:]):
-                arr[i].p[j] = float(v)
-        check(_lib.lib().pvgpu_batch_set_postchain(self._h, arr, len(chain)))
+        arr, n = _fx_array(chain)
+        check(_lib.lib().pvgpu_batch_set_postchain(self._h, arr, n))
 
     def set_fused(self, enable=True):
         """True: the fused inverse-FFT + overlap-add + resampler kernel; False: the split kernels; None: automatic (split unless the
@@ -383,7 +400,7 @@ def run_wav_files(pairs, timeratio=1.0, pitchshift=0.0, mode=NORMAL_SHIFT, corem
 
 def equalizer_chain(paramlist=None):
     """The reference's equalizer object (eight biquad sections, paramlist = [use, cutoff, Q, gain] x 8, None = its defaults)
-    as a list of ("biquad", type, cutoff, q, gain) entries for PhaseVocoderBatch.set_postchain."""
+    as a list of ("biquad", type, cutoff, q, gain) entries for PhaseVocoderBatch.set_postchain and phasevocoder.set_postchain."""
     arr = (_lib.Fx * 8)()
     n = C.c_int()
     pl = None

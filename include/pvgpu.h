@@ -111,6 +111,27 @@ int pvgpu_process_block_s16(pvgpu_stream *s, int16_t *const *buf, int n, int *re
 int pvgpu_process_device_s16(pvgpu_stream *s, const int16_t *d_in, int64_t in_pitch, int n, void *cuda_stream);
 int pvgpu_retrieve_device_s16(pvgpu_stream *s, int16_t *d_out, int64_t out_pitch, int n, void *cuda_stream);   /* returns the count, < 0: -error */
 int pvgpu_process_block_device_s16(pvgpu_stream *s, int16_t *d_buf, int64_t pitch, int n, void *cuda_stream, int *ready);
+/* Post-chain of FFT-free effects (gain, compressor, limiter, biquad sections; the kinds, parameters and limits of
+ * pvgpu_batch_set_postchain below, coefficients from cfg->sample_rate exactly as the batch computes them; at most 12 entries,
+ * pvgpu_equalizer_chain output works unchanged) on a streaming instance or live batch -- the reference's effect objects chained
+ * after the phase vocoder in SDK use (gain / compressor / limiter / equalizer after phasevocoder).
+ *   What it runs on: the instance's output stream.  Every sample the instance produces goes through the chain once, in order,
+ *   before it enters the output ring: the result is what the reference's effect objects compute when fed everything getOutData
+ *   returns, in order.  Each effect's state is carried per row from call to call, so call sizes and partial retrieves do not
+ *   change the result.  Sample counts, pvgpu_available and the *ready rule do not change; processBlock leaves the buffer
+ *   untouched while output is not ready, and input that passes through unprocessed never meets the chain.
+ *   Live batch: one chain serves all n_streams * channels rows; each stream gets what its own instance with the chain produces.
+ *   Setting, changing, clearing: before the first data call or between calls.  A new chain takes effect at the next data call
+ *   with fresh effect state, as if the effect objects had just been constructed; samples already in the output ring are not
+ *   touched; n_fx = 0 clears the chain and later output is the plain output again, bit for bit.  The phase vocoder's own state
+ *   is never touched.  Not a real-time call: it waits for the instance's outstanding device work.  Device-row calls enqueue the
+ *   chain on their stream and still do not wait.
+ *   int16 instances (*_s16): the chain runs on the float samples and its result is quantised by the int16 rule above, so each
+ *   stream equals quantise(float32 instance with the same chain fed s / 32768).
+ *   Errors: PVGPU_EINVAL for n_fx < 0 or > 12, a null chain with n_fx > 0, an unknown kind, a compressor ratio <= 0 (the
+ *   batch's messages).  On an instance whose mode does nothing (an unknown mode) it succeeds and changes nothing. */
+typedef struct pvgpu_fx pvgpu_fx;
+int pvgpu_set_postchain(pvgpu_stream *s, const pvgpu_fx *chain, int n_fx);
 /* phasevocoder::~phasevocoder (phasevocoder.cc:62-67) */
 void pvgpu_destroy(pvgpu_stream *s);
 /* modbase_offline::processInData (modbase.h:89, phasevocoder.cc:87-108): consume n samples per channel */
@@ -159,7 +180,7 @@ int pvgpu_batch_run_host(pvgpu_batch *b, const void *const *in_rows, void *const
  *                        (0 highPass, 1 lowShelf, 2 peaking, 3 notch, 4 highShelf, 5 lowPass, 6 / 7 band-pass, 8 allpass)
  * n_fx = 0 clears the chain; at most 12 effects.  Takes effect at the next run. */
 enum { PVGPU_FX_GAIN = 1, PVGPU_FX_COMPRESSOR = 2, PVGPU_FX_LIMITER = 3, PVGPU_FX_BIQUAD = 4 };
-typedef struct pvgpu_fx { int kind; float p[6]; } pvgpu_fx;
+struct pvgpu_fx { int kind; float p[6]; };   /* typedef above, at pvgpu_set_postchain */
 int pvgpu_batch_set_postchain(pvgpu_batch *b, const pvgpu_fx *chain, int n_fx);
 /* the equalizer object (src/equalizer/equalizer.cc: eight biquad sections in a fixed order, paramlist = {use, cutoff, Q, gain} x 8,
  * NULL = its defaults) expanded into PVGPU_FX_BIQUAD entries for pvgpu_batch_set_postchain; chain must hold 8 entries */
@@ -250,6 +271,9 @@ int pvgpu_test_inverse_polar(int device, int fftsize, int n_frames, const float 
 int pvgpu_test_atan2f(int device, int64_t n, const float *y, const float *x, float *out);
 /* princarg (src/common/system/sys.h:84-91) */
 int pvgpu_test_princarg(int device, int64_t n, const double *a, double *out);
+/* the post-chain once over [rows][n] float32 host samples, in place, from fresh effect state: the conversion and the kernel of
+ * pvgpu_batch_set_postchain / pvgpu_set_postchain at this sample rate (a bit-exact anchor for the streaming post-chain's tests) */
+int pvgpu_test_postchain(int device, int sample_rate, const pvgpu_fx *chain, int n_fx, int rows, int64_t n, float *samples);
 /* host-only self-test of the live batch's containers (ring FIFO, row-copy pool, non-temporal copies; float32 and int16 samples):
  * 0 = ok, else the number of the failed check (negative: an error code).  Needs no device. */
 int pvgpu_test_host_structs(void);
