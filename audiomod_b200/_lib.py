@@ -75,6 +75,7 @@ SYMBOLS = {
     "pvgpu_process_block": (C.c_int, [C.c_void_p, _fpp, C.c_int, C.POINTER(C.c_int)]),
     "pvgpu_stream_info": (C.c_int, [C.c_void_p, C.POINTER(Info)]),
     "pvgpu_set_postchain": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int]),
+    "pvgpu_set_stream_postchain": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_int]),
     "pvgpu_batch_create": (C.c_int, [C.POINTER(Config), C.c_int, C.c_int64, _vpp]),
     "pvgpu_batch_destroy": (None, [C.c_void_p]),
     "pvgpu_batch_plan": (C.c_int, [C.c_void_p, _i64p, C.c_int, _i64p]),

@@ -1700,6 +1700,18 @@ struct pvgpu_stream {
     // resynthesis stores float32 into post_in ([R][out_stride]) and the chain quantises into d_out.
     DevBuf post_in;
     bool post_fresh = false;
+    // Per-stream parameters of the chain (pvgpu_set_stream_postchain): post_coef is the host mirror [S][pl.post.n * 6] of every
+    // stream's coefficients (the p[] of pl.post.fx), d_post_coef the device table the per-row kernel reads.  post_differs[j]: stream
+    // j's coefficients are not pl.post's, post_n_differ counts them (> 0: the per-row kernel runs).  post_pending lists the streams
+    // whose mirror rows the next call that runs the chain uploads, once each (post_is_pending), as records of 1 + 6n floats
+    // (post_upd) scattered into the table from d_post_upd.  The setter of the chain sizes all of it.
+    std::vector<float> post_coef, post_upd;
+    std::vector<unsigned char> post_differs, post_is_pending;
+    std::vector<int> post_pending;
+    int post_n_differ = 0;
+    bool post_force_per_row = false;   // PVGPU_POST_PER_ROW=1 when the instance was created: the per-row kernel for every chain (to
+                                       // measure it against the uniform kernel on identical parameters)
+    DevBuf d_post_coef, d_post_upd;
     std::vector<float> h_stage, scratch;
     std::vector<unsigned char> h_pack;
     PinnedArena arena;
@@ -1767,7 +1779,8 @@ static int stream_run_new(pvgpu_stream *s, long k0, int added, const T *const *i
     {   // room for everything this call stages (nothing is in flight between calls)
         const size_t lists = p.rs_active ? (size_t)(new_out + 8 * 32 * ((added + 3) / 4 + 1) + 64) * 24 + (size_t)added * sizeof(ResampleRun) : 0;
         const size_t need = sizeof(float) * ((size_t)R * (pend + 16) + s->car_tail.size() + sc.norm().size()) + sizeof(SliceRec) * sc.recs().size() +
-                            lists + (pl.d.whisper ? sizeof(float) * (size_t)added * C * p.H : 0) + 64 * 16 + sizeof(int64_t) * (2 * R + 1);
+                            lists + (pl.d.whisper ? sizeof(float) * (size_t)added * C * p.H : 0) + 64 * 16 + sizeof(int64_t) * (2 * R + 1) +
+                            sizeof(float) * s->post_pending.size() * (1 + 6 * (size_t)pl.post.n);
         PinnedArena *ar = &s->arena;
         if (dev) {   // no call waits for the device: rotate the arenas, each is free again when the call that used it has run
             const unsigned i = s->dev_arena_i++ % pvgpu_stream::kDevArenas;
@@ -1864,7 +1877,24 @@ static int stream_run_new(pvgpu_stream *s, long k0, int added, const T *const *i
         if ((rc = pl.run_frames(g, k, (int)std::min<long>(s->ws.F, k0 + added - k), st))) return rc;
     if (chain && new_out > 0) {   // every sample the call produced, once and in order, before it enters an output ring
         if (s->post_fresh) { launch_postchain_reset(pl.post, s->ws.post_state.as<float>(), R, st); s->post_fresh = false; }
-        launch_postchain_stream(g, pl.post, s->ws.post_state.as<float>(), out_base, out_base + new_out, s->d_out.p, g.fmt, st);
+        if (!s->post_pending.empty()) {   // per-stream parameters set since the last such call: only their rows move
+            const size_t n6 = 6 * (size_t)pl.post.n, k = s->post_pending.size();
+            s->post_upd.resize(k * (1 + n6));
+            for (size_t i = 0; i < k; ++i) {
+                const int j = s->post_pending[i];
+                float *r = &s->post_upd[i * (1 + n6)];
+                std::memcpy(r, &j, sizeof(int));
+                std::memcpy(r + 1, &s->post_coef[(size_t)j * n6], sizeof(float) * n6);
+                s->post_is_pending[j] = 0;
+            }
+            s->post_pending.clear();
+            if ((rc = pl.h2d(s->d_post_upd.p, s->post_upd.data(), sizeof(float) * s->post_upd.size(), st))) return rc;
+            if (!pl.staged_all) { CU(cudaStreamSynchronize(st)); pl.staged_all = true; }   // post_upd is rewritten by the next call
+            launch_postchain_coef_scatter(s->d_post_upd.as<float>(), (int)k, (int)n6, s->d_post_coef.as<float>(), st);
+        }
+        const bool per_row = s->post_n_differ > 0 || s->post_force_per_row;   // the per-row kernel when some stream's coefficients are its own
+        launch_postchain_stream(g, pl.post, s->ws.post_state.as<float>(), out_base, out_base + new_out, s->d_out.p, g.fmt,
+                                per_row ? s->d_post_coef.as<float>() : nullptr, st);
         ++pl.launches;
     }
     CU(cudaGetLastError());
@@ -2057,6 +2087,10 @@ static int pvgpu_create_body(const pvgpu_config *cfg, int n_streams, pvgpu_strea
     if (!s) return fail(PVGPU_ENOMEM, "out of host memory");
     s->cfg = *cfg;
     s->S = n_streams;
+    {
+        const char *v = std::getenv("PVGPU_POST_PER_ROW");
+        s->post_force_per_row = v && v[0] == '1';
+    }
     if ((rc = s->pl.init(*cfg))) return rc;
     s->sched.reset(new Scheduler(s->pl.d, true));
     if (s->pl.d.vocoder) s->carrier.reset(new Carrier(cfg->sample_rate, cfg->mode == PVGPU_VOCODER_CHORD));
@@ -2110,13 +2144,68 @@ static int pvgpu_set_postchain_body(pvgpu_stream *s, const pvgpu_fx *chain, int 
     CU(cudaStreamSynchronize(s->st));
     for (int i = 0; i < pvgpu_stream::kDevArenas; ++i)
         if (s->dev_arena_used[i]) CU(cudaEventSynchronize(s->dev_arena_ev[i]));
-    if (pc.n > 0) CU(s->ws.post_state.ensure(sizeof(float) * (size_t)s->R() * postchain_state_stride(pc)));
+    const size_t S = (size_t)s->S, n6 = 6 * (size_t)pc.n;
+    if (pc.n > 0) {   // every stream starts with the chain's coefficients; the per-stream setter allocates nothing
+        CU(s->ws.post_state.ensure(sizeof(float) * (size_t)s->R() * postchain_state_stride(pc)));
+        CU(s->d_post_coef.ensure(sizeof(float) * S * n6));
+        CU(s->d_post_upd.ensure(sizeof(float) * S * (1 + n6)));
+        s->post_coef.resize(S * n6);
+        for (size_t j = 0; j < S; ++j)
+            for (int k = 0; k < pc.n; ++k) std::memcpy(&s->post_coef[(j * pc.n + k) * 6], pc.fx[k].p, sizeof(float) * 6);
+        CU(cudaMemcpy(s->d_post_coef.p, s->post_coef.data(), sizeof(float) * S * n6, cudaMemcpyHostToDevice));
+        s->post_upd.reserve(S * (1 + n6));
+        s->post_pending.reserve(S);
+    }
+    s->post_differs.assign(S, 0);
+    s->post_is_pending.assign(S, 0);
+    s->post_pending.clear();
+    s->post_n_differ = 0;
     s->pl.post = pc;
     s->post_fresh = pc.n > 0;   // fresh effect state, reset on the stream of the next call that runs the chain
     return PVGPU_OK;
 }
 int pvgpu_set_postchain(pvgpu_stream *s, const pvgpu_fx *chain, int n_fx) {
     return guarded([&]() -> int { return pvgpu_set_postchain_body(s, chain, n_fx); });
+}
+
+static const char *fx_name(int kind) {
+    switch (kind) {
+        case PVGPU_FX_GAIN: return "gain";
+        case PVGPU_FX_COMPRESSOR: return "compressor";
+        case PVGPU_FX_LIMITER: return "limiter";
+        case PVGPU_FX_BIQUAD: return "biquad";
+        default: return "unknown effect";
+    }
+}
+
+// Host arithmetic and bookkeeping only: no device work, no allocation (the setter of the chain sized everything).
+static int pvgpu_set_stream_postchain_body(pvgpu_stream *s, int stream, const pvgpu_fx *chain, int n_fx) {
+    if (!s) return fail(PVGPU_EINVAL, "null instance");
+    if (stream < 0 || stream >= s->S) return fail(PVGPU_EINVAL, "stream %d outside [0, %d)", stream, s->S);
+    if (!chain) return fail(PVGPU_EINVAL, "null chain");
+    PostChain pc{};
+    int rc = make_postchain(s->cfg.sample_rate, chain, n_fx, &pc);
+    if (rc) return rc;
+    if (!s->pl.d.valid_mode) return PVGPU_OK;   // an instance of an unknown mode produces nothing (phasevocoder.cc:104-106)
+    const PostChain &have = s->pl.post;
+    if (have.n == 0) return fail(PVGPU_EINVAL, "this instance has no post-chain (pvgpu_set_postchain first)");
+    if (pc.n != have.n) return fail(PVGPU_EINVAL, "chain of %d effects; this instance's chain has %d", pc.n, have.n);
+    for (int k = 0; k < pc.n; ++k)
+        if (pc.fx[k].kind != have.fx[k].kind)
+            return fail(PVGPU_EINVAL, "effect %d is a %s; this instance's effect %d is a %s", k, fx_name(pc.fx[k].kind), k, fx_name(have.fx[k].kind));
+    float *row = &s->post_coef[(size_t)stream * pc.n * 6];
+    bool differs = false;
+    for (int k = 0; k < pc.n; ++k) {
+        std::memcpy(row + 6 * k, pc.fx[k].p, sizeof(float) * 6);
+        differs = differs || std::memcmp(pc.fx[k].p, have.fx[k].p, sizeof(float) * 6) != 0;
+    }
+    s->post_n_differ += (int)differs - (int)s->post_differs[stream];
+    s->post_differs[stream] = differs;
+    if (!s->post_is_pending[stream]) { s->post_is_pending[stream] = 1; s->post_pending.push_back(stream); }
+    return PVGPU_OK;
+}
+int pvgpu_set_stream_postchain(pvgpu_stream *s, int stream, const pvgpu_fx *chain, int n_fx) {
+    return guarded([&]() -> int { return pvgpu_set_stream_postchain_body(s, stream, chain, n_fx); });
 }
 
 }  // extern "C"

@@ -160,8 +160,12 @@ int postchain_state_stride(const PostChain &pc);
 void launch_postchain_reset(const PostChain &pc, float *state, int rows, cudaStream_t st);
 void launch_postchain(const DevRows &g, const PostChain &pc, float *state, int64_t col0, int64_t col1, cudaStream_t st);
 // the streaming instances' launch: g.out holds float32 rows, the chained samples go to dst (indexed like g.out) as dst_fmt
-// (PVGPU_F32: dst == g.out, in place; PVGPU_S16: quantised like pcm_store)
-void launch_postchain_stream(const DevRows &g, const PostChain &pc, float *state, int64_t col0, int64_t col1, void *dst, int dst_fmt, cudaStream_t st);
+// (PVGPU_F32: dst == g.out, in place; PVGPU_S16: quantised like pcm_store); coef: null (pc's coefficients in every row) or
+// per-stream coefficients [streams][pc.n][6] (the p[] of pc.fx; row r is stream r / g.channels)
+void launch_postchain_stream(const DevRows &g, const PostChain &pc, float *state, int64_t col0, int64_t col1, void *dst, int dst_fmt, const float *coef,
+                             cudaStream_t st);
+// k records of 1 + n6 floats (stream index as int bits, then its n6 coefficients) into the rows of table ([streams][n6])
+void launch_postchain_coef_scatter(const float *upd, int k, int n6, float *table, cudaStream_t st);
 
 // row-wise copy with independent pitches (in elements) and any element alignment (live batch input placement); T = float or short
 template <typename T>

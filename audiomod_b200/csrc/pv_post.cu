@@ -68,15 +68,23 @@ constexpr int kPostWarps = 4;   // the batch's shape: 4 warps of 32 rows per CTA
 // (DST_S16 false; dst == g.out, in place) or int16 quantised by pcm_store's rule (DST_S16 true: a streaming instance of int16 rows,
 // whose resynthesis stored float32 into g.out).  WARPS warps of 32 rows each per CTA.  The one-warp shape may take all 255
 // registers (without the bound ptxas stopped at 128 and spilled); the batch's shape keeps the plain bound (168 registers).
-template <int WARPS, bool DST_S16>
+// PER_ROW: every stream has its own coefficients, coef = [streams][pc.n][6] floats (the p[] of pc.fx, row r is stream
+// r / g.channels); the kinds, delays and n stay pc's, so control flow is warp-uniform.  Each warp stages its rows' coefficients
+// in shared memory as [fx][param][lane] (one conflict-free access per lane and read); the uniform instantiations ignore coef.
+template <int WARPS, bool DST_S16, bool PER_ROW>
 __global__ void __launch_bounds__(32 * WARPS, WARPS == 1 ? 8 : 0) k_postchain(const DevRows g, const PostChain pc, float *__restrict__ state, int state_stride,
-                                                          int64_t col0, int64_t col1, void *dst) {
+                                                          int64_t col0, int64_t col1, void *dst, const float *__restrict__ coef) {
     __shared__ float tile[WARPS][32][33];
+    __shared__ float row_p[PER_ROW ? WARPS : 1][PER_ROW ? kMaxPostFx * 6 : 1][32];
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int row_base = (blockIdx.x * WARPS + warp) * 32;
     if (row_base >= g.rows) return;
     const int row = row_base + lane;
     const bool have_row = row < g.rows;
+    if (PER_ROW && have_row) {   // a lane without a row stages nothing and runs no sample
+        const float *c = coef + (int64_t)(row / g.channels) * pc.n * 6;
+        for (int i = 0; i < pc.n * 6; ++i) row_p[PER_ROW ? warp : 0][i][lane] = c[i];
+    }
     const float *out = (const float *)g.out;
     float *st = state + (int64_t)(have_row ? row : row_base) * state_stride;
     FxRegs regs[kMaxPostFx];
@@ -108,7 +116,13 @@ __global__ void __launch_bounds__(32 * WARPS, WARPS == 1 ? 8 : 0) k_postchain(co
 #pragma unroll
             for (int k = 0; k < kMaxPostFx; ++k) {
                 if (k >= pc.n) break;
-                const PostFx &f = pc.fx[k];
+                PostFx rf;   // PER_ROW: this row's coefficients of effect k
+                if (PER_ROW) {
+                    rf.kind = pc.fx[k].kind; rf.delay = pc.fx[k].delay;
+#pragma unroll
+                    for (int i = 0; i < 6; ++i) rf.p[i] = row_p[PER_ROW ? warp : 0][6 * k + i][lane];
+                }
+                const PostFx &f = PER_ROW ? rf : pc.fx[k];
                 if (f.kind == kFxGain) {
                     x = __fmul_rn(x, f.p[0]);
                     if (x > 1.f) x = 1.f;
@@ -167,26 +181,47 @@ void launch_postchain_reset(const PostChain &pc, float *state, int rows, cudaStr
 void launch_postchain(const DevRows &g, const PostChain &pc, float *state, int64_t col0, int64_t col1, cudaStream_t st) {
     if (pc.n == 0 || col1 <= col0) return;
     const int rows_per_cta = 32 * kPostWarps;
-    k_postchain<kPostWarps, false><<<(g.rows + rows_per_cta - 1) / rows_per_cta, 32 * kPostWarps, 0, st>>>(g, pc, state, postchain_state_stride(pc), col0, col1, g.out);
+    k_postchain<kPostWarps, false, false><<<(g.rows + rows_per_cta - 1) / rows_per_cta, 32 * kPostWarps, 0, st>>>(g, pc, state, postchain_state_stride(pc), col0, col1, g.out, nullptr);
 }
 
 // Streaming instances: a call's few hundred columns per row are walked serially by one thread per row, so the rows are spread
 // over as many SMs as possible -- one warp (32 rows) per CTA, 128 CTAs for 4096 rows instead of the batch's 32.  Measured faster
 // at both sizes (compressor + limiter: 0.91 against 1.08 ms per call at 1024 rows, 1.68 against 2.08 ms at 4096; B200,
-// profiles/r04_live_postchain_latency.jsonl), so there is one shape.  PVGPU_POST_WARPS=4 selects the batch's shape (read at every
-// launch, for that comparison).
-void launch_postchain_stream(const DevRows &g, const PostChain &pc, float *state, int64_t col0, int64_t col1, void *dst, int dst_fmt, cudaStream_t st) {
+// profiles/r04_live_postchain_latency.jsonl), so there is one shape.  PVGPU_POST_WARPS=4 selects the batch's shape for chains
+// whose coefficients are the same in every stream (read at every launch, for that comparison).  coef non-null: per-stream
+// coefficients (k_postchain<1, *, true>, one warp per CTA: four warps of staged coefficients would not fit 48 KB).  The engine
+// passes its table when some stream's parameters differ from the chain's, or always with PVGPU_POST_PER_ROW=1 (pv_engine.cu; for
+// measuring the two kernels on identical parameters).
+void launch_postchain_stream(const DevRows &g, const PostChain &pc, float *state, int64_t col0, int64_t col1, void *dst, int dst_fmt, const float *coef,
+                             cudaStream_t st) {
     if (pc.n == 0 || col1 <= col0) return;
     const char *v = std::getenv("PVGPU_POST_WARPS");
-    const int warps = v && v[0] == '4' ? 4 : 1;
+    const int warps = !coef && v && v[0] == '4' ? 4 : 1;
     const int stride = postchain_state_stride(pc), ctas = (g.rows + 32 * warps - 1) / (32 * warps);
-    if (warps == 4) {
-        if (dst_fmt == PVGPU_S16) k_postchain<4, true><<<ctas, 128, 0, st>>>(g, pc, state, stride, col0, col1, dst);
-        else k_postchain<4, false><<<ctas, 128, 0, st>>>(g, pc, state, stride, col0, col1, dst);
+    if (coef) {
+        if (dst_fmt == PVGPU_S16) k_postchain<1, true, true><<<ctas, 32, 0, st>>>(g, pc, state, stride, col0, col1, dst, coef);
+        else k_postchain<1, false, true><<<ctas, 32, 0, st>>>(g, pc, state, stride, col0, col1, dst, coef);
+    } else if (warps == 4) {
+        if (dst_fmt == PVGPU_S16) k_postchain<4, true, false><<<ctas, 128, 0, st>>>(g, pc, state, stride, col0, col1, dst, nullptr);
+        else k_postchain<4, false, false><<<ctas, 128, 0, st>>>(g, pc, state, stride, col0, col1, dst, nullptr);
     } else {
-        if (dst_fmt == PVGPU_S16) k_postchain<1, true><<<ctas, 32, 0, st>>>(g, pc, state, stride, col0, col1, dst);
-        else k_postchain<1, false><<<ctas, 32, 0, st>>>(g, pc, state, stride, col0, col1, dst);
+        if (dst_fmt == PVGPU_S16) k_postchain<1, true, false><<<ctas, 32, 0, st>>>(g, pc, state, stride, col0, col1, dst, nullptr);
+        else k_postchain<1, false, false><<<ctas, 32, 0, st>>>(g, pc, state, stride, col0, col1, dst, nullptr);
     }
+}
+
+// Pending per-stream coefficient updates into the [streams][n6] table: upd holds k records of 1 + n6 floats, the stream index
+// (int bits) and then its coefficients.  One thread per coefficient.
+__global__ void k_postchain_coef_scatter(const float *__restrict__ upd, int k, int n6, float *__restrict__ table) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= k * n6) return;
+    const float *r = upd + (int64_t)(i / n6) * (1 + n6);
+    table[(int64_t)__float_as_int(r[0]) * n6 + i % n6] = r[1 + i % n6];
+}
+
+void launch_postchain_coef_scatter(const float *upd, int k, int n6, float *table, cudaStream_t st) {
+    if (k <= 0 || n6 <= 0) return;
+    k_postchain_coef_scatter<<<(k * n6 + 255) / 256, 256, 0, st>>>(upd, k, n6, table);
 }
 
 }  // namespace pvgpu

@@ -182,6 +182,13 @@ class phasevocoder:
         arr, n = _fx_array(chain)
         check(_lib.lib().pvgpu_set_postchain(self._h, arr, n))
 
+    def set_stream_postchain(self, stream, chain):
+        """Parameters of one stream's chain (pvgpu_set_stream_postchain), spelled as in set_postchain: the same number and kinds of
+        effects as the instance's chain, other arguments.  Output produced by later calls uses them; the stream's effect state
+        carries over and other streams are untouched.  No device work: safe between real-time calls."""
+        arr, n = _fx_array(chain)
+        check(_lib.lib().pvgpu_set_stream_postchain(self._h, int(stream), arr, n))
+
 
 class PhaseVocoderBatch:
     """n_streams independent streams with one configuration (rows are channel-planar)."""

@@ -132,6 +132,29 @@ int pvgpu_process_block_device_s16(pvgpu_stream *s, int16_t *d_buf, int64_t pitc
  *   batch's messages).  On an instance whose mode does nothing (an unknown mode) it succeeds and changes nothing. */
 typedef struct pvgpu_fx pvgpu_fx;
 int pvgpu_set_postchain(pvgpu_stream *s, const pvgpu_fx *chain, int n_fx);
+/* Parameters of one stream's post-chain on a streaming instance or live batch (each user's level, EQ preset or limiter ceiling
+ * on a voice server, changed while they talk).
+ *   What it changes: the parameters of the chain pvgpu_set_postchain gave the instance, for one stream (all of its channel rows).
+ *   n_fx and the kind in every position must equal the instance's chain; the parameters are the same constructor arguments,
+ *   converted the same way at cfg->sample_rate.  Other streams are not touched, bit for bit.
+ *   When it takes effect: every output sample produced by a data call after this one uses the new parameters, every sample
+ *   produced earlier used the old ones; samples already in the output ring (host or device) keep their values.
+ *   State is kept: the stream's effect state carries over (biquad x1, x2, y1, y2; the compressor's level; the limiter's peak,
+ *   gain, delay line and position) and the new coefficients apply from the next sample on, as if the effect objects'
+ *   coefficient members had been recomputed in place.  The limiter's delay length depends only on the sample rate.
+ *   Real-time safe: no device work, never waits for the device, allocates nothing.  It converts one chain on the host and records
+ *   the change; the next data call that runs the chain uploads the pending changes on that call's stream (host rows: the
+ *   instance's stream; device rows: the caller's stream) before the chain runs.  Several updates between two calls coalesce;
+ *   the last one for a stream wins.
+ *   pvgpu_set_postchain is unchanged: it sets the kinds and gives every stream the same parameters with fresh state, discarding
+ *   earlier per-stream parameters.  pvgpu_set_stream_postchain right after it, before the next data call, gives that stream its
+ *   own parameters with fresh state -- per-user presets are one pvgpu_set_postchain, then one call per stream.
+ *   A pvgpu_create instance is a live batch of one: stream 0.
+ *   Errors (PVGPU_EINVAL, the instance unchanged): stream outside [0, n_streams); no chain on the instance; n_fx other than the
+ *   instance's; a kind other than the instance's in some position (the message names the position and both kinds); a null
+ *   chain; the argument errors of pvgpu_set_postchain (a compressor ratio <= 0, ...).  On an instance whose mode does nothing
+ *   (an unknown mode) it succeeds and changes nothing. */
+int pvgpu_set_stream_postchain(pvgpu_stream *s, int stream, const pvgpu_fx *chain, int n_fx);
 /* phasevocoder::~phasevocoder (phasevocoder.cc:62-67) */
 void pvgpu_destroy(pvgpu_stream *s);
 /* modbase_offline::processInData (modbase.h:89, phasevocoder.cc:87-108): consume n samples per channel */
