@@ -76,6 +76,10 @@ SYMBOLS = {
     "pvgpu_stream_info": (C.c_int, [C.c_void_p, C.POINTER(Info)]),
     "pvgpu_set_postchain": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int]),
     "pvgpu_set_stream_postchain": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_int]),
+    "pvgpu_set_meters": (C.c_int, [C.c_void_p, C.c_int]),
+    "pvgpu_get_meters": (C.c_int, [C.c_void_p, _fp, _fp, _fp, _i64p]),
+    "pvgpu_get_meters_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, _i64p]),
+    "pvgpu_kweighting_design": (C.c_int, [C.c_int, C.POINTER(C.c_double)]),
     "pvgpu_batch_create": (C.c_int, [C.POINTER(Config), C.c_int, C.c_int64, _vpp]),
     "pvgpu_batch_destroy": (None, [C.c_void_p]),
     "pvgpu_batch_plan": (C.c_int, [C.c_void_p, _i64p, C.c_int, _i64p]),
@@ -109,6 +113,7 @@ SYMBOLS = {
     "pvgpu_test_atan2f": (C.c_int, [C.c_int, C.c_int64, _fp, _fp, _fp]),
     "pvgpu_test_princarg": (C.c_int, [C.c_int, C.c_int64, C.POINTER(C.c_double), C.POINTER(C.c_double)]),
     "pvgpu_test_postchain": (C.c_int, [C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_int64, _fp]),
+    "pvgpu_test_loudness": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int, C.c_int64, C.c_int, _fp, _fp, _fp, _fp]),
     "pvgpu_test_host_structs": (C.c_int, []),
 }
 

@@ -1524,6 +1524,45 @@ int pvgpu_test_postchain(int device, int sample_rate, const pvgpu_fx *chain, int
     return PVGPU_OK;
 }
 
+int pvgpu_kweighting_design(int sample_rate, double *coeffs) {
+    if (sample_rate <= 0 || !coeffs) return fail(PVGPU_EINVAL, "bad argument (sample_rate > 0, non-null coeffs)");
+    kweighting_design(sample_rate, coeffs);
+    return PVGPU_OK;
+}
+
+int pvgpu_test_loudness(int device, int sample_rate, int channels, int streams, int64_t n, int call, const float *samples, float *momentary,
+                        float *short_term, float *peak) {
+    if (sample_rate < 1 || channels < 1 || streams < 1 || (int64_t)channels * streams > 65535 || n < 0 || call < 1 || (n > 0 && !samples) ||
+        !momentary || !short_term || !peak)
+        return fail(PVGPU_EINVAL, "bad argument");
+    int ndev = 0;
+    if (cudaGetDeviceCount(&ndev) != cudaSuccess || device < 0 || device >= ndev) return fail(PVGPU_ECUDA, "no CUDA device");
+    CU(cudaSetDevice(device));
+    const size_t R = (size_t)streams * channels, S = (size_t)streams;
+    std::vector<float> out(2 * S + R, 0.f);
+    std::fill(out.begin(), out.begin() + 2 * S, -INFINITY);
+    DevBuf d_x, d_state, d_ring, d_out;
+    int rc;
+    if (n > 0 && (rc = Pipeline::upload(d_x, samples, sizeof(float) * R * n))) return rc;
+    if ((rc = Pipeline::upload(d_out, out.data(), sizeof(float) * out.size()))) return rc;
+    CU(d_state.ensure(sizeof(double) * kMeterState * R));
+    CU(d_ring.ensure(sizeof(double) * kMeterRing * R));
+    CU(cudaMemset(d_state.p, 0, sizeof(double) * kMeterState * R));
+    CU(cudaMemset(d_ring.p, 0, sizeof(double) * kMeterRing * R));
+    KWeighting kw{};
+    kweighting_design(sample_rate, kw.c);
+    int pos = 0, ri = 0;
+    for (int64_t c0 = 0; c0 < n; c0 += call)   // the engine's launch, one piece after the other
+        launch_meters(d_x.as<float>() + c0, PVGPU_F32, n, (int)std::min<int64_t>(call, n - c0), streams, channels, kw, (sample_rate + 5) / 10,
+                      d_state.as<double>(), d_ring.as<double>(), d_out.as<float>(), &pos, &ri, nullptr);
+    CU(cudaGetLastError());
+    CU(cudaMemcpy(out.data(), d_out.p, sizeof(float) * out.size(), cudaMemcpyDeviceToHost));
+    std::memcpy(momentary, out.data(), sizeof(float) * S);
+    std::memcpy(short_term, out.data() + S, sizeof(float) * S);
+    std::memcpy(peak, out.data() + 2 * S, sizeof(float) * R);
+    return PVGPU_OK;
+}
+
 }  // extern "C"
 
 // ------------------------------------------------------------------------------------------------
@@ -1712,6 +1751,16 @@ struct pvgpu_stream {
     bool post_force_per_row = false;   // PVGPU_POST_PER_ROW=1 when the instance was created: the per-row kernel for every chain (to
                                        // measure it against the uniform kernel on identical parameters)
     DevBuf d_post_coef, d_post_upd;
+    // Loudness meters (pvgpu_set_meters): K-weighting state [kMeterState][R] and sub-block energies [kMeterRing][R] in doubles,
+    // results d_meter = [momentary S][short-term S][peak R] floats.  Host rows: every producing call copies d_meter back with its
+    // output, through the arena, into meter_host.  The rows advance in lock-step, so one set of counters serves them all: samples
+    // measured, samples in the open sub-block of meter_L, ring slot of the next completed sub-block.
+    bool meters = false;
+    KWeighting kw{};
+    int meter_L = 0, meter_pos = 0, meter_ri = 0;
+    int64_t measured = 0;
+    DevBuf d_meter_state, d_meter_ring, d_meter;
+    std::vector<float> meter_host;
     std::vector<float> h_stage, scratch;
     std::vector<unsigned char> h_pack;
     PinnedArena arena;
@@ -1780,7 +1829,8 @@ static int stream_run_new(pvgpu_stream *s, long k0, int added, const T *const *i
         const size_t lists = p.rs_active ? (size_t)(new_out + 8 * 32 * ((added + 3) / 4 + 1) + 64) * 24 + (size_t)added * sizeof(ResampleRun) : 0;
         const size_t need = sizeof(float) * ((size_t)R * (pend + 16) + s->car_tail.size() + sc.norm().size()) + sizeof(SliceRec) * sc.recs().size() +
                             lists + (pl.d.whisper ? sizeof(float) * (size_t)added * C * p.H : 0) + 64 * 16 + sizeof(int64_t) * (2 * R + 1) +
-                            sizeof(float) * s->post_pending.size() * (1 + 6 * (size_t)pl.post.n);
+                            sizeof(float) * s->post_pending.size() * (1 + 6 * (size_t)pl.post.n) +
+                            (s->meters && !dev ? sizeof(float) * s->meter_host.size() + 64 : 0);
         PinnedArena *ar = &s->arena;
         if (dev) {   // no call waits for the device: rotate the arenas, each is free again when the call that used it has run
             const unsigned i = s->dev_arena_i++ % pvgpu_stream::kDevArenas;
@@ -1897,6 +1947,17 @@ static int stream_run_new(pvgpu_stream *s, long k0, int added, const T *const *i
                                 per_row ? s->d_post_coef.as<float>() : nullptr, st);
         ++pl.launches;
     }
+    float *meter_pin = nullptr;
+    if (s->meters && new_out > 0) {   // the delivered samples, after the chain and before either ring
+        launch_meters(s->d_out.p, g.fmt, out_stride, (int)new_out, s->S, C, s->kw, s->meter_L, s->d_meter_state.as<double>(),
+                      s->d_meter_ring.as<double>(), s->d_meter.as<float>(), &s->meter_pos, &s->meter_ri, st);
+        s->measured += new_out;
+        if (!dev) {   // back with the output; without page-locked memory straight into the mirror
+            const size_t bytes = sizeof(float) * s->meter_host.size();
+            meter_pin = (float *)s->arena.take(bytes);
+            CU(cudaMemcpyAsync(meter_pin ? (void *)meter_pin : (void *)s->meter_host.data(), s->d_meter.p, bytes, cudaMemcpyDeviceToHost, st));
+        }
+    }
     CU(cudaGetLastError());
     if (trace) cudaEventRecord(s->tr_ev[2], st);   // kernels done
     if (new_out > 0 && dev) {   // device rows: append to the device-resident ring
@@ -1948,6 +2009,7 @@ static int stream_run_new(pvgpu_stream *s, long k0, int added, const T *const *i
     if (trace) for (int i = 0; i < 4; ++i) { float ms = 0; cudaEventElapsedTime(&ms, s->tr_ev[i], s->tr_ev[i + 1]); s->tr_dev[i] += 1e3 * ms; }
     if (trace && pend > 0) { float ms = 0; cudaEventElapsedTime(&ms, s->tr_ev[0], s->tr_ev[5]); s->tr_dev2[0] += 1e3 * ms; cudaEventElapsedTime(&ms, s->tr_ev[5], s->tr_ev[6]); s->tr_dev2[1] += 1e3 * ms; }
     pl.staged_all = true;
+    if (meter_pin) std::memcpy(s->meter_host.data(), meter_pin, sizeof(float) * s->meter_host.size());
     if (new_out > 0 && !dev) host_fifo<T>(s).commit((size_t)new_out);
     s->pend_len = 0;
     s->dev_len = keep;
@@ -2132,18 +2194,23 @@ int pvgpu_stream_info(const pvgpu_stream *s, pvgpu_info *info) {
     return PVGPU_OK;
 }
 
+// Earlier calls' kernels may still use the instance's device state (device-row calls do not wait): host-row calls ran on s->st,
+// every device-row call recorded the event of its staging arena after its kernels.
+static int stream_wait_idle(pvgpu_stream *s) {
+    CU(cudaSetDevice(s->pl.device));
+    CU(cudaStreamSynchronize(s->st));
+    for (int i = 0; i < pvgpu_stream::kDevArenas; ++i)
+        if (s->dev_arena_used[i]) CU(cudaEventSynchronize(s->dev_arena_ev[i]));
+    return PVGPU_OK;
+}
+
 static int pvgpu_set_postchain_body(pvgpu_stream *s, const pvgpu_fx *chain, int n_fx) {
     if (!s) return fail(PVGPU_EINVAL, "bad post-chain (at most %d effects)", kMaxPostFx);
     PostChain pc{};
     int rc = make_postchain(s->cfg.sample_rate, chain, n_fx, &pc);
     if (rc) return rc;
     if (!s->pl.d.valid_mode) return PVGPU_OK;   // an instance of an unknown mode produces nothing (phasevocoder.cc:104-106)
-    CU(cudaSetDevice(s->pl.device));
-    // Earlier calls' kernels may still use the effect state (device-row calls do not wait): host-row calls ran on s->st, every
-    // device-row call recorded the event of its staging arena after its kernels.
-    CU(cudaStreamSynchronize(s->st));
-    for (int i = 0; i < pvgpu_stream::kDevArenas; ++i)
-        if (s->dev_arena_used[i]) CU(cudaEventSynchronize(s->dev_arena_ev[i]));
+    if ((rc = stream_wait_idle(s))) return rc;
     const size_t S = (size_t)s->S, n6 = 6 * (size_t)pc.n;
     if (pc.n > 0) {   // every stream starts with the chain's coefficients; the per-stream setter allocates nothing
         CU(s->ws.post_state.ensure(sizeof(float) * (size_t)s->R() * postchain_state_stride(pc)));
@@ -2380,6 +2447,65 @@ int pvgpu_process_block_device(pvgpu_stream *s, float *d_buf, int64_t pitch, int
 }
 int pvgpu_process_block_device_s16(pvgpu_stream *s, int16_t *d_buf, int64_t pitch, int n, void *cuda_stream, int *ready) {
     return process_block_device<int16_t>(s, d_buf, pitch, n, cuda_stream, ready);
+}
+
+static int pvgpu_set_meters_body(pvgpu_stream *s, int enable) {
+    if (!s || (enable != 0 && enable != 1)) return fail(PVGPU_EINVAL, "bad argument (enable is 0 or 1)");
+    int rc;
+    if ((rc = stream_wait_idle(s))) return rc;   // earlier calls' kernels may still read or write the meter state
+    s->meters = false;
+    if (!enable) return PVGPU_OK;
+    const size_t R = (size_t)s->R(), S = (size_t)s->S;
+    CU(s->d_meter_state.ensure(sizeof(double) * kMeterState * R));
+    CU(s->d_meter_ring.ensure(sizeof(double) * kMeterRing * R));   // sub-blocks before the first measured sample are silence
+    CU(s->d_meter.ensure(sizeof(float) * (2 * S + R)));
+    s->meter_host.assign(2 * S + R, 0.f);
+    std::fill(s->meter_host.begin(), s->meter_host.begin() + 2 * S, -INFINITY);
+    CU(cudaMemsetAsync(s->d_meter_state.p, 0, sizeof(double) * kMeterState * R, s->st));
+    CU(cudaMemsetAsync(s->d_meter_ring.p, 0, sizeof(double) * kMeterRing * R, s->st));
+    CU(cudaMemcpyAsync(s->d_meter.p, s->meter_host.data(), sizeof(float) * s->meter_host.size(), cudaMemcpyHostToDevice, s->st));
+    CU(cudaStreamSynchronize(s->st));   // device-row calls run on the caller's stream: the fresh state must be in place first
+    kweighting_design(s->cfg.sample_rate, s->kw.c);
+    s->meter_L = (s->cfg.sample_rate + 5) / 10;
+    s->meter_pos = s->meter_ri = 0;
+    s->measured = 0;
+    s->meters = true;
+    return PVGPU_OK;
+}
+int pvgpu_set_meters(pvgpu_stream *s, int enable) {
+    return guarded([&]() -> int { return pvgpu_set_meters_body(s, enable); });
+}
+
+// A getter of the other kind of rows is refused with the name of the one to use; before the first data call either works.
+static int check_meters(const pvgpu_stream *s, bool device_getter) {
+    if (!s->meters) return fail(PVGPU_ESTATE, "meters are off on this instance (pvgpu_set_meters)");
+    if (s->io_mode && s->dev_rows() != device_getter)
+        return fail(PVGPU_ESTATE, "this instance is fed %s rows; use %s", kRowKind[s->io_mode], s->dev_rows() ? "pvgpu_get_meters_device" : "pvgpu_get_meters");
+    return PVGPU_OK;
+}
+
+int pvgpu_get_meters(const pvgpu_stream *s, float *momentary, float *short_term, float *peak, int64_t *measured) {
+    if (!s) return fail(PVGPU_EINVAL, "null instance");
+    int rc;
+    if ((rc = check_meters(s, false))) return rc;
+    const size_t S = (size_t)s->S;
+    const float *h = s->meter_host.data();
+    if (momentary) std::memcpy(momentary, h, sizeof(float) * S);
+    if (short_term) std::memcpy(short_term, h + S, sizeof(float) * S);
+    if (peak) std::memcpy(peak, h + 2 * S, sizeof(float) * (size_t)s->R());
+    if (measured) *measured = s->measured;
+    return PVGPU_OK;
+}
+
+int pvgpu_get_meters_device(pvgpu_stream *s, float *d_dst, void *cuda_stream, int64_t *measured) {
+    if (!s || !d_dst) return fail(PVGPU_EINVAL, "null argument");
+    int rc;
+    if ((rc = check_meters(s, true))) return rc;
+    CU(cudaSetDevice(s->pl.device));
+    CU(cudaMemcpyAsync(d_dst, s->d_meter.p, sizeof(float) * s->meter_host.size(), cudaMemcpyDeviceToDevice,
+                       cuda_stream ? (cudaStream_t)cuda_stream : cudaStreamLegacy));
+    if (measured) *measured = s->measured;
+    return PVGPU_OK;
 }
 
 }  // extern "C"

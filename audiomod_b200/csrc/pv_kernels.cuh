@@ -167,6 +167,18 @@ void launch_postchain_stream(const DevRows &g, const PostChain &pc, float *state
 // k records of 1 + n6 floats (stream index as int bits, then its n6 coefficients) into the rows of table ([streams][n6])
 void launch_postchain_coef_scatter(const float *upd, int k, int n6, float *table, cudaStream_t st);
 
+// ---- loudness meters on the output rows of streaming instances (pv_meter.cu) ----
+constexpr int kMeterRing = 30;    // sub-blocks of the short-term window, the longest one kept
+constexpr int kMeterState = 9;    // doubles per row: shelf x1 x2 y1 y2, high-pass x1 x2 y1 y2, energy of the open sub-block
+struct KWeighting { double c[7]; };   // shelf b0, b1, b2, a1, a2; high-pass a1, a2 (b = 1, -2, 1); a0 = 1
+void kweighting_design(int sample_rate, double *c /*[7]*/);
+// Meters over columns [0, n) of rows = streams * channels rows of x (row r at x + r * pitch, float32 or int16 by fmt): the K-weighting
+// state [kMeterState][rows] and the ring of sub-block energies [kMeterRing][rows] advance; out = [momentary S][short-term S][peak R]
+// floats: the peaks are rewritten, the loudness values only when a sub-block completes.  *pos (samples in the open sub-block of L)
+// and *ri (ring slot of the next completed sub-block) are the host's counters, advanced here.
+void launch_meters(const void *x, int fmt, int64_t pitch, int n, int streams, int channels, const KWeighting &kw, int L, double *state,
+                   double *ring, float *out, int *pos, int *ri, cudaStream_t st);
+
 // row-wise copy with independent pitches (in elements) and any element alignment (live batch input placement); T = float or short
 template <typename T>
 void launch_place_rows(T *dst, int64_t dst_pitch, const T *src, int64_t src_pitch, int width, int rows, cudaStream_t st);

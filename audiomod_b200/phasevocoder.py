@@ -189,6 +189,28 @@ class phasevocoder:
         arr, n = _fx_array(chain)
         check(_lib.lib().pvgpu_set_stream_postchain(self._h, int(stream), arr, n))
 
+    def set_meters(self, enable=True):
+        """Loudness meters on everything this instance outputs, after the post-chain (pvgpu_set_meters): BS.1770-4 momentary
+        (400 ms) and short-term (3 s) loudness per stream, ungated, and the sample peak per row.  True starts from fresh state
+        (also when already on); False stops them.  Waits for the device: not for the real-time thread."""
+        check(_lib.lib().pvgpu_set_meters(self._h, int(bool(enable))))
+
+    def meters(self) -> dict:
+        """Host rows: {"momentary": float32 [streams], "short_term": float32 [streams], "peak": float32 [streams, channels],
+        "measured": samples per row measured}, as of the last call (pvgpu_get_meters: no device work)."""
+        S, ch = self.streams_, self.num_channels_ // self.streams_
+        m, s, p = np.empty(S, np.float32), np.empty(S, np.float32), np.empty((S, ch), np.float32)
+        n = C.c_int64()
+        check(_lib.lib().pvgpu_get_meters(self._h, m.ctypes.data_as(_fp), s.ctypes.data_as(_fp), p.ctypes.data_as(_fp), C.byref(n)))
+        return {"momentary": m, "short_term": s, "peak": p, "measured": n.value}
+
+    def metersDevice(self, d_ptr: int, cuda_stream: int = 0) -> int:
+        """Device rows: enqueue the copy of [momentary S][short-term S][peak S * channels] float32 to d_ptr on cuda_stream
+        (pvgpu_get_meters_device, no wait); returns the samples per row measured."""
+        n = C.c_int64()
+        check(_lib.lib().pvgpu_get_meters_device(self._h, C.c_void_p(d_ptr), C.c_void_p(cuda_stream), C.byref(n)))
+        return n.value
+
 
 class PhaseVocoderBatch:
     """n_streams independent streams with one configuration (rows are channel-planar)."""
@@ -421,3 +443,11 @@ def biquad_design(type, sample_rate, cutoff, q, db_gain):
     c = (C.c_float * 6)()
     check(_lib.lib().pvgpu_biquad_design(int(type), int(sample_rate), float(cutoff), float(q), float(db_gain), c))
     return [c[i] for i in range(6)]
+
+
+def kweighting_design(sample_rate) -> np.ndarray:
+    """The meters' K-weighting at this sample rate (pvgpu_kweighting_design, needs no GPU): float64 [shelf b0, b1, b2, a1, a2,
+    high-pass a1, a2]; the high-pass has b = (1, -2, 1), both sections a0 = 1."""
+    c = np.zeros(7, np.float64)
+    check(_lib.lib().pvgpu_kweighting_design(int(sample_rate), c.ctypes.data_as(C.POINTER(C.c_double))))
+    return c

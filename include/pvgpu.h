@@ -155,6 +155,47 @@ int pvgpu_set_postchain(pvgpu_stream *s, const pvgpu_fx *chain, int n_fx);
  *   chain; the argument errors of pvgpu_set_postchain (a compressor ratio <= 0, ...).  On an instance whose mode does nothing
  *   (an unknown mode) it succeeds and changes nothing. */
 int pvgpu_set_stream_postchain(pvgpu_stream *s, int stream, const pvgpu_fx *chain, int n_fx);
+/* Loudness meters on a streaming instance or live batch (ITU-R BS.1770-4 / EBU Tech 3341 momentary and short-term loudness,
+ * sample peak).  Not the reference's loudnessmeter object: specified by the published standard, and nothing here restates
+ * src/meter/loudnessmeter.cc.  Per stream: momentary and short-term loudness in LUFS; per row (stream * channels + channel): peak.
+ *   What is measured: every sample the instance produces, once, in order, after the post-chain -- the chain's rule: input that
+ *   passes through unprocessed is not measured.  float32 rows as the float value; int16 rows as delivered, s / 32768 in double.
+ *   K-weighting: two direct-form-I biquad sections per row, shelf then high-pass, in double precision, each evaluated as
+ *   b0*x + b1*x1 + b2*x2 - a1*y1 - a2*y2 from left to right with every product and sum rounded on its own (__dmul_rn /
+ *   __dadd_rn / __dsub_rn, no contraction); the state carries from call to call.  Coefficients: pvgpu_kweighting_design.
+ *   Windows: sub-blocks of L = (sample_rate + 5) / 10 samples (integer division) counted from the first measured sample; a row's
+ *   sub-block energy is the sum of z^2 in double, in sample order; a stream's loudness over the last W sub-blocks is
+ *   -0.691 + 10 log10(sum over channels of sum over sub-blocks of E / (W * L)), summed over the sub-blocks oldest to newest, then over
+ *   the channels in order.  Momentary: W = 4 (400 ms); short-term: W = 30 (3 s).  No gating, every channel weighs 1.0; sub-blocks
+ *   before the first measured sample count as silence; zero energy gives -inf.  Both values are updated at the end of every data
+ *   call from the sub-blocks completed so far, and a call that completes no sub-block leaves them unchanged, so call sizes never
+ *   change the values at equal `measured`.
+ *   peak: the sample peak (not true peak), max |x| per row over the samples the most recent call that produced output produced.
+ *   measured: samples per row measured since the meters were enabled.
+ *   pvgpu_set_meters: before the first data call or between calls.  Not a real-time call: it allocates and waits for the
+ *   instance's outstanding device work.  enable = 1 starts from fresh meter state (momentary and short-term -inf, peaks 0,
+ *   measured 0), also when the meters were on already; enable = 0 stops every meter launch and copy, and the getters return
+ *   PVGPU_ESTATE.  Meters never change output samples, counts, *ready or anything else.  On an instance whose mode does nothing
+ *   (an unknown mode) it succeeds and nothing is ever measured.
+ *   pvgpu_get_meters (host rows): reads a host mirror -- no device work, never waits, allocates nothing: real-time safe.  The
+ *   values came back with the data call's own output copy, before its one synchronisation.  Any pointer may be NULL.
+ *   pvgpu_get_meters_device (device rows): enqueues one device-to-device cudaMemcpyAsync of [2*S + S*C] floats (momentary S,
+ *   short-term S, peak S*C) to d_dst on cuda_stream (NULL = the legacy default stream) and does not wait; it is ordered after the
+ *   calls enqueued before it on that stream (use one stream for all calls of an instance).
+ *   Before the first data call either getter works; afterwards the getter of the other kind of rows returns PVGPU_ESTATE and its
+ *   message names the getter to use.  Errors: PVGPU_EINVAL for a null instance or d_dst, enable other than 0 or 1; PVGPU_ESTATE
+ *   when the meters are off. */
+int pvgpu_set_meters(pvgpu_stream *s, int enable);
+int pvgpu_get_meters(const pvgpu_stream *s, float *momentary /*[S] or NULL*/, float *short_term /*[S] or NULL*/,
+                     float *peak /*[S*C] or NULL*/, int64_t *measured /*or NULL*/);
+int pvgpu_get_meters_device(pvgpu_stream *s, float *d_dst /*[2*S + S*C]: momentary, short-term, peak*/, void *cuda_stream,
+                            int64_t *measured /*or NULL*/);
+/* K-weighting at this sample rate, needs no GPU: {shelf b0, b1, b2, a1, a2, high-pass a1, a2} (high-pass b = {1, -2, 1}, a0 = 1).
+ * libebur128's analog-prototype formulas restated in double: shelf f0 = 1681.974450955533, G = 3.999843853973347,
+ * Q = 0.7071752369554196, K = tan(pi f0 / sr), Vh = 10^(G/20), Vb = Vh^0.4996667741545416, a0 = 1 + K/Q + K^2,
+ * b = {(Vh + Vb K/Q + K^2)/a0, 2(K^2 - Vh)/a0, (Vh - Vb K/Q + K^2)/a0}, a1 = 2(K^2 - 1)/a0, a2 = (1 - K/Q + K^2)/a0; high-pass
+ * f0 = 38.13547087602444, Q = 0.5003270373238773, the same a1 and a2.  At 48 kHz: BS.1770-4's tables.  sample_rate <= 0: PVGPU_EINVAL. */
+int pvgpu_kweighting_design(int sample_rate, double *coeffs /*[7]*/);
 /* phasevocoder::~phasevocoder (phasevocoder.cc:62-67) */
 void pvgpu_destroy(pvgpu_stream *s);
 /* modbase_offline::processInData (modbase.h:89, phasevocoder.cc:87-108): consume n samples per channel */
@@ -297,6 +338,10 @@ int pvgpu_test_princarg(int device, int64_t n, const double *a, double *out);
 /* the post-chain once over [rows][n] float32 host samples, in place, from fresh effect state: the conversion and the kernel of
  * pvgpu_batch_set_postchain / pvgpu_set_postchain at this sample rate (a bit-exact anchor for the streaming post-chain's tests) */
 int pvgpu_test_postchain(int device, int sample_rate, const pvgpu_fx *chain, int n_fx, int rows, int64_t n, float *samples);
+/* the meter kernels of pvgpu_set_meters over [streams*channels][n] float32 host samples from fresh state, fed in pieces of `call`
+ * samples; momentary / short_term [streams], peak [streams*channels] (over the last piece) */
+int pvgpu_test_loudness(int device, int sample_rate, int channels, int streams, int64_t n, int call, const float *samples,
+                        float *momentary, float *short_term, float *peak);
 /* host-only self-test of the live batch's containers (ring FIFO, row-copy pool, non-temporal copies; float32 and int16 samples):
  * 0 = ok, else the number of the failed check (negative: an error code).  Needs no device. */
 int pvgpu_test_host_structs(void);
