@@ -152,7 +152,6 @@ struct Pipeline {
     // unless the schedule overlaps more frames / history slices than their per-CTA tables hold, then the fused kernel, which
     // has no such limit), 0 split only, 1 fused wherever the FFT size has one.  PVGPU_FUSED=0/1 overrides for every instance.
     int fused_pref = -1;
-    bool ola_ws = false;   // pvgpu_batch_set_fused(b, 2): k_ola_resample_ws (pv_ola_ws.cu) instead of k_ola_resample; PVGPU_OLA_WS=1 for every instance
     PostChain post{};           // FFT-free effects applied to the output columns a chunk completes (pv_post.cu); n == 0: none
     FusedArgs fa{};             // run / ring / window shape; per-launch fields are filled in run_synth_ola
     // host copy of the uploaded records + the resampler work lists built from them (ResampleRun, pv_kernels.cuh)
@@ -446,9 +445,8 @@ struct Pipeline {
                     // 1.60 / 1.27 / 1.13 for pools of 128 / 256 / 512 entries; ncu measured 1.32 at 256).  The stores of a row are
                     // scattered either way (same-phase outputs are ~8 samples apart) and merge in L2.
                     constexpr int kWin = 2048;
-                    static const int win_env = []() { const char *v = getenv("PVGPU_RS_WIN"); int w = v ? atoi(v) : kWin; return w < 32 ? 32 : (w > kWin ? kWin : (w / 32) * 32); }();
-                    for (size_t b0 = 0; b0 < e.size(); b0 += win_env) {
-                        const int n = (int)std::min<size_t>(win_env, e.size() - b0), nrow = (n + 31) / 32;
+                    for (size_t b0 = 0; b0 < e.size(); b0 += kWin) {
+                        const int n = (int)std::min<size_t>(kWin, e.size() - b0), nrow = (n + 31) / 32;
                         static thread_local int rows[kWin / 32][32], spill[kWin];
                         int cnt[kWin / 32] = {}, nspill = 0;
                         int seen[32] = {};   // the r-th entry of a bank goes to row r
@@ -579,9 +577,7 @@ struct Pipeline {
         if (pref == 0 || (pref < 0 && split_ok)) return false;
         if (fused_frames_in_flight(p.N) == 0) return false;
         FusedArgs a{};
-        const char *fr = std::getenv("PVGPU_FUSED_RUN");
-        const char *ws = std::getenv("PVGPU_FUSED_WS");
-        if (!fused_plan(p, frames_per_chunk, max_shift, max_shift, max_out_bound, (size_t)200 * 1024, fr ? std::atoi(fr) : 0, ws && ws[0] == '1', &a)) return false;
+        if (!fused_plan(p, frames_per_chunk, max_shift, max_shift, max_out_bound, (size_t)200 * 1024, &a)) return false;
         fa = a;
         fused = true;
         return true;
@@ -601,13 +597,8 @@ struct Pipeline {
     void run_ola(const DevRows &g, long k0, int nf, cudaStream_t st) {
         const SliceRec *recs = b_recs.as<SliceRec>();
         Span *sp = span_begin(3, st);
-        static const bool ws_env = []() { const char *v = std::getenv("PVGPU_OLA_WS"); return v && v[0] == '1'; }();
-        cudaError_t werr = cudaSuccess;
-        if (!((ws_env || ola_ws) && launch_ola_resample_ws(p, g, recs, b_norm.as<float>(), norm_base, recs_base, k0, nf, table_run, max_consumed, b_runs.as<ResampleRun>(),
-                                               b_rsent.as<unsigned>(), b_rsfrac.as<float>(), b_rssteps.as<unsigned>(), run_origin, st, &werr)))
-            launch_ola_resample(p, g, recs, b_norm.as<float>(), norm_base, recs_base, k0, nf, table_run, max_consumed, b_runs.as<ResampleRun>(),
-                                b_rsent.as<unsigned>(), b_rsfrac.as<float>(), b_rssteps.as<unsigned>(), run_origin, st);
-        (void)werr;   // a failed launch surfaces at the next synchronisation (sticky error), like every other kernel's
+        launch_ola_resample(p, g, recs, b_norm.as<float>(), norm_base, recs_base, k0, nf, table_run, max_consumed, b_runs.as<ResampleRun>(),
+                            b_rsent.as<unsigned>(), b_rsfrac.as<float>(), b_rssteps.as<unsigned>(), run_origin, st);
         span_end(sp, st); ++launches;
     }
     int run_frames(const DevRows &g, long k0, int nf, cudaStream_t st) {
@@ -796,7 +787,6 @@ struct pvgpu_batch {
         const int hist_all = hist_slices_of(pl.h_recs, pl.p.rs_active ? (int)pl.p.rs_filt_len : 1);
         const bool split_ok = hist_all + 2 <= ola_max_table_slices() - 1 && halo + 1 <= 90;
         pl.plan_fused(frames_per_chunk, pl.max_consumed, pl.max_out, split_ok);   // fused kernel (and its shape) or the split kernels
-        if (const char *v = getenv("PVGPU_OLA_RUN")) { const int r = atoi(v); if (r >= 1 && r <= 32) pl.ola_run = r; }   // tuning experiments
         if (!pl.fused) {   // k_ola_resample's per-CTA tables: frames overlapping a run, slices holding the resampler history before it
             const int hist = hist_slices_of(pl.h_recs, pl.p.rs_active ? (int)pl.p.rs_filt_len : 1);
             if (hist + 2 > ola_max_table_slices() - 1)
@@ -1090,7 +1080,6 @@ int pvgpu_batch_set_postchain(pvgpu_batch *b, const pvgpu_fx *chain, int n_fx) {
 int pvgpu_batch_set_fused(pvgpu_batch *b, int enable) {
     if (!b) return fail(PVGPU_EINVAL, "null batch");
     b->pl.fused_pref = enable < 0 ? -1 : (enable == 1 ? 1 : 0);
-    b->pl.ola_ws = enable == 2;   // split kernels with the warp-specialised overlap-add + resampler
     b->run_for_chunk = 0;   // re-plan the launches at the next run
     return PVGPU_OK;
 }

@@ -187,12 +187,12 @@ static size_t fused_smem(const DevPlan &p, const FusedArgs &a) {
     const bool quad = p.rs_active && !p.rs_direct;
     const int NC = p.N / 2, padded = NC + NC / 16 + NC / 256 + 2;
     const int G = fused_frames_in_flight(p.N);
-    return (quad ? sizeof(float4) * (size_t)p.rs_table_len : 0) + sizeof(float) * ((size_t)a.in_len * (a.ws ? 2 : 1) + a.acc_len) + sizeof(float2) * (size_t)G * padded;
+    return (quad ? sizeof(float4) * (size_t)p.rs_table_len : 0) + sizeof(float) * ((size_t)a.in_len + a.acc_len) + sizeof(float2) * (size_t)G * padded;
 }
 
 // Shape of the fused kernel for a schedule: frames per run (a multiple of the frames in flight that divides
 // frames_per_chunk), ring length, resampler window.  Returns false when no run length fits the shared-memory budget.
-bool fused_plan(const DevPlan &p, int frames_per_chunk, int max_shift, int max_consumed, int max_out, size_t smem_limit, int force_run, bool want_ws, FusedArgs *out) {
+bool fused_plan(const DevPlan &p, int frames_per_chunk, int max_shift, int max_consumed, int max_out, size_t smem_limit, FusedArgs *out) {
     const int G = fused_frames_in_flight(p.N);
     if (G == 0) return false;
     const int L = p.rs_active ? (int)p.rs_filt_len : 0;
@@ -203,10 +203,8 @@ bool fused_plan(const DevPlan &p, int frames_per_chunk, int max_shift, int max_c
     // padding of the resampler's work lists, shorter ones keep the ring small
     for (int run = G; run <= 64; run += G) {
         if (frames_per_chunk % run) continue;
-        if (force_run > 0 && run != force_run) continue;   // PVGPU_FUSED_RUN: tuning experiments
         FusedArgs a{};
         a.run = run;
-        a.ws = (want_ws && p.rs_active) ? 1 : 0;   // the warp-specialised kernel needs a resampler for its second role
         a.hist_len = p.rs_active ? L + 8 : 0;
         a.acc_len = pow2_at_least(p.N + (run - 1) * max_shift);
         a.in_len = p.rs_active ? ((a.hist_len + run * max_consumed + 8 + 3) & ~3) : 4;
@@ -214,9 +212,9 @@ bool fused_plan(const DevPlan &p, int frames_per_chunk, int max_shift, int max_c
         if (p.rs_active && (run * max_consumed + L + 8 + kResPad >= 65536 || run * max_out >= 65535)) break;
         const size_t sm = fused_smem(p, a);
         if (sm > smem_limit) break;
-        const int target = a.ws ? (p.N <= 2048 ? 2 : 1) : (p.N <= 2048 ? 3 : 2);   // resident CTAs per SM the launch bounds aim for
+        const int target = p.N <= 2048 ? 3 : 2;   // resident CTAs per SM the launch bounds aim for
         const size_t per_cta = ((size_t)227 * 1024) / target - 1024;
-        if (found && sm > per_cta && force_run <= 0) break;     // do not trade a resident CTA for a longer run
+        if (found && sm > per_cta) break;     // do not trade a resident CTA for a longer run
         best = a;
         found = true;
     }
@@ -227,17 +225,14 @@ bool fused_plan(const DevPlan &p, int frames_per_chunk, int max_shift, int max_c
 template <int N, int kPre, bool kOV8>
 static cudaError_t launch_one(const DevPlan &p, const DevRows &g, const FusedArgs &a, cudaStream_t st) {
     const size_t sm = fused_smem(p, a);
-    static bool configured[16][2] = {};   // per device and kernel: shared-memory opt-in done
+    static bool configured[16] = {};   // per device: shared-memory opt-in done
     int dev = 0;
     cudaGetDevice(&dev);
-    if (dev < 16 && !configured[dev][a.ws]) {
-        if (!a.ws) {
-            cudaError_t e = cudaFuncSetAttribute(k_synth_ola<N, kPre, kOV8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(200 * 1024));
-            if (e != cudaSuccess) return e;
-        }
-        configured[dev][a.ws] = true;
+    if (dev < 16 && !configured[dev]) {
+        cudaError_t e = cudaFuncSetAttribute(k_synth_ola<N, kPre, kOV8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(200 * 1024));
+        if (e != cudaSuccess) return e;
+        configured[dev] = true;
     }
-    if (a.ws) return launch_synth_ola_ws(p, g, a, kPre, kOV8, sm, st);   // pv_fused_ws.cu
     k_synth_ola<N, kPre, kOV8><<<g.rows, FusedShape<N>::kThreads, sm, st>>>(p, g, a);
     return cudaSuccess;
 }

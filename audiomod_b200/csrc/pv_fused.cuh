@@ -1,4 +1,4 @@
-// Pieces shared by the fused resynthesis kernels (pv_fused.cu: k_synth_ola; pv_fused_ws.cu: k_synth_ola_ws).
+// Pieces of the fused resynthesis kernel (pv_fused.cu: k_synth_ola).
 #pragma once
 #include "pv_fft.cuh"
 #include "pv_kernels.cuh"
@@ -49,8 +49,5 @@ __device__ __forceinline__ void fused_add_frame(const float2 (&v)[16], float *s_
         }
     }
 }
-
-// the warp-specialised variant lives in its own translation unit (compile time); pre = 0 / 1 / 2 as k_synth_ola's kPre
-cudaError_t launch_synth_ola_ws(const DevPlan &p, const DevRows &g, const FusedArgs &a, int pre, bool ov8, size_t smem, cudaStream_t st);
 
 }  // namespace pvgpu

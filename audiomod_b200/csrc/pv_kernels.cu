@@ -18,7 +18,6 @@
 // contracts into FMAs, in the reference's operation order.  The synthesis side (inverse FFT, OLA,
 // resampler) is held to the 1e-4 / 90 dB tolerance and may use FMA.
 #include <algorithm>
-#include <cstdlib>
 
 #include "pv_kernels.cuh"
 #include "pv_fft.cuh"
@@ -117,11 +116,7 @@ __global__ void k_analyse(const DevPlan p, const DevRows g, long k0) {
 // k_analyse_t<N>: register-tiled version for N = 512..8192 (pv_fft.cuh).  T = N/32 threads own a frame; a CTA of
 // max(T, 256) threads handles 256/T consecutive frames of the chunk.
 // ------------------------------------------------------------------------------------------------
-// kBulk (float32 rows only; PVGPU_ANALYSE_BULK=1, an A/B experiment for the north_star's "TMA-staged frame tiles"): the frame's
-// N input samples arrive through one cp.async.bulk (SASS UBLKCP) into the frame's exchange buffer -- 16-byte aligned start,
-// up to 12 bytes over-fetched on either side -- signalled on an mbarrier, and the threads pick their sample pairs from shared
-// memory instead of issuing 16 global loads each.
-template <int N, bool kS16, bool kCart, bool kBulk = false>
+template <int N, bool kS16, bool kCart>
 __global__ void __launch_bounds__((N / 32 > 256 ? N / 32 : 256)) k_analyse_t(const DevPlan p, const DevRows g, long k0, int nf, int total) {
     constexpr int NC = N / 2;
     using S = FftShape<NC>;
@@ -133,38 +128,6 @@ __global__ void __launch_bounds__((N / 32 > 256 ? N / 32 : 256)) k_analyse_t(con
     const int fid = blockIdx.x * G + group;
     const bool active = fid < total;   // whole groups are active or not, so group barriers stay consistent
     const int row = active ? fid / nf : 0, f = active ? fid % nf : 0;
-    float bx0[kBulk ? 16 : 1], bx1[kBulk ? 16 : 1];
-    bool bulk_done = false;
-    if (kBulk) {
-        // one mbarrier per frame group, behind the exchange buffers
-        uint64_t *mbar = (uint64_t *)(sbuf + G * S::kPadded) + group;
-        const unsigned mb = (unsigned)__cvta_generic_to_shared(mbar);
-        if (t == 0) {
-            asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(mb));
-            asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-        }
-        frame_sync<T>(group);
-        const int64_t start = (int64_t)(k0 + f) * p.hop;
-        const int64_t left = active ? g.n_in[row] - start : 0;
-        if (active && left >= N) {   // whole frame inside the stream (the common case); others take the per-sample path below
-            const float *src = (const float *)g.in + (int64_t)row * g.in_stride + (start - g.in_base);
-            const uintptr_t a0 = reinterpret_cast<uintptr_t>(src) & ~(uintptr_t)15;
-            const int lead = (int)((reinterpret_cast<uintptr_t>(src) - a0) >> 2);          // 0..3 floats fetched before the frame
-            const unsigned bytes = (unsigned)(((lead + N) * 4 + 15) & ~15);
-            const unsigned dst = (unsigned)__cvta_generic_to_shared(buf);
-            if (t == 0) {
-                asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(mb), "r"(bytes) : "memory");
-                asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(dst), "l"(a0), "r"(bytes), "r"(mb)
-                             : "memory");
-            }
-            asm volatile("{\n.reg .pred p;\nWAIT_%=:\nmbarrier.try_wait.parity.shared::cta.b64 p, [%0], 0;\n@p bra DONE_%=;\nbra WAIT_%=;\nDONE_%=:\n}" ::"r"(mb) : "memory");
-            const float *tile = (const float *)buf + lead + 2 * t;
-#pragma unroll
-            for (int i = 0; i < 16; ++i) { bx0[i] = tile[2 * T * i]; bx1[i] = tile[2 * T * i + 1]; }
-            bulk_done = true;
-        }
-        frame_sync<T>(group);   // every thread has its samples: the buffer may now take the permuted, windowed frame
-    }
     if (active) {
         const long k = k0 + f;
         const int64_t start = (int64_t)k * p.hop;
@@ -197,9 +160,6 @@ __global__ void __launch_bounds__((N / 32 > 256 ? N / 32 : 256)) k_analyse_t(con
                     x1[i] = s0 + 1 < valid ? (float)xp[2 * T * i + 1] * (1.0f / 32768.0f) : 0.f;
                 }
             }
-        } else if (kBulk && bulk_done) {
-#pragma unroll
-            for (int i = 0; i < 16; ++i) { x0[i] = bx0[i]; x1[i] = bx1[i]; }
         } else {
             const float *__restrict__ xp = (const float *)g.in + xoff + 2 * t;
             if (valid == N && ((reinterpret_cast<uintptr_t>(xp) & 7) == 0)) {   // even frame start: one 64-bit load per sample pair
@@ -1022,14 +982,6 @@ template <int N> static void launch_analyse_t(const DevPlan &p, const DevRows &g
     const int total = nframes * g.rows;
     const int grid = (total + G - 1) / G, block = T >= 256 ? T : 256;
     const size_t sm = sizeof(float2) * G * S::kPadded;
-    static const bool bulk = [] { const char *e = std::getenv("PVGPU_ANALYSE_BULK"); return e && e[0] == '1'; }();
-    if (bulk && g.spec && !g.fmt && (N * sizeof(float) + 16 <= sizeof(float2) * S::kPadded) && (sizeof(float2) * S::kPadded) % 16 == 0) {
-        // the over-fetch stays inside the row: rows are in_stride apart and both the base and the stride are 16-byte multiples
-        if ((reinterpret_cast<uintptr_t>(g.in) & 15) == 0 && (g.in_stride & 3) == 0) {
-            k_analyse_t<N, false, true, true><<<grid, block, sm + 8 * G + 8, st>>>(p, g, k0, nframes, total);
-            return;
-        }
-    }
     if (g.spec) {
         if (g.fmt) k_analyse_t<N, true, true><<<grid, block, sm, st>>>(p, g, k0, nframes, total);
         else k_analyse_t<N, false, true><<<grid, block, sm, st>>>(p, g, k0, nframes, total);
@@ -1171,7 +1123,6 @@ template void launch_ring_rows<float>(float *, int64_t, int64_t, int64_t, const 
 template void launch_ring_rows<short>(short *, int64_t, int64_t, int64_t, const short *, int64_t, int64_t, int64_t, int, int, cudaStream_t);
 
 int ola_max_table_slices() { return kOlaMaxSlices; }
-int ola_max_table_frames() { return kOlaMaxFrames; }
 
 int ola_run_limit(const DevPlan &p, int run, int max_consumed, int max_out) {
     if (run > kOlaMaxSlices - 16) run = kOlaMaxSlices - 16;

@@ -113,9 +113,8 @@ static_assert(sizeof(ResampleRun) == 72, "ResampleRun layout");
 
 // largest run (slices per CTA) not above `run` that the packed entries and the CTA tables can hold
 int ola_run_limit(const DevPlan &p, int run, int max_consumed, int max_out);
-// sizes of k_ola_resample's per-CTA tables: slices (run + resampler history) and the frames overlapping them
+// size of k_ola_resample's per-CTA slice table (run + resampler history)
 int ola_max_table_slices();
-int ola_max_table_frames();
 // dynamic shared memory of the phase-locked core's kernels on Cartesian spectra for C channels per stream
 size_t lock_smem_bytes(const DevPlan &p, int channels, int maxpk);
 // overlap-add + normalisation (+ resampler when p.rs_active); `run` consecutive slices per CTA starting at k0 (which must
@@ -123,11 +122,6 @@ size_t lock_smem_bytes(const DevPlan &p, int channels, int maxpk);
 void launch_ola_resample(const DevPlan &p, const DevRows &g, const SliceRec *recs, const float *norm, int64_t norm_base, long recs_base,
                          long k0, int nframes, int run, int max_consumed, const ResampleRun *runs, const unsigned *rs_ent, const float *rs_frac,
                          const unsigned *rs_steps, long run_origin, cudaStream_t st);
-// The same stage as a persistent, warp-specialised kernel (pv_ola_ws.cu): producer warps build the normalised stream of the next
-// run while consumer warps filter the current one.  false: no such kernel for this plan (launch k_ola_resample instead).
-bool launch_ola_resample_ws(const DevPlan &p, const DevRows &g, const SliceRec *recs, const float *norm, int64_t norm_base, long recs_base, long k0, int nframes,
-                            int run, int max_consumed, const ResampleRun *runs, const unsigned *rs_ent, const float *rs_frac, const unsigned *rs_steps,
-                            long run_origin, cudaStream_t st, cudaError_t *err);
 // Fused inverse FFT + window + overlap-add + normalisation + resampler (k_synth_ola, pv_fused.cu): one CTA per row runs the
 // frames [k0, k0 + nf) of a chunk in order, `run` frames per round (a multiple of the frames it has in flight).
 struct FusedArgs {
@@ -138,12 +132,11 @@ struct FusedArgs {
     int acc_len;      // floats of the shared-memory accumulator ring: power of two >= N + (run - 1) * largest shift increment
     int in_len;       // floats of the resampler input window: hist_len + run * largest per-slice contribution (+ pad)
     int hist_len;     // filt_len + 8 normalised samples carried between rounds / launches (0 without resampler)
-    int ws;           // 1: warp-specialised kernel (k_synth_ola_ws: producer warps + resampler warps, two input windows)
     const ResampleRun *runs; const unsigned *rs_ent; const float *rs_frac; const unsigned *rs_steps; long run_origin;
     const float *car_mag, *car_phase;   // vocoder carrier spectra or null
 };
 int fused_frames_in_flight(int N);   // 0: this FFT size has no fused kernel
-bool fused_plan(const DevPlan &p, int frames_per_chunk, int max_shift, int max_consumed, int max_out, size_t smem_limit, int force_run, bool want_ws, FusedArgs *out);
+bool fused_plan(const DevPlan &p, int frames_per_chunk, int max_shift, int max_consumed, int max_out, size_t smem_limit, FusedArgs *out);
 cudaError_t launch_synth_ola(const DevPlan &p, const DevRows &g, const FusedArgs &a, cudaStream_t st);
 
 // cepstral spectral-envelope modification of the chunk's spectra in place (pv_cepstral.cu); false: no kernel for this FFT size

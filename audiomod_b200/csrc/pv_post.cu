@@ -8,8 +8,6 @@
 // sample tiles through shared memory so that every global access is a coalesced 128-byte row segment.
 // Arithmetic follows the reference's types expression by expression (float members, the double literals where it has them,
 // no FMA contraction); log10f / pow are CUDA's, within an ulp or two of glibc's (tolerance path, like the resampler).
-#include <cstdlib>
-
 #include "../../include/pvgpu.h"
 #include "pv_kernels.cuh"
 #include "pv_synth.cuh"
@@ -187,23 +185,17 @@ void launch_postchain(const DevRows &g, const PostChain &pc, float *state, int64
 // Streaming instances: a call's few hundred columns per row are walked serially by one thread per row, so the rows are spread
 // over as many SMs as possible -- one warp (32 rows) per CTA, 128 CTAs for 4096 rows instead of the batch's 32.  Measured faster
 // at both sizes (compressor + limiter: 0.91 against 1.08 ms per call at 1024 rows, 1.68 against 2.08 ms at 4096; B200,
-// profiles/r04_live_postchain_latency.jsonl), so there is one shape.  PVGPU_POST_WARPS=4 selects the batch's shape for chains
-// whose coefficients are the same in every stream (read at every launch, for that comparison).  coef non-null: per-stream
-// coefficients (k_postchain<1, *, true>, one warp per CTA: four warps of staged coefficients would not fit 48 KB).  The engine
-// passes its table when some stream's parameters differ from the chain's, or always with PVGPU_POST_PER_ROW=1 (pv_engine.cu; for
-// measuring the two kernels on identical parameters).
+// profiles/r04_live_postchain_latency.jsonl), so there is one shape.  coef non-null: per-stream coefficients (k_postchain<1, *,
+// true>, one warp per CTA: four warps of staged coefficients would not fit 48 KB).  The engine passes its table when some
+// stream's parameters differ from the chain's, or always with PVGPU_POST_PER_ROW=1 (pv_engine.cu; for measuring the two
+// kernels on identical parameters).
 void launch_postchain_stream(const DevRows &g, const PostChain &pc, float *state, int64_t col0, int64_t col1, void *dst, int dst_fmt, const float *coef,
                              cudaStream_t st) {
     if (pc.n == 0 || col1 <= col0) return;
-    const char *v = std::getenv("PVGPU_POST_WARPS");
-    const int warps = !coef && v && v[0] == '4' ? 4 : 1;
-    const int stride = postchain_state_stride(pc), ctas = (g.rows + 32 * warps - 1) / (32 * warps);
+    const int stride = postchain_state_stride(pc), ctas = (g.rows + 31) / 32;
     if (coef) {
         if (dst_fmt == PVGPU_S16) k_postchain<1, true, true><<<ctas, 32, 0, st>>>(g, pc, state, stride, col0, col1, dst, coef);
         else k_postchain<1, false, true><<<ctas, 32, 0, st>>>(g, pc, state, stride, col0, col1, dst, coef);
-    } else if (warps == 4) {
-        if (dst_fmt == PVGPU_S16) k_postchain<4, true, false><<<ctas, 128, 0, st>>>(g, pc, state, stride, col0, col1, dst, nullptr);
-        else k_postchain<4, false, false><<<ctas, 128, 0, st>>>(g, pc, state, stride, col0, col1, dst, nullptr);
     } else {
         if (dst_fmt == PVGPU_S16) k_postchain<1, true, false><<<ctas, 32, 0, st>>>(g, pc, state, stride, col0, col1, dst, nullptr);
         else k_postchain<1, false, false><<<ctas, 32, 0, st>>>(g, pc, state, stride, col0, col1, dst, nullptr);

@@ -289,9 +289,8 @@ class PhaseVocoderBatch:
 
     def set_fused(self, enable=True):
         """True: the fused inverse-FFT + overlap-add + resampler kernel; False: the split kernels; None: automatic (split unless the
-        stretch ratio exceeds their table limits); "ola-ws": the split kernels with the warp-specialised overlap-add + resampler
-        stage.  Bit-identical results in every case."""
-        check(_lib.lib().pvgpu_batch_set_fused(self._h, -1 if enable is None else (2 if enable == "ola-ws" else int(bool(enable)))))
+        stretch ratio exceeds their table limits).  Bit-identical results in every case."""
+        check(_lib.lib().pvgpu_batch_set_fused(self._h, -1 if enable is None else int(bool(enable))))
 
     KERNEL_KINDS = ("analyse", "phase_core", "synthesise", "ola_resample", "synth_ola", "fixed_phase", "lock_peaks", "lock_chain")
 

@@ -270,9 +270,7 @@ int pvgpu_batch_tune(pvgpu_batch *b, int frames_per_chunk, int rows_per_group, i
  * (512..8192); -1 (default) = automatic: the split kernels -- measured faster on B200, profiles/r02_summary.md -- unless the
  * stretch ratio overlaps more frames than their per-CTA tables hold, then the fused kernel, which has no such limit.  Both
  * produce bit-identical samples (tests/test_gpu_fused.py).  The environment variable PVGPU_FUSED=0/1 overrides the choice for
- * every instance, including streaming ones.  2 = the split kernels with the persistent, warp-specialised variant of the
- * overlap-add + resampler stage (producer warps gather the next run while consumer warps filter the current one; same
- * samples, measured 5 % slower than the plain stage on B200 -- kept for the comparison; PVGPU_OLA_WS=1 selects it everywhere). */
+ * every instance, including streaming ones. */
 int pvgpu_batch_set_fused(pvgpu_batch *b, int enable);
 
 /* ---------------------------------------------------------------------------------------------

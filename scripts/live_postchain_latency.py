@@ -4,9 +4,7 @@ mono 44.1 kHz, +7 semitones, FFT 2048, 480-sample blocks, S = 1024 and 4096 stre
 Variants, alternating in one process:
   * none                     -- no chain;
   * comp_lim                 -- [compressor, limiter];
-  * voice                    -- equalizer_chain(VOICE_EQ) + compressor + limiter (the usual chain of a voice path);
-  each chained variant in the streaming launch shape (one warp of 32 rows per CTA) and, with PVGPU_POST_WARPS=4, in the batch's
-  shape (four warps per CTA), to choose the shape by measurement.
+  * voice                    -- equalizer_chain(VOICE_EQ) + compressor + limiter (the usual chain of a voice path).
 Passes: host rows through processBlock, float32 and int16 (p50 / p99 / max wall time per call, what the chain adds at p50 and
 p99, real-time streams per GPU at p99); float32 device rows through processBlockDevice, sustained time per call; the post-chain
 kernel's own device time per launch (torch.profiler); the card's name, power limit and maximum SM clock (nvidia-smi) in the
@@ -34,11 +32,7 @@ VOICE_EQ = [1, 100, 0.7, 0.0,  0, 400, 0.3, -1.5,  1, 300, 1.0, -2.0,  0, 2000, 
             1, 3000, 1.0, 3.0,  0, 4000, 0.3, 1.5,  0, 5000, 0.3, -1.5,  1, 8000, 0.7, 0.0]
 COMP_LIM = [("compressor", -20.0, 4.0, 3.0, 5.0, 50.0), ("limiter", -3.0, 0.0, 1.0, 80.0)]
 CHAINS = {"none": [], "comp_lim": COMP_LIM, "voice": A.equalizer_chain(VOICE_EQ) + COMP_LIM}
-VARIANTS = [("none", 1), ("comp_lim", 1), ("comp_lim", 4), ("voice", 1), ("voice", 4)]   # (chain, warps per CTA of the chain)
-
-
-def vname(v):
-    return v[0] if v[0] == "none" else f"{v[0]}_w{v[1]}"
+VARIANTS = ("none", "comp_lim", "voice")
 
 
 def inputs(S):
@@ -47,9 +41,8 @@ def inputs(S):
 
 
 def make(S, fmt, variant):
-    os.environ["PVGPU_POST_WARPS"] = str(variant[1])   # read at every launch of the chain
     pv = A.phasevocoder(SR, 1, 1.0, SHIFT, A.NORMAL_SHIFT, A.PHASE_LOCKED, FFT, streams=S, fmt=fmt)
-    pv.set_postchain(CHAINS[variant[0]])
+    pv.set_postchain(CHAINS[variant])
     return pv
 
 
@@ -107,12 +100,11 @@ def profile_child():
     for S in SIZES:
         x = inputs(S)[A.F32]
         for v in VARIANTS:
-            if v[0] == "none":
+            if v == "none":
                 continue
             us, count = chain_kernel_us(S, x, v)
-            print(json.dumps({"pass": "k_postchain_device_time (torch.profiler, device rows)", "streams": S, "variant": vname(v),
-                              "warps_per_cta": v[1], "ctas": (S + 32 * v[1] - 1) // (32 * v[1]), "launches": count,
-                              "us_per_launch": round(us, 2)}), flush=True)
+            print(json.dumps({"pass": "k_postchain_device_time (torch.profiler, device rows)", "streams": S, "variant": v,
+                              "ctas": (S + 31) // 32, "launches": count, "us_per_launch": round(us, 2)}), flush=True)
 
 
 def main():
@@ -141,14 +133,14 @@ def main():
             for _ in range(ROUNDS):
                 for v in VARIANTS:
                     host[v] += host_calls(S, fmt, xs[fmt], v)
-            base = np.array(host[("none", 1)]) * 1e3
+            base = np.array(host["none"]) * 1e3
             for v in VARIANTS:
                 t = np.array(host[v]) * 1e3
                 p50, p99 = float(np.median(t)), float(np.percentile(t, 99))
-                rec = {"pass": "host_rows_processBlock", "rows_fmt": fname, "streams": S, "variant": vname(v), "calls": int(t.size),
+                rec = {"pass": "host_rows_processBlock", "rows_fmt": fname, "streams": S, "variant": v, "calls": int(t.size),
                        "p50_ms": round(p50, 4), "p99_ms": round(p99, 4), "max_ms": round(float(t.max()), 4),
                        "realtime_streams_per_gpu_at_p99": int(S * (B / SR) * 1e3 / p99)}
-                if v[0] != "none":
+                if v != "none":
                     rec["chain_adds_p50_ms"] = round(p50 - float(np.median(base)), 4)
                     rec["chain_adds_p99_ms"] = round(p99 - float(np.percentile(base, 99)), 4)
                 emit(rec)
@@ -156,17 +148,16 @@ def main():
         for _ in range(ROUNDS):
             for v in VARIANTS:
                 dev[v].append(device_calls(S, xs[A.F32], v))
-        base = float(np.median(dev[("none", 1)]))
+        base = float(np.median(dev["none"]))
         for v in VARIANTS:
             per = float(np.median(dev[v]))
-            rec = {"pass": "device_rows_processBlockDevice", "rows_fmt": "f32", "streams": S, "variant": vname(v),
+            rec = {"pass": "device_rows_processBlockDevice", "rows_fmt": "f32", "streams": S, "variant": v,
                    "rounds_ms_per_call": [round(u, 4) for u in dev[v]], "ms_per_call": round(per, 4),
                    "realtime_streams_per_gpu": int(S * (B / SR) * 1e3 / per)}
-            if v[0] != "none":
+            if v != "none":
                 rec["chain_adds_ms"] = round(per - base, 4)
             emit(rec)
         del xs
-    os.environ.pop("PVGPU_POST_WARPS", None)
     child = subprocess.run([sys.executable, os.path.abspath(__file__), "--profile-child"], capture_output=True, text=True)
     if child.returncode != 0:
         raise SystemExit(f"profiler pass failed ({child.returncode}):\n{child.stderr[-4000:]}")

@@ -1,9 +1,8 @@
 """Small cases for compute-sanitizer (one tool per run):
     compute-sanitizer --tool memcheck  python scripts/sanitize_case.py
     compute-sanitizer --tool racecheck python scripts/sanitize_case.py
-cfg1 (stereo +4 st) and cfg4 (mono +7 st) batches through the split kernels, the fused kernel and its warp-specialised variant,
-a formant case, a robotic case (no resampler: the fused kernel stores straight from the accumulator) and one streaming
-instance.  Prints one line per case; the sanitizer's own summary follows."""
+cfg1 (stereo +4 st) and cfg4 (mono +7 st) batches through the split kernels and the fused kernel, a formant case, a robotic
+case (no resampler: the fused kernel stores straight from the accumulator) and one streaming instance.  Prints one line per case; the sanitizer's own summary follows."""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np
@@ -14,8 +13,7 @@ secs = float(sys.argv[1]) if len(sys.argv) > 1 else 0.25
 ref = {}
 for name, ch, st, mode, fft in (("cfg1", 2, 4.0, 0, 2048), ("cfg4", 1, 7.0, 0, 2048), ("formant", 1, 4.0, 2, 2048), ("robotic", 2, 0.0, 6, 1024)):
     xs = [synth(100 + i, 44100, secs * (1.0 - 0.3 * i), ch) for i in range(3)]
-    for variant, fused, ws in (("split", False, "0"), ("fused", True, "0"), ("fused-ws", True, "1")):
-        os.environ["PVGPU_FUSED_WS"] = ws
+    for variant, fused in (("split", False), ("fused", True)):
         b = A.PhaseVocoderBatch(len(xs), xs[0].shape[1], 44100, ch, 1.0, st, mode, 1, fft)
         b.set_fused(fused)
         b.tune(frames_per_chunk=16)

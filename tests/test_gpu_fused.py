@@ -107,18 +107,3 @@ def test_many_channels_take_the_polar_core(A, oracle):
     kw = dict(semitones=3.0, mode=0, coremode=1, fftsize=4096)
     (y,), _ = _run(A, [x], sr, ch, kw, None)
     assert_parity(y, oracle.run_offline(x, sr, **kw), "6 channels, FFT 4096")
-
-
-@pytest.mark.parametrize("case", [c for c in CASES if ctor_args(c[1])[1] != 0.0], ids=[c[0] for c in CASES if ctor_args(c[1])[1] != 0.0])
-def test_warp_specialised_overlap_add_equals_plain_stage(A, case):
-    """set_fused("ola-ws"): k_ola_resample_ws (pv_ola_ws.cu; producer warps gather run i+1 while consumer warps filter run i,
-    persistent CTAs over a list of (row, run) items) must give the samples of k_ola_resample bit for bit -- every pitch case,
-    three ragged streams, and chunk sizes that leave a CTA one run per row and several."""
-    name, kw, sr, ch, secs, seed = case
-    xs = [make_input(name, sr, ch, secs * f, seed + 3 * i) for i, f in enumerate((1.0, 0.37, 1.21))]
-    want, _ = _run(A, xs, sr, ch, kw, False)
-    for fpc in (0, 16):
-        got, kt = _run(A, xs, sr, ch, kw, "ola-ws", fpc)
-        for i, (a, b) in enumerate(zip(got, want)):
-            assert a.shape == b.shape
-            assert np.array_equal(a.view(np.uint32), b.view(np.uint32)), f"{name}[{i}] fpc={fpc}: warp-specialised and plain overlap-add differ"
