@@ -1557,7 +1557,7 @@ int pvgpu_test_loudness(int device, int sample_rate, int channels, int streams, 
 // ------------------------------------------------------------------------------------------------
 // streaming instance: one audiomod::phasevocoder object.  Each process call appends the new input,
 // lets the scheduler decide which slices that call runs (exactly the reference's block loop), runs
-// those frames on the device and moves the produced samples into a host FIFO.
+// those frames on the device and moves the produced samples into the instance's output ring.
 // ------------------------------------------------------------------------------------------------
 // Small persistent pool for the per-row host copies of a live batch (thousands of rows per call: a single thread moves them at
 // ~6 GB/s, which is what bounds the call).  run(n, samples_per_item, f) calls f(i) for i in [0, n) on the workers and the caller
@@ -1613,55 +1613,115 @@ struct RowPool {
     }
 };
 
-// Output FIFO of a streaming instance: every row holds the same number of samples (the rows advance in lock-step), so it is
-// one [rows][cap] block with a common read position -- a ring (cap a power of two), no per-row containers, no compaction.
-// The block is page-locked when it can be: the device-to-host copy of a call's output lands in the ring directly.  T is the
-// instance's sample type (float, or int16_t for int16 rows).
-template <typename T>
-struct RowFifo {
-    T *buf = nullptr;
-    bool pinned = false;
+// Output ring of a streaming instance (the reference's outbuf): every row holds the same number of samples (the rows advance in
+// lock-step), so it is one [rows][cap] block with a common read position -- cap a power of two, no per-row containers, no
+// compaction.  Its storage is chosen when the instance's kind of rows is locked: host rows get page-locked host memory when it
+// can be had (the device-to-host copy of a call's output lands in the ring directly), else malloc; device rows get device
+// memory.  The positions are the same for every storage; only the data movement differs.  T is the instance's sample type
+// (float, or int16_t for int16 rows).
+struct RowRing {
+    enum Storage { kMalloc, kPinned, kDevice };
+    void *buf = nullptr;
+    Storage mem = kMalloc;
     size_t rows = 0, cap = 0, rd = 0, count = 0;
-    ~RowFifo() { release(); }
-    void release() { if (buf) { if (pinned) cudaFreeHost(buf); else std::free(buf); } buf = nullptr; cap = 0; }
-    void init(size_t rows_) { release(); rows = rows_; rd = count = 0; }
-    static T *alloc(size_t bytes, bool *pinned) {
-        void *p = nullptr;
-        if (cudaHostAlloc(&p, bytes, cudaHostAllocDefault) == cudaSuccess) { *pinned = true; return (T *)p; }
-        cudaGetLastError();
-        *pinned = false;
-        return (T *)std::malloc(bytes);
+    ~RowRing() { release(); }
+    void release() {
+        if (buf) { if (mem == kDevice) cudaFree(buf); else if (mem == kPinned) cudaFreeHost(buf); else std::free(buf); }
+        buf = nullptr; cap = 0;
     }
-    // only between calls (no copy in flight)
-    bool reserve(size_t need) {
-        if (need <= cap) return true;
-        size_t ncap = cap ? cap : 4096;
-        while (ncap < need) ncap *= 2;
-        bool np = false;
-        T *nb = alloc(sizeof(T) * rows * ncap, &np);
-        if (!nb) return false;
-        for (size_t r = 0; r < rows; ++r)
-            for (size_t i = 0; i < count; ++i) nb[r * ncap + i] = buf[r * cap + ((rd + i) & (cap - 1))];
-        release();
-        buf = nb; pinned = np; cap = ncap; rd = 0;
-        return true;
-    }
-    // where the next n samples of every row go: [w, w + first) and, if the ring wraps, [0, n - first); call after reserve
-    void write_span(size_t n, size_t *w, size_t *first) const { *w = (rd + count) & (cap - 1); *first = std::min(n, cap - *w); }
+    void init(size_t rows_, bool device) { release(); rows = rows_; mem = device ? kDevice : kMalloc; rd = count = 0; }
+    template <typename T> T *as() const { return (T *)buf; }
+    // where the next samples of every row go; of n samples from position `at`, those before the end of the row (the rest
+    // continue at 0)
+    size_t write_pos() const { return (rd + count) & (cap - 1); }
+    size_t first_span(size_t at, size_t n) const { return std::min(n, cap - at); }
+    int64_t mask() const { return (int64_t)cap - 1; }
     void commit(size_t n) { count += n; }
-    // remove the oldest k samples of every row into out[r]
-    void pop(T *const *out, size_t k, RowPool &pool) {
-        if (k == 0) return;
-        const size_t first = std::min(k, cap - rd);
-        pool.run(rows, k, [&, first, k](size_t r) {
-            std::memcpy(out[r], &buf[r * cap + rd], sizeof(T) * first);
-            if (first < k) std::memcpy(out[r] + first, &buf[r * cap], sizeof(T) * (k - first));
-        });
+    void advance(size_t k) {
         rd = (rd + k) & (cap - 1);
         count -= k;
         if (count == 0) rd = 0;
     }
+    // Room for `need` samples per row, only between calls (no copy in flight).  Host storage is re-laid on the host; device
+    // storage by a kernel on `st`, which is synchronised before the old block goes.
+    template <typename T> int reserve(size_t need, cudaStream_t st) {
+        if (need <= cap) return PVGPU_OK;
+        size_t ncap = cap ? cap : 4096;
+        while (ncap < need) ncap *= 2;
+        if (mem == kDevice) {
+            DevBuf grown;
+            CU(grown.ensure(sizeof(T) * rows * ncap));
+            if (count) launch_ring_rows(grown.as<T>(), (int64_t)ncap, 0, -1, as<T>(), (int64_t)cap, (int64_t)rd, mask(), (int)count, (int)rows, st);
+            CU(cudaStreamSynchronize(st));
+            std::swap(buf, grown.p);   // grown frees the old block
+        } else {
+            void *p = nullptr;
+            Storage m = kPinned;
+            if (cudaHostAlloc(&p, sizeof(T) * rows * ncap, cudaHostAllocDefault) != cudaSuccess) {
+                cudaGetLastError();
+                m = kMalloc;
+                p = std::malloc(sizeof(T) * rows * ncap);
+            }
+            if (!p) return fail(PVGPU_ENOMEM, "out of host memory");
+            const size_t first = first_span(rd, count);
+            if (count)
+                for (size_t r = 0; r < rows; ++r) {
+                    std::memcpy((T *)p + r * ncap, as<T>() + r * cap + rd, sizeof(T) * first);
+                    std::memcpy((T *)p + r * ncap + first, as<T>() + r * cap, sizeof(T) * (count - first));
+                }
+            release();
+            buf = p; mem = m;
+        }
+        cap = ncap; rd = 0;
+        return PVGPU_OK;
+    }
+    // Enqueue on `st` the copy of n samples of every row of the device block src (rows `pitch` samples apart) to the write
+    // position: one or two device-to-host 2-D copies into host storage, one kernel into device storage.  Call after reserve;
+    // the samples count once commit(n) is called, for host storage after the copies have completed.
+    template <typename T> int append(const T *src, int64_t pitch, size_t n, cudaStream_t st) {
+        const size_t w = write_pos();
+        if (mem == kDevice) {
+            launch_ring_rows(as<T>(), (int64_t)cap, (int64_t)w, mask(), src, pitch, 0, -1, (int)n, (int)rows, st);
+            return PVGPU_OK;
+        }
+        const size_t first = first_span(w, n);
+        CU(cudaMemcpy2DAsync(as<T>() + w, sizeof(T) * cap, src, sizeof(T) * pitch, sizeof(T) * first, rows, cudaMemcpyDeviceToHost, st));
+        if (first < n)
+            CU(cudaMemcpy2DAsync(as<T>(), sizeof(T) * cap, src + first, sizeof(T) * pitch, sizeof(T) * (n - first), rows, cudaMemcpyDeviceToHost, st));
+        return PVGPU_OK;
+    }
+    // Remove the oldest k samples of every row.  Host storage: into the caller's rows out[r], copied on the pool.
+    template <typename T> void pop(T *const *out, size_t k, RowPool &pool) {
+        if (k == 0) return;
+        const T *b = as<T>();
+        const size_t first = first_span(rd, k);
+        pool.run(rows, k, [&, first, k](size_t r) {
+            std::memcpy(out[r], &b[r * cap + rd], sizeof(T) * first);
+            if (first < k) std::memcpy(out[r] + first, &b[r * cap], sizeof(T) * (k - first));
+        });
+        advance(k);
+    }
+    // Device storage: into the caller's block d_out (rows `pitch` samples apart), by a kernel on the caller's stream.
+    template <typename T> void pop(T *d_out, int64_t pitch, size_t k, cudaStream_t st) {
+        if (k == 0) return;
+        launch_ring_rows(d_out, pitch, 0, -1, as<T>(), (int64_t)cap, (int64_t)rd, mask(), (int)k, (int)rows, st);
+        advance(k);
+    }
 };
+
+// The kinds of rows a streaming instance can be fed: where they live, their sample type and the names of their calls.  The
+// kind is fixed by the instance's first data call; a call of another kind is refused with the name of the call to use.
+struct RowKind {
+    const char *name;
+    bool dev;                              // device memory, every call enqueued on the caller's stream
+    size_t esz;                            // bytes per sample: float32 or int16
+    const char *process, *retrieve, *meters;
+};
+static const RowKind kHostRows = {"host", false, sizeof(float), "pvgpu_process", "pvgpu_retrieve", "pvgpu_get_meters"};
+static const RowKind kDeviceRows = {"device", true, sizeof(float), "pvgpu_process_device", "pvgpu_retrieve_device", "pvgpu_get_meters_device"};
+static const RowKind kHostS16Rows = {"host int16", false, sizeof(int16_t), "pvgpu_process_s16", "pvgpu_retrieve_s16", "pvgpu_get_meters"};
+static const RowKind kDeviceS16Rows = {"device int16", true, sizeof(int16_t), "pvgpu_process_device_s16", "pvgpu_retrieve_device_s16",
+                                       "pvgpu_get_meters_device"};
 
 struct pvgpu_stream {
     pvgpu_config cfg{};
@@ -1673,12 +1733,10 @@ struct pvgpu_stream {
     std::unique_ptr<Carrier> carrier;
     GlibcRand rng;
     Workspace ws;
-    // Kind of rows the instance is fed, fixed by its first data call: 0 not used yet, 1 host rows, 2 device rows (float32),
-    // 3 host rows, 4 device rows (int16).  An int16 instance keeps int16 end to end: pending input, packed upload, device window,
-    // output rings; the kernels convert as they load and quantise as they store (g.fmt = PVGPU_S16).
-    int io_mode = 0;
-    bool dev_rows() const { return io_mode == 2 || io_mode == 4; }
-    size_t esz() const { return io_mode >= 3 ? sizeof(int16_t) : sizeof(float); }   // bytes per sample of the instance's rows
+    // Kind of rows the instance is fed, null until its first data call.  An int16 instance keeps int16 end to end: pending
+    // input, packed upload, device window, output ring; the kernels convert as they load and quantise as they store
+    // (g.fmt = PVGPU_S16).
+    const RowKind *kind = nullptr;
     // input fed by calls that completed no slice (not yet on the device): [rows][pend_cap] samples of the instance's type,
     // pend_len valid per row
     std::vector<unsigned char> pend;
@@ -1704,18 +1762,15 @@ struct pvgpu_stream {
     int64_t in_cap = 0, dev_len = 0;
     std::vector<float> car_tail;
     int64_t in_base = 0;
-    RowFifo<float> fifo;                   // output FIFO of all rows (the reference's outbuf ring)
-    RowFifo<int16_t> fifo16;               // the same for int16 rows
-    // Device-resident I/O (pvgpu_process_device / _retrieve_device): rows come from and go to device memory, everything is
-    // enqueued on the caller's stream and no call waits for the device.  The output FIFO is a ring [rows][dfifo_cap] on the
-    // device; what a call uploads is staged in one of four page-locked arenas, each guarded by an event.
-    DevBuf d_fifo;
-    size_t dfifo_cap = 0, dfifo_rd = 0, dfifo_count = 0;
-    static constexpr int kDevArenas = 4;
-    PinnedArena dev_arena[kDevArenas];
-    cudaEvent_t dev_arena_ev[kDevArenas] = {};
-    bool dev_arena_used[kDevArenas] = {};
-    unsigned dev_arena_i = 0;
+    RowRing ring;                          // output of all rows, in host or device memory by the kind of rows
+    // What a call uploads is staged in a page-locked arena.  Host-row calls synchronise, so arena 0 serves all of them.
+    // Device-row calls do not wait for the device (everything is enqueued on the caller's stream): they rotate through the
+    // arenas, each guarded by an event recorded after the call that used it.
+    static constexpr int kArenas = 4;
+    PinnedArena arena[kArenas];
+    cudaEvent_t arena_ev[kArenas] = {};
+    bool arena_used[kArenas] = {};
+    unsigned arena_i = 0;
     RowPool pool;                          // host copies of a live batch's rows
     double tr_us[6] = {}, tr_dev[4] = {};  // PVGPU_STREAM_TRACE=1: accumulated microseconds per phase of a call (host) and per device phase
     cudaEvent_t tr_ev[7] = {};
@@ -1752,13 +1807,12 @@ struct pvgpu_stream {
     std::vector<float> meter_host;
     std::vector<float> h_stage, scratch;
     std::vector<unsigned char> h_pack;
-    PinnedArena arena;
     cudaStream_t st = nullptr;
     static constexpr int kF = 64;
     ~pvgpu_stream() {
         if (st) cudaStreamDestroy(st);
         for (auto e : tr_ev) if (e) cudaEventDestroy(e);
-        for (auto e : dev_arena_ev) if (e) cudaEventDestroy(e);
+        for (auto e : arena_ev) if (e) cudaEventDestroy(e);
     }
 };
 
@@ -1767,7 +1821,7 @@ struct pvgpu_stream {
 static int stream_ensure_window(pvgpu_stream *s, int64_t len, cudaStream_t st) {
     if (len <= s->in_cap) return PVGPU_OK;
     const int R = s->R();
-    const size_t es = s->esz();
+    const size_t es = s->kind->esz;
     const int64_t cap = (std::max<int64_t>(2 * s->in_cap, len + 4096) + 3) & ~(int64_t)3;
     DevBuf grown;
     CU(grown.ensure(es * (size_t)R * cap));
@@ -1782,17 +1836,13 @@ static int stream_ensure_window(pvgpu_stream *s, int64_t len, cudaStream_t st) {
     return PVGPU_OK;
 }
 
-template <typename T> static RowFifo<T> &host_fifo(pvgpu_stream *s) {
-    if constexpr (std::is_same<T, float>::value) return s->fifo; else return s->fifo16;
-}
-
 // One pvgpu_process call that completed `added` new slices starting at slice k0.  Steady state: no heap allocation (the
 // vectors keep their capacity), every upload goes through the page-locked arena, one stream synchronisation at the end.
 // T is the sample type of the instance's rows (float or int16_t).
 template <typename T>
 static int stream_run_new(pvgpu_stream *s, long k0, int added, const T *const *in, int n_new, cudaStream_t user_st = nullptr) {
     static_assert(std::is_same<T, float>::value || std::is_same<T, int16_t>::value, "float32 or int16 rows");
-    const bool dev = s->dev_rows();        // device rows: the input is already in the window, everything goes on the caller's stream
+    const bool dev = s->kind->dev;         // device rows: the input is already in the window, everything goes on the caller's stream
     cudaStream_t const st = dev ? user_st : s->st;
     Pipeline &pl = s->pl;
     Scheduler &sc = *s->sched;
@@ -1814,21 +1864,20 @@ static int stream_run_new(pvgpu_stream *s, long k0, int added, const T *const *i
     const int64_t out_base = first.out_off;
     const int64_t new_out = sc.total_out() - out_base;
     const int64_t out_stride = std::max<int64_t>((new_out + 3) & ~(int64_t)3, 4);
+    const unsigned ai = dev ? s->arena_i++ % pvgpu_stream::kArenas : 0;   // the call's staging arena
+    PinnedArena &arena = s->arena[ai];
     {   // room for everything this call stages (nothing is in flight between calls)
         const size_t lists = p.rs_active ? (size_t)(new_out + 8 * 32 * ((added + 3) / 4 + 1) + 64) * 24 + (size_t)added * sizeof(ResampleRun) : 0;
         const size_t need = sizeof(float) * ((size_t)R * (pend + 16) + s->car_tail.size() + sc.norm().size()) + sizeof(SliceRec) * sc.recs().size() +
                             lists + (pl.d.whisper ? sizeof(float) * (size_t)added * C * p.H : 0) + 64 * 16 + sizeof(int64_t) * (2 * R + 1) +
                             sizeof(float) * s->post_pending.size() * (1 + 6 * (size_t)pl.post.n) +
                             (s->meters && !dev ? sizeof(float) * s->meter_host.size() + 64 : 0);
-        PinnedArena *ar = &s->arena;
         if (dev) {   // no call waits for the device: rotate the arenas, each is free again when the call that used it has run
-            const unsigned i = s->dev_arena_i++ % pvgpu_stream::kDevArenas;
-            if (!s->dev_arena_ev[i]) CU(cudaEventCreateWithFlags(&s->dev_arena_ev[i], cudaEventDisableTiming));
-            if (s->dev_arena_used[i]) CU(cudaEventSynchronize(s->dev_arena_ev[i]));
-            ar = &s->dev_arena[i];
+            if (!s->arena_ev[ai]) CU(cudaEventCreateWithFlags(&s->arena_ev[ai], cudaEventDisableTiming));
+            if (s->arena_used[ai]) CU(cudaEventSynchronize(s->arena_ev[ai]));
         }
-        ar->reserve(need);
-        pl.arena = ar;
+        arena.reserve(need);
+        pl.arena = &arena;
         pl.staged_all = true;
     }
     int rc;
@@ -1840,7 +1889,7 @@ static int stream_run_new(pvgpu_stream *s, long k0, int added, const T *const *i
         // of rows must not issue a copy per row); without page-locked memory the same block is pageable and the copy synchronous
         constexpr int64_t line = 64 / sizeof(T);
         const int64_t pp = (pend + line - 1) & ~(line - 1);   // packed row pitch: rows start on 64-byte lines
-        T *pin = (T *)s->arena.take(sizeof(T) * (size_t)R * pp);
+        T *pin = (T *)arena.take(sizeof(T) * (size_t)R * pp);
         const bool locked = pin != nullptr;
         if (!pin) { s->h_pack.resize(sizeof(T) * (size_t)R * pp); pin = (T *)s->h_pack.data(); }
         const size_t pl_ = s->pend_len;
@@ -1943,36 +1992,15 @@ static int stream_run_new(pvgpu_stream *s, long k0, int added, const T *const *i
         s->measured += new_out;
         if (!dev) {   // back with the output; without page-locked memory straight into the mirror
             const size_t bytes = sizeof(float) * s->meter_host.size();
-            meter_pin = (float *)s->arena.take(bytes);
+            meter_pin = (float *)arena.take(bytes);
             CU(cudaMemcpyAsync(meter_pin ? (void *)meter_pin : (void *)s->meter_host.data(), s->d_meter.p, bytes, cudaMemcpyDeviceToHost, st));
         }
     }
     CU(cudaGetLastError());
     if (trace) cudaEventRecord(s->tr_ev[2], st);   // kernels done
-    if (new_out > 0 && dev) {   // device rows: append to the device-resident ring
-        if (s->dfifo_count + (size_t)new_out > s->dfifo_cap) {   // grow (rare): stop the world, re-lay the ring out
-            size_t ncap = s->dfifo_cap ? s->dfifo_cap : 4096;
-            while (ncap < s->dfifo_count + (size_t)new_out) ncap *= 2;
-            DevBuf grown;
-            CU(grown.ensure(sizeof(T) * (size_t)R * ncap));
-            if (s->dfifo_count) launch_ring_rows(grown.as<T>(), (int64_t)ncap, 0, -1, s->d_fifo.as<T>(), (int64_t)s->dfifo_cap, (int64_t)s->dfifo_rd, (int64_t)s->dfifo_cap - 1, (int)s->dfifo_count, R, st);
-            CU(cudaStreamSynchronize(st));
-            std::swap(s->d_fifo.p, grown.p);
-            std::swap(s->d_fifo.bytes, grown.bytes);
-            s->dfifo_cap = ncap; s->dfifo_rd = 0;
-        }
-        launch_ring_rows(s->d_fifo.as<T>(), (int64_t)s->dfifo_cap, (int64_t)((s->dfifo_rd + s->dfifo_count) & (s->dfifo_cap - 1)), (int64_t)s->dfifo_cap - 1, s->d_out.as<T>(), out_stride, 0, -1,
-                         (int)new_out, R, st);
-        s->dfifo_count += (size_t)new_out;
-    } else if (new_out > 0) {   // the output goes straight into the (page-locked) FIFO ring
-        RowFifo<T> &fifo = host_fifo<T>(s);
-        if (!fifo.reserve(fifo.count + (size_t)new_out)) return fail(PVGPU_ENOMEM, "out of host memory");
-        size_t w, first;
-        fifo.write_span((size_t)new_out, &w, &first);
-        CU(cudaMemcpy2DAsync(fifo.buf + w, sizeof(T) * fifo.cap, s->d_out.p, sizeof(T) * out_stride, sizeof(T) * first, R, cudaMemcpyDeviceToHost, st));
-        if (first < (size_t)new_out)
-            CU(cudaMemcpy2DAsync(fifo.buf, sizeof(T) * fifo.cap, s->d_out.as<T>() + first, sizeof(T) * out_stride, sizeof(T) * ((size_t)new_out - first), R,
-                                 cudaMemcpyDeviceToHost, st));
+    if (new_out > 0) {   // the output goes straight into the ring (grown first if it must, which is rare)
+        if ((rc = s->ring.reserve<T>(s->ring.count + (size_t)new_out, st))) return rc;
+        if ((rc = s->ring.append(s->d_out.as<T>(), out_stride, (size_t)new_out, st))) return rc;
     }
     if (trace) cudaEventRecord(s->tr_ev[3], st);   // output copy done
     // forget the input no later slice can need: the rest of the window moves to the front of the other buffer, on the device
@@ -1988,9 +2016,8 @@ static int stream_run_new(pvgpu_stream *s, long k0, int added, const T *const *i
     if (trace) cudaEventRecord(s->tr_ev[4], st);   // window compaction done
     mark(1);   // enqueue: schedule upload, work lists, launches, copies
     if (dev) {
-        const unsigned i = (s->dev_arena_i - 1) % pvgpu_stream::kDevArenas;
-        CU(cudaEventRecord(s->dev_arena_ev[i], st));
-        s->dev_arena_used[i] = true;
+        CU(cudaEventRecord(s->arena_ev[ai], st));
+        s->arena_used[ai] = true;
     } else {
         CU(cudaStreamSynchronize(st));   // the call's only synchronisation
     }
@@ -1999,7 +2026,7 @@ static int stream_run_new(pvgpu_stream *s, long k0, int added, const T *const *i
     if (trace && pend > 0) { float ms = 0; cudaEventElapsedTime(&ms, s->tr_ev[0], s->tr_ev[5]); s->tr_dev2[0] += 1e3 * ms; cudaEventElapsedTime(&ms, s->tr_ev[5], s->tr_ev[6]); s->tr_dev2[1] += 1e3 * ms; }
     pl.staged_all = true;
     if (meter_pin) std::memcpy(s->meter_host.data(), meter_pin, sizeof(float) * s->meter_host.size());
-    if (new_out > 0 && !dev) host_fifo<T>(s).commit((size_t)new_out);
+    s->ring.commit((size_t)new_out);   // host rows: the copies have completed
     s->pend_len = 0;
     s->dev_len = keep;
     if (pl.d.vocoder) s->car_tail.erase(s->car_tail.begin(), s->car_tail.begin() + std::min<int64_t>(dropn, (int64_t)s->car_tail.size()));
@@ -2029,12 +2056,13 @@ static int stream_run_new(pvgpu_stream *s, long k0, int added, const T *const *i
     return PVGPU_OK;
 }
 
-// Ring FIFO of one sample type across wrap-arounds, growth and partial pops against a plain model.  Returns 0 or base + the
-// number of the failed check (1 reserve, 2 popped samples, 3 a sample past the popped ones written, 4 count).
-template <typename T> static int fifo_selftest(int base) {
+// Output ring in host storage, of one sample type, across wrap-arounds, growth and partial pops against a plain model (the
+// positions are those of device storage too).  Returns 0 or base + the number of the failed check (1 reserve, 2 popped
+// samples, 3 a sample past the popped ones written, 4 count).
+template <typename T> static int ring_selftest(int base) {
     const size_t R = 7;
-    RowFifo<T> f;
-    f.init(R);
+    RowRing f;
+    f.init(R, false);
     RowPool none;
     std::vector<std::vector<T>> model(R);
     std::vector<T *> out(R);
@@ -2044,16 +2072,15 @@ template <typename T> static int fifo_selftest(int base) {
     for (int it = 0; it < 400; ++it) {
         seed = seed * 1664525u + 1013904223u;
         const size_t n = (seed >> 16) % (it % 50 == 49 ? 9000 : 700);
-        if (!f.reserve(f.count + n)) return base + 1;
-        size_t w, first;
-        f.write_span(n, &w, &first);
+        if (f.reserve<T>(f.count + n, nullptr)) return base + 1;
+        const size_t w = f.write_pos(), first = f.first_span(w, n);
         for (size_t r = 0; r < R; ++r)
             for (size_t i = 0; i < n; ++i) {
                 T v;
                 if constexpr (std::is_same<T, float>::value) v = next + (float)r * 0.25f + (float)i;
                 else v = (T)(uint16_t)((unsigned)it * 977u + (unsigned)r * 131u + (unsigned)i);   // every bit pattern, -1 included
                 model[r].push_back(v);
-                if (i < first) f.buf[r * f.cap + w + i] = v; else f.buf[r * f.cap + (i - first)] = v;
+                if (i < first) f.as<T>()[r * f.cap + w + i] = v; else f.as<T>()[r * f.cap + (i - first)] = v;
             }
         next += 1000.f;
         f.commit(n);
@@ -2071,12 +2098,12 @@ template <typename T> static int fifo_selftest(int base) {
     return 0;
 }
 
-// Host-only self-test of the live batch's containers (no device work): the ring FIFO across wrap-arounds and growth, the
+// Host-only self-test of the live batch's containers (no device work): the output ring across wrap-arounds and growth, the
 // row-copy pool against a serial copy, non-temporal copies at every alignment; float32 rows (checks 1-6), int16 rows (7-11).
 // Returns 0 or the number of the failed check.
 static int host_structs_selftest() {
     int rc;
-    if ((rc = fifo_selftest<float>(0))) return rc;
+    if ((rc = ring_selftest<float>(0))) return rc;
     {   // RowPool + copy_nt
         RowPool pool;
         pool.start(3);
@@ -2095,7 +2122,7 @@ static int host_structs_selftest() {
         for (unsigned char c : seen) hits += c;
         if (hits != R) return 6;
     }
-    if ((rc = fifo_selftest<int16_t>(6))) return rc;
+    if ((rc = ring_selftest<int16_t>(6))) return rc;
     {   // 16-bit copy_nt at every 2-byte destination alignment of a 16-byte line, odd and even lengths, through the pool
         RowPool pool;
         pool.start(3);
@@ -2145,8 +2172,6 @@ static int pvgpu_create_body(const pvgpu_config *cfg, int n_streams, pvgpu_strea
     if ((rc = s->pl.init(*cfg))) return rc;
     s->sched.reset(new Scheduler(s->pl.d, true));
     if (s->pl.d.vocoder) s->carrier.reset(new Carrier(cfg->sample_rate, cfg->mode == PVGPU_VOCODER_CHORD));
-    s->fifo.init((size_t)s->R());
-    s->fifo16.init((size_t)s->R());
     if (s->R() >= 256) s->pool.start((int)std::min(7u, std::max(1u, std::thread::hardware_concurrency() / 2)));   // live batch: parallel row copies
     CU(cudaStreamCreateWithFlags(&s->st, cudaStreamNonBlocking));
     const int halo = 80;
@@ -2188,8 +2213,8 @@ int pvgpu_stream_info(const pvgpu_stream *s, pvgpu_info *info) {
 static int stream_wait_idle(pvgpu_stream *s) {
     CU(cudaSetDevice(s->pl.device));
     CU(cudaStreamSynchronize(s->st));
-    for (int i = 0; i < pvgpu_stream::kDevArenas; ++i)
-        if (s->dev_arena_used[i]) CU(cudaEventSynchronize(s->dev_arena_ev[i]));
+    for (int i = 0; i < pvgpu_stream::kArenas; ++i)
+        if (s->arena_used[i]) CU(cudaEventSynchronize(s->arena_ev[i]));
     return PVGPU_OK;
 }
 
@@ -2266,38 +2291,38 @@ int pvgpu_set_stream_postchain(pvgpu_stream *s, int stream, const pvgpu_fx *chai
 
 }  // extern "C"
 
-// The kind of rows an instance takes is fixed by its first data call (pvgpu_stream::io_mode); a call of another kind is refused
-// with the name of the call to use.
-static const char *const kRowKind[5] = {"", "host", "device", "host int16", "device int16"};
-static const char *const kProcessCall[5] = {"", "pvgpu_process", "pvgpu_process_device", "pvgpu_process_s16", "pvgpu_process_device_s16"};
-static const char *const kRetrieveCall[5] = {"", "pvgpu_retrieve", "pvgpu_retrieve_device", "pvgpu_retrieve_s16", "pvgpu_retrieve_device_s16"};
-static int lock_rows(pvgpu_stream *s, int mode) {
-    const int have = s->io_mode;
-    if (have && have != mode)
-        return fail(PVGPU_ESTATE, "this instance is fed %s rows (%s); %s rows cannot be mixed", kRowKind[have], kProcessCall[have],
-                    (have >= 3) != (mode >= 3) ? "float32 and int16" : "host and device");
-    s->io_mode = mode;
-    return PVGPU_OK;
-}
-static int check_retrieve_rows(const pvgpu_stream *s, int mode) {
-    const int have = s->io_mode;
-    if (have && have != mode) return fail(PVGPU_ESTATE, "this instance is fed %s rows; use %s", kRowKind[have], kRetrieveCall[have]);
+// The first data call locks the instance's kind of rows (a call of another kind is refused with the name of the call to use)
+// and chooses the storage of its output ring.
+static int lock_rows(pvgpu_stream *s, const RowKind &kind) {
+    const RowKind *have = s->kind;
+    if (have && have != &kind)
+        return fail(PVGPU_ESTATE, "this instance is fed %s rows (%s); %s rows cannot be mixed", have->name, have->process,
+                    have->esz != kind.esz ? "float32 and int16" : "host and device");
+    if (!have) s->ring.init((size_t)s->R(), kind.dev);
+    s->kind = &kind;
     return PVGPU_OK;
 }
 
-template <typename T>
-static int process_host(pvgpu_stream *s, const T *const *in, int n) {
-    if (!s || n < 0 || (n > 0 && !in)) return fail(PVGPU_EINVAL, "bad argument");
-    if (!s->pl.d.valid_mode) { s->num_res = 0; return PVGPU_OK; }  // phasevocoder.cc:104-106: unknown mode does nothing
-    int rc;
-    if ((rc = lock_rows(s, std::is_same<T, float>::value ? 1 : 3))) return rc;
+// Start of every process call: the carrier's next n samples, then the schedule takes n more input samples.  Returns the number
+// of slices they complete, the first of which is *k0.
+static int stream_feed(pvgpu_stream *s, int n, long *k0) {
     if (s->carrier) {
         const size_t at = s->car_tail.size();
         s->car_tail.resize(at + n);
         s->carrier->generate(s->car_tail.data() + at, (size_t)n);
     }
-    const long k0 = s->sched->recs_base() + s->sched->slices();
-    const int added = s->sched->feed(n);   // the schedule does not depend on the data
+    *k0 = s->sched->recs_base() + s->sched->slices();
+    return s->sched->feed(n);   // the schedule does not depend on the data: no call has to wait for the device
+}
+
+template <typename T>
+static int process_host(pvgpu_stream *s, const RowKind &kind, const T *const *in, int n) {
+    if (!s || n < 0 || (n > 0 && !in)) return fail(PVGPU_EINVAL, "bad argument");
+    if (!s->pl.d.valid_mode) { s->num_res = 0; return PVGPU_OK; }  // phasevocoder.cc:104-106: unknown mode does nothing
+    int rc;
+    if ((rc = lock_rows(s, kind))) return rc;
+    long k0;
+    const int added = stream_feed(s, n, &k0);
     if (added > 0) {
         if ((rc = stream_run_new<T>(s, k0, added, in, n))) return rc;
     } else if (n > 0) {
@@ -2308,50 +2333,15 @@ static int process_host(pvgpu_stream *s, const T *const *in, int n) {
 }
 
 template <typename T>
-static int retrieve_host(pvgpu_stream *s, T *const *out, int n) {
-    if (!s || n < 0 || (n > 0 && !out)) return -fail(PVGPU_EINVAL, "bad argument");
-    if (check_retrieve_rows(s, std::is_same<T, float>::value ? 1 : 3)) return -PVGPU_ESTATE;
-    RowFifo<T> &fifo = host_fifo<T>(s);
-    long k = std::min<long>(n, s->num_res);  // phasevocoder.cc:111-113
-    k = std::min<long>(k, s->sched->available());
-    k = std::min<long>(k, (long)fifo.count);
-    fifo.pop(out, (size_t)k, s->pool);
-    s->sched->drain(k);
-    return (int)k;
-}
-
-template <typename T>
-static int process_block_host(pvgpu_stream *s, T *const *buf, int n, int *ready) {
-    if (!s || !ready) return fail(PVGPU_EINVAL, "bad argument");
-    const int m = s->cfg.mode;
-    if (m == PVGPU_NORMAL_STRETCH || m < -1 || m > PVGPU_FORMANT_CEPSTRAL) { *ready = 1; return PVGPU_OK; }  // processBlock routes neither (phasevocoder.cc:133-146)
-    int rc = guarded([&]() -> int { return process_host<T>(s, buf, n); });
-    if (rc) return rc;
-    if (s->num_res >= n) {  // processBlockNormal, phasevocoder.cc:156-183
-        const int saved = s->num_res;
-        retrieve_host<T>(s, buf, n);
-        s->num_res = saved;
-        *ready = 1;
-    } else {
-        *ready = 0;
-    }
-    return PVGPU_OK;
-}
-
-template <typename T>
-static int process_device(pvgpu_stream *s, const T *d_in, int64_t in_pitch, int n, cudaStream_t st) {
+static int process_device(pvgpu_stream *s, const RowKind &kind, const T *d_in, int64_t in_pitch, int n, void *cuda_stream) {
     if (!s || n < 0 || (n > 0 && !d_in) || in_pitch < n) return fail(PVGPU_EINVAL, "bad argument");
     if (!s->pl.d.valid_mode) { s->num_res = 0; return PVGPU_OK; }
     int rc;
-    if ((rc = lock_rows(s, std::is_same<T, float>::value ? 2 : 4))) return rc;
+    if ((rc = lock_rows(s, kind))) return rc;
     CU(cudaSetDevice(s->pl.device));
-    if (s->carrier) {
-        const size_t at = s->car_tail.size();
-        s->car_tail.resize(at + n);
-        s->carrier->generate(s->car_tail.data() + at, (size_t)n);
-    }
-    const long k0 = s->sched->recs_base() + s->sched->slices();
-    const int added = s->sched->feed(n);   // the schedule does not depend on the data: no call has to wait for the device
+    const cudaStream_t st = cuda_stream ? (cudaStream_t)cuda_stream : cudaStreamLegacy;
+    long k0;
+    const int added = stream_feed(s, n, &k0);
     if (n > 0) {   // the new samples join the device-resident window right away
         if ((rc = stream_ensure_window(s, s->dev_len + n, st))) return rc;
         launch_place_rows(s->d_inbuf[s->cur_in].as<T>() + s->dev_len, s->in_cap, d_in, in_pitch, n, s->R(), st);
@@ -2362,35 +2352,36 @@ static int process_device(pvgpu_stream *s, const T *d_in, int64_t in_pitch, int 
     return PVGPU_OK;
 }
 
+// Every kind of rows: host rows are popped into the caller's rows `out`, device rows into the caller's block `d_out` (rows
+// `out_pitch` samples apart) on the caller's stream.  Returns the samples per row, or -error.
 template <typename T>
-static int retrieve_device(pvgpu_stream *s, T *d_out, int64_t out_pitch, int n, void *cuda_stream) {
-    if (!s || n < 0 || (n > 0 && !d_out) || out_pitch < n) return -fail(PVGPU_EINVAL, "bad argument");
-    if (check_retrieve_rows(s, std::is_same<T, float>::value ? 2 : 4)) return -PVGPU_ESTATE;
-    long k = std::min<long>(n, s->num_res);
+static int retrieve(pvgpu_stream *s, const RowKind &kind, T *const *out, T *d_out, int64_t out_pitch, int n, void *cuda_stream) {
+    if (!s || n < 0 || (n > 0 && (kind.dev ? !d_out : !out)) || (kind.dev && out_pitch < n)) return -fail(PVGPU_EINVAL, "bad argument");
+    if (s->kind && s->kind != &kind) return -fail(PVGPU_ESTATE, "this instance is fed %s rows; use %s", s->kind->name, s->kind->retrieve);
+    long k = std::min<long>(n, s->num_res);  // phasevocoder.cc:111-113
     k = std::min<long>(k, s->sched->available());
-    k = std::min<long>(k, (long)s->dfifo_count);
-    if (k > 0) {
+    k = std::min<long>(k, (long)s->ring.count);
+    if (k > 0 && kind.dev) {
         if (cudaSetDevice(s->pl.device) != cudaSuccess) return -fail(PVGPU_ECUDA, "cudaSetDevice failed");
-        launch_ring_rows(d_out, out_pitch, 0, -1, s->d_fifo.as<T>(), (int64_t)s->dfifo_cap, (int64_t)s->dfifo_rd, (int64_t)s->dfifo_cap - 1, (int)k, s->R(),
-                         cuda_stream ? (cudaStream_t)cuda_stream : cudaStreamLegacy);
-        s->dfifo_rd = (s->dfifo_rd + (size_t)k) & (s->dfifo_cap - 1);
-        s->dfifo_count -= (size_t)k;
-        if (s->dfifo_count == 0) s->dfifo_rd = 0;
+        s->ring.pop(d_out, out_pitch, (size_t)k, cuda_stream ? (cudaStream_t)cuda_stream : cudaStreamLegacy);
+    } else if (k > 0) {
+        s->ring.pop(out, (size_t)k, s->pool);
     }
     s->sched->drain(k);
     return (int)k;
 }
 
+// The in-place block protocol on the caller's rows: `buf` for host rows, `d_buf` (rows `pitch` samples apart) for device rows.
 template <typename T>
-static int process_block_device(pvgpu_stream *s, T *d_buf, int64_t pitch, int n, void *cuda_stream, int *ready) {
+static int process_block(pvgpu_stream *s, const RowKind &kind, T *const *buf, T *d_buf, int64_t pitch, int n, void *cuda_stream, int *ready) {
     if (!s || !ready) return fail(PVGPU_EINVAL, "bad argument");
     const int m = s->cfg.mode;
-    if (m == PVGPU_NORMAL_STRETCH || m < -1 || m > PVGPU_FORMANT_CEPSTRAL) { *ready = 1; return PVGPU_OK; }
-    int rc = guarded([&]() -> int { return process_device<T>(s, d_buf, pitch, n, cuda_stream ? (cudaStream_t)cuda_stream : cudaStreamLegacy); });
+    if (m == PVGPU_NORMAL_STRETCH || m < -1 || m > PVGPU_FORMANT_CEPSTRAL) { *ready = 1; return PVGPU_OK; }  // processBlock routes neither (phasevocoder.cc:133-146)
+    int rc = guarded([&]() -> int { return kind.dev ? process_device<T>(s, kind, d_buf, pitch, n, cuda_stream) : process_host<T>(s, kind, buf, n); });
     if (rc) return rc;
-    if (s->num_res >= n) {
+    if (s->num_res >= n) {  // processBlockNormal, phasevocoder.cc:156-183
         const int saved = s->num_res;
-        const int k = retrieve_device<T>(s, d_buf, pitch, n, cuda_stream);
+        const int k = retrieve<T>(s, kind, buf, d_buf, pitch, n, cuda_stream);
         if (k < 0) return -k;
         s->num_res = saved;
         *ready = 1;
@@ -2403,39 +2394,43 @@ static int process_block_device(pvgpu_stream *s, T *d_buf, int64_t pitch, int n,
 extern "C" {
 
 int pvgpu_process(pvgpu_stream *s, const float *const *in, int n) {
-    return guarded([&]() -> int { return process_host<float>(s, in, n); });
+    return guarded([&]() -> int { return process_host(s, kHostRows, in, n); });
 }
 int pvgpu_process_s16(pvgpu_stream *s, const int16_t *const *in, int n) {
-    return guarded([&]() -> int { return process_host<int16_t>(s, in, n); });
+    return guarded([&]() -> int { return process_host(s, kHostS16Rows, in, n); });
 }
 
 int pvgpu_available(const pvgpu_stream *s) { return s ? s->num_res : 0; }
 
-int pvgpu_retrieve(pvgpu_stream *s, float *const *out, int n) { return retrieve_host<float>(s, out, n); }
-int pvgpu_retrieve_s16(pvgpu_stream *s, int16_t *const *out, int n) { return retrieve_host<int16_t>(s, out, n); }
+int pvgpu_retrieve(pvgpu_stream *s, float *const *out, int n) { return retrieve<float>(s, kHostRows, out, nullptr, 0, n, nullptr); }
+int pvgpu_retrieve_s16(pvgpu_stream *s, int16_t *const *out, int n) { return retrieve<int16_t>(s, kHostS16Rows, out, nullptr, 0, n, nullptr); }
 
-int pvgpu_process_block(pvgpu_stream *s, float *const *buf, int n, int *ready) { return process_block_host<float>(s, buf, n, ready); }
-int pvgpu_process_block_s16(pvgpu_stream *s, int16_t *const *buf, int n, int *ready) { return process_block_host<int16_t>(s, buf, n, ready); }
+int pvgpu_process_block(pvgpu_stream *s, float *const *buf, int n, int *ready) {
+    return process_block<float>(s, kHostRows, buf, nullptr, 0, n, nullptr, ready);
+}
+int pvgpu_process_block_s16(pvgpu_stream *s, int16_t *const *buf, int n, int *ready) {
+    return process_block<int16_t>(s, kHostS16Rows, buf, nullptr, 0, n, nullptr, ready);
+}
 
 int pvgpu_process_device(pvgpu_stream *s, const float *d_in, int64_t in_pitch, int n, void *cuda_stream) {
-    return guarded([&]() -> int { return process_device<float>(s, d_in, in_pitch, n, cuda_stream ? (cudaStream_t)cuda_stream : cudaStreamLegacy); });
+    return guarded([&]() -> int { return process_device(s, kDeviceRows, d_in, in_pitch, n, cuda_stream); });
 }
 int pvgpu_process_device_s16(pvgpu_stream *s, const int16_t *d_in, int64_t in_pitch, int n, void *cuda_stream) {
-    return guarded([&]() -> int { return process_device<int16_t>(s, d_in, in_pitch, n, cuda_stream ? (cudaStream_t)cuda_stream : cudaStreamLegacy); });
+    return guarded([&]() -> int { return process_device(s, kDeviceS16Rows, d_in, in_pitch, n, cuda_stream); });
 }
 
 int pvgpu_retrieve_device(pvgpu_stream *s, float *d_out, int64_t out_pitch, int n, void *cuda_stream) {
-    return retrieve_device<float>(s, d_out, out_pitch, n, cuda_stream);
+    return retrieve<float>(s, kDeviceRows, nullptr, d_out, out_pitch, n, cuda_stream);
 }
 int pvgpu_retrieve_device_s16(pvgpu_stream *s, int16_t *d_out, int64_t out_pitch, int n, void *cuda_stream) {
-    return retrieve_device<int16_t>(s, d_out, out_pitch, n, cuda_stream);
+    return retrieve<int16_t>(s, kDeviceS16Rows, nullptr, d_out, out_pitch, n, cuda_stream);
 }
 
 int pvgpu_process_block_device(pvgpu_stream *s, float *d_buf, int64_t pitch, int n, void *cuda_stream, int *ready) {
-    return process_block_device<float>(s, d_buf, pitch, n, cuda_stream, ready);
+    return process_block<float>(s, kDeviceRows, nullptr, d_buf, pitch, n, cuda_stream, ready);
 }
 int pvgpu_process_block_device_s16(pvgpu_stream *s, int16_t *d_buf, int64_t pitch, int n, void *cuda_stream, int *ready) {
-    return process_block_device<int16_t>(s, d_buf, pitch, n, cuda_stream, ready);
+    return process_block<int16_t>(s, kDeviceS16Rows, nullptr, d_buf, pitch, n, cuda_stream, ready);
 }
 
 static int pvgpu_set_meters_body(pvgpu_stream *s, int enable) {
@@ -2468,8 +2463,8 @@ int pvgpu_set_meters(pvgpu_stream *s, int enable) {
 // A getter of the other kind of rows is refused with the name of the one to use; before the first data call either works.
 static int check_meters(const pvgpu_stream *s, bool device_getter) {
     if (!s->meters) return fail(PVGPU_ESTATE, "meters are off on this instance (pvgpu_set_meters)");
-    if (s->io_mode && s->dev_rows() != device_getter)
-        return fail(PVGPU_ESTATE, "this instance is fed %s rows; use %s", kRowKind[s->io_mode], s->dev_rows() ? "pvgpu_get_meters_device" : "pvgpu_get_meters");
+    if (s->kind && s->kind->dev != device_getter)
+        return fail(PVGPU_ESTATE, "this instance is fed %s rows; use %s", s->kind->name, s->kind->meters);
     return PVGPU_OK;
 }
 
