@@ -110,6 +110,10 @@ SYMBOLS = {
     "pvgpu_bind_thread_to_device": (C.c_int, [C.c_int]),
     "pvgpu_test_forward_polar": (C.c_int, [C.c_int, C.c_int, C.c_int, _fp, _fp, _fp]),
     "pvgpu_test_inverse_polar": (C.c_int, [C.c_int, C.c_int, C.c_int, _fp, _fp, _fp]),
+    "pvgpu_test_analyse": (C.c_int, [C.POINTER(Config), C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_int64, C.c_int64, _i64p, C.c_int64, C.c_int,
+                                     _fp, _fp]),
+    "pvgpu_test_phase_core": (C.c_int, [C.POINTER(Config), C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_int), _fp, _fp,
+                                        C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(C.c_int), _fp, _fp, _fp, _fp, _fp]),
     "pvgpu_test_atan2f": (C.c_int, [C.c_int, C.c_int64, _fp, _fp, _fp]),
     "pvgpu_test_princarg": (C.c_int, [C.c_int, C.c_int64, C.POINTER(C.c_double), C.POINTER(C.c_double)]),
     "pvgpu_test_postchain": (C.c_int, [C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_int64, _fp]),

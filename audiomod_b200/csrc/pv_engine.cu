@@ -16,6 +16,7 @@
 #include <condition_variable>
 #include <exception>
 #include <functional>
+#include <limits>
 #include <map>
 #include <memory>
 #include <mutex>
@@ -536,16 +537,12 @@ struct Pipeline {
         launch_analyse(p, g, k0, nf, st);
         span_end(sp, st); ++launches;
     }
-    int run_modify_synth(const DevRows &g, long k0, int nf, cudaStream_t st) {
+    // The phase core of the shift / stretch / formant / gender modes over frames [k0, k0+nf), state carried in g from the
+    // previous call.  Also run on its own by pvgpu_test_phase_core.
+    int run_core(const DevRows &g, long k0, int nf, cudaStream_t st) {
         const SliceRec *recs = b_recs.as<SliceRec>();
         Span *sp;
-        if (d.robotic || d.whisper) {
-            if (g.spec) { /* phases are produced inside the synthesis kernel */ } else {
-            sp = span_begin(5, st);
-            launch_fixed_phase(p, g, d.whisper ? b_whisper.as<float>() : nullptr, k0, nf, st);
-            span_end(sp, st); ++launches;
-            }
-        } else if (g.spec && cartesian_lock()) {
+        if (g.spec && cartesian_lock()) {
             // phase-locked core on Cartesian spectra: frame-parallel peak / link / advance records, then the serial chain
             sp = span_begin(6, st); launch_lock_peaks(p, g, recs, recs_base, k0, nf, st); span_end(sp, st); ++launches;
             // the chunk's last frame is what the next launch links to (before the chain touches classic frames in place)
@@ -553,8 +550,22 @@ struct Pipeline {
             CU(cudaMemcpy2DAsync(g.lock_tail, 2 * w, g.mag + (size_t)(nf - 1) * p.Hp, pitch, w, g.rows, cudaMemcpyDeviceToDevice, st));
             CU(cudaMemcpy2DAsync(g.lock_tail + p.Hp, 2 * w, g.phase + (size_t)(nf - 1) * p.Hp, pitch, w, g.rows, cudaMemcpyDeviceToDevice, st));
             sp = span_begin(7, st); launch_lock_chain(p, g, nf, st); span_end(sp, st); ++launches;
-        } else if (!d.vocoder && !d.constant_mode) {
+        } else {
             sp = span_begin(1, st); launch_phase_core(p, g, d.cfg.coremode, recs, recs_base, k0, nf, st); span_end(sp, st); ++launches;
+        }
+        return PVGPU_OK;
+    }
+    int run_modify_synth(const DevRows &g, long k0, int nf, cudaStream_t st) {
+        Span *sp;
+        if (d.robotic || d.whisper) {
+            if (g.spec) { /* phases are produced inside the synthesis kernel */ } else {
+            sp = span_begin(5, st);
+            launch_fixed_phase(p, g, d.whisper ? b_whisper.as<float>() : nullptr, k0, nf, st);
+            span_end(sp, st); ++launches;
+            }
+        } else if (!d.vocoder && !d.constant_mode) {
+            const int rc = run_core(g, k0, nf, st);
+            if (rc) return rc;
         }
         if (d.cepstral) {   // optional modes 8 / 9: whiten by the cepstral envelope, put the warped envelope back (pv_cepstral.cu)
             sp = span_begin(5, st);
@@ -1454,6 +1465,136 @@ int pvgpu_test_inverse_polar(int device, int fftsize, int n_frames, const float 
     launch_synthesise(pl.p, g, nullptr, nullptr, 0, n_frames, nullptr);
     CU(cudaGetLastError());
     CU(cudaMemcpy(frames, d_fr.p, sizeof(float) * (size_t)n_frames * N, cudaMemcpyDeviceToHost));
+    return PVGPU_OK;
+}
+
+static bool templated_size(int n) { return n == 512 || n == 1024 || n == 2048 || n == 4096 || n == 8192; }
+
+int pvgpu_test_analyse(const pvgpu_config *cfg, int spec, int fmt, int rows, const void *in, int64_t in_stride, int64_t in_base,
+                       const int64_t *n_in, int64_t k0, int n_frames, float *a, float *b) {
+    if (!in || !n_in || !a || !b || rows < 1 || rows > 65535 || n_frames < 1 || k0 < 0 || in_stride < 1 || in_base < 0 || (spec != 0 && spec != 1) ||
+        (fmt != PVGPU_F32 && fmt != PVGPU_S16))
+        return fail(PVGPU_EINVAL, "bad argument");
+    int rc = validate(cfg);
+    if (rc) return rc;
+    if (cfg->hopsize < 1) return fail(PVGPU_EINVAL, "the analysis hook needs an explicit hopsize");
+    if (spec && !templated_size(cfg->fftsize)) return fail(PVGPU_EINVAL, "Cartesian spectra exist only for FFT sizes 512..8192 (got %d)", cfg->fftsize);
+    Pipeline pl;
+    if ((rc = pl.init(*cfg))) return rc;
+    const int N = pl.p.N, H = pl.p.H, Hp = pl.p.Hp;
+    const int64_t hop = pl.p.hop;
+    // the kernel reads samples [k * hop, min(n_in, k * hop + N)) of each frame: they must lie in the caller's rows
+    for (int r = 0; r < rows; ++r) {
+        const int64_t lo = k0 * hop, hi = std::min(n_in[r], (k0 + n_frames - 1) * hop + N);
+        if (hi > lo && (lo < in_base || hi - in_base > in_stride))
+            return fail(PVGPU_EINVAL, "row %d: samples [%lld, %lld) are read, the rows hold [%lld, %lld)", r, (long long)lo, (long long)hi,
+                        (long long)in_base, (long long)(in_base + in_stride));
+    }
+    const size_t esz = fmt == PVGPU_S16 ? sizeof(int16_t) : sizeof(float);
+    DevBuf d_in, d_len, d_a, d_b;
+    if ((rc = Pipeline::upload(d_in, in, esz * (size_t)rows * in_stride))) return rc;
+    if ((rc = Pipeline::upload(d_len, n_in, sizeof(int64_t) * rows))) return rc;
+    const size_t slots = (size_t)rows * n_frames;
+    CU(d_a.ensure(sizeof(float) * slots * Hp));
+    CU(d_b.ensure(sizeof(float) * slots * Hp));
+    DevRows g{};
+    g.rows = rows; g.channels = 1; g.fmt = fmt; g.spec = spec;
+    g.in = d_in.p; g.in_stride = in_stride; g.in_base = in_base; g.n_in = d_len.as<int64_t>();
+    g.mag = d_a.as<float>(); g.phase = d_b.as<float>(); g.F = n_frames;
+    launch_analyse(pl.p, g, k0, n_frames, nullptr);   // the pipeline's launch (Pipeline::run_analyse)
+    CU(cudaGetLastError());
+    CU(cudaMemcpy2D(a, sizeof(float) * H, d_a.p, sizeof(float) * Hp, sizeof(float) * H, slots, cudaMemcpyDeviceToHost));
+    CU(cudaMemcpy2D(b, sizeof(float) * H, d_b.p, sizeof(float) * Hp, sizeof(float) * H, slots, cudaMemcpyDeviceToHost));
+    return PVGPU_OK;
+}
+
+int pvgpu_test_phase_core(const pvgpu_config *cfg, int spec, int streams, int n_frames, int frames_per_launch, const int *phase_inc, const float *a,
+                          const float *b, int *kind, int *npeaks, int *region, float *csn, float *rot, float *out_a, float *out_b, float *frames) {
+    if (!phase_inc || !a || !b || !out_a || !out_b || streams < 1 || n_frames < 1 || frames_per_launch < 1 || (spec != 0 && spec != 1))
+        return fail(PVGPU_EINVAL, "bad argument");
+    int rc = validate(cfg);
+    if (rc) return rc;
+    Pipeline pl;
+    if ((rc = pl.init(*cfg))) return rc;
+    const Derived &d = pl.d;
+    if (d.robotic || d.whisper || d.vocoder || d.constant_mode || d.cepstral)
+        return fail(PVGPU_EINVAL, "the phase core runs in the shift / stretch / formant / gender modes only");
+    if (spec && !(pl.cartesian() && pl.cartesian_lock()))
+        return fail(PVGPU_EINVAL, "this configuration does not run the phase-locked core on Cartesian spectra (coremode 1, FFT 512..8192)");
+    const DevPlan &p = pl.p;
+    const int C = d.cfg.channels, rows = streams * C, N = p.N, H = p.H, Hp = p.Hp, half = p.half, maxpk = pl.max_peaks();
+    const int F = std::min(frames_per_launch, n_frames);
+    if ((int64_t)rows * F > INT32_MAX / 2) return fail(PVGPU_EINVAL, "too many rows x frames");
+    // the cores read only phase_inc of the slice records
+    std::vector<SliceRec> recs((size_t)n_frames);
+    for (int f = 0; f < n_frames; ++f) recs[f].phase_inc = phase_inc[f];
+    if ((rc = Pipeline::upload(pl.b_recs, recs.data(), sizeof(SliceRec) * recs.size()))) return rc;
+    pl.recs_base = 0;
+    Workspace ws;
+    if ((rc = ws.ensure(pl, rows, F, 0))) return rc;
+    if ((rc = ws.reset_state(pl, nullptr))) return rc;
+    DevRows g{};
+    g.rows = rows; g.channels = C;
+    g.spec = spec; g.synth_kind = spec ? 4 : 0;
+    ws.bind(pl, g);
+    const size_t slots = (size_t)rows * F;
+    std::vector<int2> hdr(spec ? slots : 0);
+    std::vector<unsigned short> map(spec ? slots * half : 0);
+    std::vector<float2> cs(spec ? slots * maxpk : 0);
+    std::vector<float> lrot(spec ? (size_t)rows * maxpk : 0);
+    std::vector<int> lkind(spec ? rows : 0);
+    const float nan = std::numeric_limits<float>::quiet_NaN();
+    for (long k0 = 0; k0 < n_frames; k0 += F) {
+        const int nf = (int)std::min<long>(F, n_frames - k0);
+        for (int r = 0; r < rows; ++r) {
+            const size_t src = ((size_t)r * n_frames + k0) * H, dst = (size_t)r * F * Hp;
+            CU(cudaMemcpy2D(g.mag + dst, sizeof(float) * Hp, a + src, sizeof(float) * H, sizeof(float) * H, nf, cudaMemcpyHostToDevice));
+            CU(cudaMemcpy2D(g.phase + dst, sizeof(float) * Hp, b + src, sizeof(float) * H, sizeof(float) * H, nf, cudaMemcpyHostToDevice));
+        }
+        if ((rc = pl.run_core(g, k0, nf, nullptr))) return rc;
+        if (frames) launch_synthesise(p, g, nullptr, nullptr, k0, nf, nullptr);
+        CU(cudaGetLastError());
+        for (int r = 0; r < rows; ++r) {
+            const size_t dst = ((size_t)r * n_frames + k0) * H, src = (size_t)r * F * Hp;
+            CU(cudaMemcpy2D(out_a + dst, sizeof(float) * H, g.mag + src, sizeof(float) * Hp, sizeof(float) * H, nf, cudaMemcpyDeviceToHost));
+            CU(cudaMemcpy2D(out_b + dst, sizeof(float) * H, g.phase + src, sizeof(float) * Hp, sizeof(float) * H, nf, cudaMemcpyDeviceToHost));
+            if (frames)
+                for (int f = 0; f < nf; ++f)
+                    CU(cudaMemcpy(frames + ((size_t)r * n_frames + k0 + f) * N, g.frames + ((size_t)r * g.Fr + (k0 + f) % g.Fr) * N, sizeof(float) * N,
+                                  cudaMemcpyDeviceToHost));
+        }
+        if (!spec) {
+            for (int r = 0; r < rows; ++r)
+                for (int f = 0; f < nf; ++f) {
+                    const size_t o = (size_t)r * n_frames + k0 + f;
+                    if (kind) kind[o] = -1;
+                    if (npeaks) npeaks[o] = -1;
+                }
+            continue;
+        }
+        CU(cudaMemcpy(hdr.data(), g.lock_hdr, sizeof(int2) * slots, cudaMemcpyDeviceToHost));
+        CU(cudaMemcpy(map.data(), g.lock_map, sizeof(unsigned short) * slots * half, cudaMemcpyDeviceToHost));
+        CU(cudaMemcpy(cs.data(), g.lock_csn, sizeof(float2) * slots * maxpk, cudaMemcpyDeviceToHost));
+        CU(cudaMemcpy(lkind.data(), g.lock_kind, sizeof(int) * rows, cudaMemcpyDeviceToHost));
+        CU(cudaMemcpy(lrot.data(), g.lock_rot, sizeof(float) * rows * maxpk, cudaMemcpyDeviceToHost));
+        for (int r = 0; r < rows; ++r)
+            for (int f = 0; f < nf; ++f) {
+                const size_t o = (size_t)r * n_frames + k0 + f, s = (size_t)r * F + f;
+                const int npk = hdr[s].x, kd = hdr[s].y;
+                const bool locked = kd == 2;
+                if (kind) kind[o] = kd;
+                if (npeaks) npeaks[o] = npk;
+                if (region)
+                    for (int i = 0; i < half; ++i) region[o * half + i] = locked ? map[s * half + i] : -1;
+                if (csn)
+                    for (int i = 0; i < maxpk; ++i) {
+                        csn[2 * (o * maxpk + i)] = locked && i < npk ? cs[s * maxpk + i].x : nan;
+                        csn[2 * (o * maxpk + i) + 1] = locked && i < npk ? cs[s * maxpk + i].y : nan;
+                    }
+                if (rot)   // lock_rot holds the rotations of the launch's last frame when that frame was locked
+                    for (int i = 0; i < maxpk; ++i) rot[o * maxpk + i] = f == nf - 1 && lkind[r] == 2 && i < npk ? lrot[(size_t)r * maxpk + i] : nan;
+            }
+    }
     return PVGPU_OK;
 }
 

@@ -329,6 +329,28 @@ int pvgpu_run_wav_files(const pvgpu_config *cfg, pvgpu_wav_job *jobs, int n_jobs
 int pvgpu_test_forward_polar(int device, int fftsize, int n_frames, const float *frames, float *mag, float *phase);
 /* 1/N scale + FFT::inversePolar + ifftshift + window (phasevocoderprocess.cc:1024-1056) */
 int pvgpu_test_inverse_polar(int device, int fftsize, int n_frames, const float *mag, const float *phase, float *frames);
+/* The pipeline's analysis launch (frame gather, Hann, fftshift, real FFT; Pipeline::run_analyse) over frames [k0, k0 + n_frames) of
+ * `rows` rows, with the plan of cfg (fftsize, hopsize > 0, device).  in: [rows][in_stride] float32 or int16 samples (fmt), element 0
+ * of a row is its global sample in_base; n_in[rows]: samples of each row that exist (global positions; zeros from there on).  Every
+ * sample a frame reads below n_in must lie in the rows (else PVGPU_EINVAL).  spec 1: a = re, b = im (FFT sizes 512..8192 only);
+ * spec 0: a = magnitude, b = phase.  a, b: [rows][n_frames][fftsize/2 + 1]. */
+int pvgpu_test_analyse(const pvgpu_config *cfg, int spec, int fmt, int rows, const void *in, int64_t in_stride, int64_t in_base,
+                       const int64_t *n_in, int64_t k0, int n_frames, float *a, float *b);
+/* The pipeline's phase core (Pipeline::run_core) over n_frames frames of `streams` streams of cfg->channels rows each, from fresh
+ * state, frames_per_launch frames per launch.  phase_inc[n_frames]: phaseIncrement of each frame.  a, b: [rows][n_frames][H]
+ * spectra, H = fftsize/2 + 1: (re, im) for spec 1 (the phase-locked core on Cartesian spectra: coremode 1, FFT 512..8192), (magnitude,
+ * phase) for spec 0 (the serial polar cores, any coremode and size).  Outputs, rows = streams * channels, maxpk = fftsize/6 + 2
+ * (each may be null; spec 0 fills kind and npeaks with -1 and leaves region, csn and rot alone):
+ *   kind, npeaks [rows][n_frames]  frame kind (0 pass-through, 1 classic propagation, 2 locked) and number of peaks
+ *   region [rows][n_frames][fftsize/2]  locked frames: the region (peak index) of every bin; -1 elsewhere
+ *   csn [rows][n_frames][maxpk][2]  locked frames: (cos, sin) of every region's rotation; NaN elsewhere
+ *   rot [rows][n_frames][maxpk]  the rotations of the last frame of each launch when it is locked; NaN elsewhere
+ *   out_a, out_b [rows][n_frames][H] (required)  the spectra after the core: spec 1 rewrites classic frames as (re, im) of the
+ *                                    propagated phase, spec 0 writes the output phases into out_b
+ *   frames [rows][n_frames][fftsize]  the synthesised frames (1/N scale, inverse FFT, ifftshift, window) */
+int pvgpu_test_phase_core(const pvgpu_config *cfg, int spec, int streams, int n_frames, int frames_per_launch, const int *phase_inc,
+                          const float *a, const float *b, int *kind, int *npeaks, int *region, float *csn, float *rot, float *out_a,
+                          float *out_b, float *frames);
 /* device atan2f restatement (FFT.cc:2629 -> glibc atan2f) */
 int pvgpu_test_atan2f(int device, int64_t n, const float *y, const float *x, float *out);
 /* princarg (src/common/system/sys.h:84-91) */

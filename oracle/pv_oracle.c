@@ -535,6 +535,9 @@ typedef struct pvo {
     rosen_t *chord;                            /* three per channel */
     int num_res, outready;
     long slices, dropped;
+    /* optional record of modify_locked (pvo_phase_core_frames): per peak its rotation and region [bin1, bin2); null = none */
+    float *rec_rot;
+    int *rec_bin1, *rec_bin2;
 } pvo_t;
 
 static void chan_init(chan_t *c, int N, long outbuf_size) {
@@ -731,6 +734,7 @@ static void modify_locked(pvo_t *p, chan_t *ad, size_t phaseIncrement) {
                 bin2 = round((p->peak[pk + 1] + p2) * 0.5);
             }
             for (i = bin1; i < bin2; i++) ad->locked[i] = princarg(ad->phase[i] + peak_phase_rotation);
+            if (p->rec_rot) { p->rec_rot[pk] = peak_phase_rotation; p->rec_bin1[pk] = bin1; p->rec_bin2[pk] = bin2; }
         }
         for (i = 0; i < halfsize; i++) {
             ad->prev_phase[i] = ad->phase[i];
@@ -1153,4 +1157,49 @@ int pvo_resampler_params(float pitch_scale, uint32_t *num, uint32_t *den, uint32
     if (table && table_cap >= n) memcpy(table, rs.table, sizeof(float) * n);
     free(rs.table); free(rs.mem);
     return n;
+}
+
+/* (re, im) -> (sqrtf(re*re + im*im), atan2f(im, re)), the polar step of forwardPolar (FFT.cc:2624-2629): polar spectra from given
+   Cartesian ones, rounded as the reference rounds them.  re_im: [n][2]. */
+void pvo_polar(long n, const float *re_im, float *mag, float *phase) {
+    long i;
+    for (i = 0; i < n; ++i) {
+        const float r = re_im[2 * i], m = re_im[2 * i + 1];
+        mag[i] = sqrtf(r * r + m * m);
+        phase[i] = atan2f(m, r);
+    }
+}
+
+/* The phase core of one stream (processSliceForChannel's modify call, :305-376) over given analysis frames, from the state of a fresh
+   process: frames in order, the channels of a frame in order, sharing the peak lists.  N: FFT size, hop: input hop, ch channels,
+   coremode 0 / 1 / 2, n frames with phase_inc[n].  mag, phase: [ch][n][N/2+1] analysis spectra.  Outputs per (channel, frame):
+   branch [ch][n]  0 pass-through first frame, 1 classic propagation, 2 locked, 3 int ratio (coremode 2);
+   npeak [ch][n], peaks [ch][n][maxpk]  the peaks picked (coremode 1; 0 otherwise);
+   rot, bin1, bin2 [ch][n][maxpk]  locked frames: each peak's peak_phase_rotation and region [bin1, bin2);
+   out_phase [ch][n][N/2+1]  the phases after the core (the Nyquist bin keeps its analysis phase).
+   maxpk: room for N/6 + 2 peaks per frame. */
+void pvo_phase_core_frames(int N, int hop, int ch, int coremode, int n, const int *phase_inc, const float *mag, const float *phase, int maxpk,
+                           int *branch, int *npeak, int *peaks, float *rot, int *bin1, int *bin2, float *out_phase) {
+    pvo_t *p = pvo_create(44100, ch, 1.0f, 0.0f, MODE_SHIFT, coremode, N, hop);
+    const int H = p->N / 2 + 1;
+    int f, c, i;
+    for (f = 0; f < n; ++f)
+        for (c = 0; c < ch; ++c) {
+            chan_t *ad = &p->chan[c];
+            const long o = (long)c * n + f;
+            const int first = coremode == 1 ? p->first_locked : p->first_simple, nprev = p->nprev;
+            memcpy(ad->mag, mag + o * H, sizeof(float) * H);
+            memcpy(ad->phase, phase + o * H, sizeof(float) * H);
+            p->rec_rot = rot + o * maxpk; p->rec_bin1 = bin1 + o * maxpk; p->rec_bin2 = bin2 + o * maxpk;
+            if (coremode == 1) modify_locked(p, ad, (size_t)phase_inc[f]);
+            else if (coremode == 2) modify_intratio(p, ad, (size_t)phase_inc[f]);
+            else modify_simple(p, ad, (size_t)phase_inc[f]);
+            p->rec_rot = NULL; p->rec_bin1 = p->rec_bin2 = NULL;
+            if (coremode == 2) branch[o] = 3;
+            else branch[o] = first ? 0 : (p->npeak == 0 || nprev == 0) ? 1 : 2;
+            npeak[o] = coremode == 1 ? p->npeak : 0;
+            for (i = 0; i < npeak[o] && i < maxpk; ++i) peaks[o * maxpk + i] = p->peak[i];
+            memcpy(out_phase + o * H, ad->phase, sizeof(float) * H);
+        }
+    pvo_destroy(p);
 }

@@ -62,6 +62,10 @@ def lib() -> C.CDLL:
                                       _fp, C.c_long, _fp, C.c_long, C.c_int, C.POINTER(C.c_long)]
         L.pvo_forward_polar.argtypes = [C.c_int, _fp, _fp, _fp, _fp]
         L.pvo_inverse_polar.argtypes = [C.c_int, _fp, _fp, _fp]
+        L.pvo_polar.argtypes = [C.c_long, _fp, _fp, _fp]
+        _ip = C.POINTER(C.c_int)
+        L.pvo_phase_core_frames.argtypes = [C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _ip, _fp, _fp, C.c_int,
+                                            _ip, _ip, _ip, _fp, _ip, _ip, _fp]
         L.pvo_host_atan2f.restype = C.c_float
         L.pvo_host_atan2f.argtypes = [C.c_float, C.c_float]
         L.pvo_host_atan2f_vec.argtypes = [_fp, _fp, _fp, C.c_long]
@@ -162,6 +166,36 @@ def inverse_polar(mag: np.ndarray, phase: np.ndarray, n: int) -> np.ndarray:
     out = np.zeros(n, np.float32)
     lib().pvo_inverse_polar(n, _ptr(mag), _ptr(phase), _ptr(out))
     return out
+
+
+def polar(re_im: np.ndarray):
+    """(re, im) pairs [..., 2] -> (sqrtf(re*re + im*im), atan2f(im, re)) rounded as the reference's forwardPolar."""
+    ri = np.ascontiguousarray(re_im, dtype=np.float32)
+    mag = np.empty(ri.shape[:-1], np.float32)
+    ph = np.empty(ri.shape[:-1], np.float32)
+    lib().pvo_polar(mag.size, _ptr(ri), _ptr(mag), _ptr(ph))
+    return mag, ph
+
+
+def phase_core_frames(mag: np.ndarray, phase: np.ndarray, phase_inc, hop: int, coremode: int = 1) -> dict:
+    """The reference's phase core (modify_locked / modify_simple / modify_intratio) over the polar frames of one stream,
+    mag / phase [ch][n][N/2+1], from fresh-process state, in the reference's channel order.  Returns per (channel, frame):
+    branch (0 pass-through, 1 classic, 2 locked, 3 int ratio), npeak, peaks / rot / bin1 / bin2 [ch][n][maxpk] (the first
+    npeak entries are valid; rot and bins on locked frames) and out_phase [ch][n][N/2+1]."""
+    mag = np.ascontiguousarray(mag, dtype=np.float32)
+    phase = np.ascontiguousarray(phase, dtype=np.float32)
+    ch, n, h = mag.shape
+    N = 2 * (h - 1)
+    maxpk = N // 6 + 2
+    inc = np.ascontiguousarray(np.broadcast_to(np.asarray(phase_inc, np.int32), (n,)))
+    ip = C.POINTER(C.c_int)
+    r = dict(branch=np.zeros((ch, n), np.int32), npeak=np.zeros((ch, n), np.int32), peaks=np.zeros((ch, n, maxpk), np.int32),
+             rot=np.full((ch, n, maxpk), np.nan, np.float32), bin1=np.zeros((ch, n, maxpk), np.int32),
+             bin2=np.zeros((ch, n, maxpk), np.int32), out_phase=np.zeros((ch, n, h), np.float32))
+    lib().pvo_phase_core_frames(N, hop, ch, coremode, n, inc.ctypes.data_as(ip), _ptr(mag), _ptr(phase), maxpk,
+                                r["branch"].ctypes.data_as(ip), r["npeak"].ctypes.data_as(ip), r["peaks"].ctypes.data_as(ip),
+                                _ptr(r["rot"]), r["bin1"].ctypes.data_as(ip), r["bin2"].ctypes.data_as(ip), _ptr(r["out_phase"]))
+    return r
 
 
 def host_atan2f(y: np.ndarray, x: np.ndarray) -> np.ndarray:
